@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- flow Mpix/s of the dense variational optical-flow path.
 
-    python bench.py --gpus N --steps K --warmup W [--workload fulldisk|conus|meso]
+    python bench.py --gpus N --steps K --warmup W [--workload fulldisk|conus|meso] [--dump-outputs DIR]
     python bench.py --impl reference ...          # the reference's own CPU flow path
 
 One "step" = one pass of the hot path over one synthetic image pair:
@@ -221,6 +221,48 @@ def flow_check(u, v, own0, nx, ny, workload, dist, write):
             "mean_abs_du": float(du.mean()), "mean_abs_dv": float(dv.mean()),
             "finite": bool(np.isfinite(us).all() and np.isfinite(vs).all()),
             "within_gates": bool(max(du.mean(), dv.mean()) <= 1e-3 and max(du.max(), dv.max()) <= 1e-2)}
+
+
+DUMP_NAMES = ("uPix", "vPix", "uVal", "vVal", "uVal2", "vVal2")
+DUMP_PIXELS = 1 << 21      # per plane: six float32 planes of at most 8 MB each
+DUMP_SEED = 20241020
+
+
+def dump_positions(nx, ny):
+    """Flat row-major pixel indices (ascending) that --dump-outputs samples, or None when the scene is written whole.
+    Fixed seed: every run of the same scene size samples the same pixels."""
+    import numpy as np
+    if nx * ny <= DUMP_PIXELS:
+        return None
+    idx = np.random.default_rng(DUMP_SEED).choice(nx * ny, DUMP_PIXELS, replace=False, shuffle=False)
+    idx.sort()
+    return idx
+
+
+def dump_outputs(out_dir, nx, ny, own0, planes, dist):
+    """--dump-outputs: the planes the timed path hands its caller (pixel displacements u, v and the four navigated
+    short planes of pix2uv) as float32 <out_dir>/<name>.npy; ny x nx when the scene has at most DUMP_PIXELS pixels,
+    else the values at dump_positions(nx, ny).  Collective: every rank calls it with the rows it owns."""
+    import numpy as np
+    import torch
+    nown = planes[0].shape[0]
+    idx = dump_positions(nx, ny)
+    if idx is None:
+        mine = [p.float().cpu().numpy() for p in planes]
+    else:
+        sel = idx[(idx >= own0 * nx) & (idx < (own0 + nown) * nx)] - own0 * nx
+        t = torch.from_numpy(sel).to(planes[0].device)
+        mine = [p.reshape(-1).index_select(0, t).float().cpu().numpy() for p in planes]
+    parts = [(own0, mine)]
+    if dist:
+        parts = [None] * dist.get_world_size() if dist.get_rank() == 0 else None
+        dist.gather_object((own0, mine), parts, dst=0)
+        if dist.get_rank() != 0:
+            return
+    parts.sort(key=lambda t: t[0])
+    os.makedirs(out_dir, exist_ok=True)
+    for k, name in enumerate(DUMP_NAMES):
+        np.save(os.path.join(out_dir, name + ".npy"), np.concatenate([m[k] for _, m in parts]))
 
 
 def reference_arm(args):
@@ -491,7 +533,14 @@ def main():
                     help="N = 1: store the strided sample of this run's flow that later runs (any N) are checked against")
     ap.add_argument("--rank-stats", action="store_true",
                     help="developer (N > 1): add every rank's per-stage CUDA-event times of the profiled step to the line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (u, v and the four short planes) as float32 DIR/<name>.npy: "
+                         f"whole planes up to {DUMP_PIXELS} pixels, else the same seeded sample of that many pixels every run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "batch64"):
+        ap.error("--dump-outputs writes the flow workloads of --impl ours")
     if args.size:
         sx, sy = (int(t) for t in args.size.split("x"))
         WORKLOADS["custom"] = (sx, sy, "conus_0.5km", False)
@@ -596,6 +645,8 @@ def main():
     if rank == 0:
         sampler.start()
     ms_step = timed(step, args.steps)
+    if args.dump_outputs:       # before the profiled step below runs the path again
+        dump_outputs(args.dump_outputs, nx, ny, own0, [u, v, *shorts], dist)
     # one more step of the same loop with per-launch CUDA events around the finest level's
     # PCG kernels (that level runs un-graphed for it): the roofline's kernel durations
     ctx.set_profile(True)

@@ -189,6 +189,19 @@ def zoomout_input(name):
     return (rng.standard_normal((ny, nx)) * 1000 + 5000).astype(np.float32), factor
 
 
+def zoomout_reference(oracle, key, field, factor, pyramid=False):
+    """The reference's oct_zoom_out_float of `field` or, with pyramid=True, its double pyramid stage oct_zoom_out
+    rounded to float.  Computed by the reference's own object when oracle/_ref is built, else the stored output
+    zoomout_ref.npz[key] (make_golden.py --zoomout-only): keys are the ZOOMOUT names and config1_<factor> for the
+    500 x 500 texture of BASELINE config 1."""
+    try:
+        return oracle.ref_zoom_out(field, factor).astype(np.float32) if pyramid else oracle.ref_zoom_out_float(field, factor)
+    except OSError:
+        import os
+        with np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "zoomout_ref.npz")) as z:
+            return z[key]
+
+
 SRSAL = {
     # cloud deck with sharp edges (range weight switches neighbours off) and smooth height variation
     "srsal_96x80_deck": dict(nx=96, ny=80, seed=31, kind="deck"),

@@ -61,10 +61,33 @@ def srsal(out):
         print(name, "u range", float(us.min()), float(us.max()), "mean |du|", float(np.abs(us - u).mean()), flush=True)
 
 
+def zoomout(out):
+    """zoomout_ref.npz: the reference's CPU regridder oct_zoom_out_float on cases.ZOOMOUT and its double pyramid stage
+    oct_zoom_out, rounded to float, on the 500 x 500 texture of BASELINE config 1 (cases.zoomout_reference).  Without
+    oracle/_ref the outputs come from the oracle's restatement, which was bit-identical to the reference's object on
+    all of these inputs in every run that had both; the committed file was written that way."""
+    from octane_b200 import synthetic as S
+    try:
+        O.ref_cpu()
+        src = "reference"
+        fn, fn_pyr = O.ref_zoom_out_float, lambda f, k: O.ref_zoom_out(f, k).astype(np.float32)
+    except OSError:
+        src = "oracle"
+        fn = fn_pyr = O.zoom_out_float
+    d = {name: fn(*cases.zoomout_input(name)) for name in sorted(cases.ZOOMOUT)}
+    i1 = S.make_pair(500, 500, seed=1, kind="shift", drift=(2.0, -1.0))[0]
+    for factor in (0.5, 0.25, 0.125):
+        d[f"config1_{factor}"] = fn_pyr(i1, factor)
+    np.savez_compressed(os.path.join(out, "zoomout_ref.npz"), **d)
+    print("zoomout_ref from the", src, {k: v.shape for k, v in d.items()}, flush=True)
+
+
 def main(out):
     os.makedirs(out, exist_ok=True)
     if "--ingest-only" in sys.argv:
         return ingest(out)
+    if "--zoomout-only" in sys.argv:
+        return zoomout(out)
     if "--srsal-only" in sys.argv:
         return srsal(out)
     for name, c in cases.VARIATIONAL.items():
@@ -113,6 +136,7 @@ def main(out):
         print("dispatch ir", ir, "CTP range", int(outs[4].min()), int(outs[4].max()), flush=True)
     ingest(out)
     srsal(out)
+    zoomout(out)
 
 
 if __name__ == "__main__":
