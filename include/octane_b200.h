@@ -303,6 +303,13 @@ int octane_pix2uv_band_dev(octane_ctx* ctx, const octane_nav* nav, double t1, do
                            const float* d_u, const float* d_v, int nx, int row0, int nrows,
                            const octane_params* p,
                            short* d_U, short* d_V, short* d_U_raw, short* d_V_raw);
+/* -srsal on row bands (collective over the context's communicator): d_u / d_v (in/out) and d_cth hold the owned rows
+ * [own0,own1) of octane_band_plan, dense.  Each rank stages its rows with 18 more on each side, exchanges those with
+ * its neighbours and filters its own rows: the gathered result is bit for bit octane_srsal_dev on the whole scene.
+ * Every band must be at least 18 rows high (else OCTANE_EINVAL on every rank) and nx, ny must exceed 18.  A rank
+ * that cannot allocate its staging makes every rank return an error; the contexts stay usable.  World 1: exactly
+ * octane_srsal_dev.  Synchronises the host with the context's stream (the vote on the staging). */
+int octane_srsal_band_dev(octane_ctx* ctx, float* d_u_own, float* d_v_own, const float* d_cth_own, int nx, int ny);
 
 /* ---- pipelined host-buffer dispatcher (sequences of pairs; one GPU or row bands) -------
  * The reference processes one pair per run (src/main.cc:439 -> oct_optical_flow, src/oct_optical_flow.cc:21);
@@ -311,14 +318,24 @@ int octane_pix2uv_band_dev(octane_ctx* ctx, const octane_nav* nav, double t1, do
  * until that pair's outputs are in host memory.  Two pairs may be in flight (slot 0 / 1), so the copies of one
  * pair run under the solve of the other.  Host buffers must be pinned for the overlap to happen and stay valid
  * until the wait returns.  img*: rows [in0,in1) of octane_band_plan (the whole scene on one GPU); every output:
- * rows [own0,own1).  upix/vpix may both be NULL (the reference writes them only with -pd).  No first guess, no
- * -srsal here.  In banded runs every rank submits the same sequence; there a pair's copy-out is enqueued by the NEXT
+ * rows [own0,own1).  upix/vpix may both be NULL (the reference writes them only with -pd).  p->dosrsal needs cth_own
+ * and upix/vpix: as in octane_optical_flow the navigation runs on the unsmoothed flow and -srsal then smooths the
+ * pixel displacements (on row bands after an 18-row exchange with the neighbours, as octane_srsal_band_dev; every
+ * band must be at least 18 rows high).  A first guess goes through octane_stream_submit_fg; here p->first_guess is
+ * OCTANE_EINVAL.  In banded runs every rank submits the same sequence; there a pair's copy-out is enqueued by the NEXT
  * submit, to start when that pair's solve reaches its finest level (a device-to-host copy in flight slows the
  * system-scope fences of the short coarse-level iterations), or by octane_stream_wait if no submit followed.
  * Returns 1 when the sector-moved guard zeroed the navigated outputs. */
 int octane_stream_submit(octane_ctx* ctx, int slot, const float* img1_band, const float* img2_band, const float* cth_own,
                          int nx, int ny, int nc, const octane_nav* nav, double t1, double t2, const octane_params* p,
                          float* upix_own, float* vpix_own, short* U, short* V, short* U_raw, short* V_raw, short* ctp_own);
+/* The same with a first guess (p->first_guess = 1, optionally p->lambdac): fg_u_band / fg_v_band are host rows
+ * [in0,in1) of the first-guess displacement field, like the images (and like octane_variational_flow_band_fg_dev);
+ * they are only read, and must stay valid until the wait returns.  upix/vpix receive the flow. */
+int octane_stream_submit_fg(octane_ctx* ctx, int slot, const float* img1_band, const float* img2_band,
+                            const float* fg_u_band, const float* fg_v_band, const float* cth_own, int nx, int ny, int nc,
+                            const octane_nav* nav, double t1, double t2, const octane_params* p,
+                            float* upix_own, float* vpix_own, short* U, short* V, short* U_raw, short* V_raw, short* ctp_own);
 int octane_stream_wait(octane_ctx* ctx, int slot);
 
 #ifdef __cplusplus

@@ -70,7 +70,7 @@ EXPORTS = [
     "octane_stage_build", "octane_stage_pcg",
     "octane_band_plan", "octane_comm_unique_id", "octane_comm_init", "octane_comm_rank",
     "octane_variational_flow_band_dev", "octane_variational_flow_band_fg_dev", "octane_pix2uv_band_dev",
-    "octane_stream_submit", "octane_stream_wait",
+    "octane_srsal_band_dev", "octane_stream_submit", "octane_stream_submit_fg", "octane_stream_wait",
 ]
 
 _lib = None
@@ -141,7 +141,9 @@ def load() -> C.CDLL:
     L.octane_variational_flow_band_dev.argtypes = [vp, vp, vp, i, i, i, PP, vp, vp]
     L.octane_variational_flow_band_fg_dev.argtypes = [vp, vp, vp, vp, vp, i, i, i, PP, vp, vp]
     L.octane_pix2uv_band_dev.argtypes = [vp, NP, d, d, vp, vp, i, i, i, PP, vp, vp, vp, vp]
+    L.octane_srsal_band_dev.argtypes = [vp, vp, vp, vp, i, i]
     L.octane_stream_submit.argtypes = [vp, i, vp, vp, vp, i, i, i, NP, d, d, PP, vp, vp, vp, vp, vp, vp, vp]
+    L.octane_stream_submit_fg.argtypes = [vp, i, vp, vp, vp, vp, vp, i, i, i, NP, d, d, PP, vp, vp, vp, vp, vp, vp, vp]
     L.octane_stream_wait.argtypes = [vp, i]
     _lib = L
     return L

@@ -288,6 +288,16 @@ class Context:
         self._before_torch()
         return rc
 
+    def oct_srsal_band(self, u_own, v_own, cth_own, nx: int, ny: int):
+        """-srsal on row bands (collective), in place on torch CUDA tensors holding the owned rows [own0,own1) of
+        band_plan(); cth_own: the same rows of the cloud-top heights.  At world size 1: oct_srsal_cu."""
+        for name, a in (("u_own", u_own), ("v_own", v_own), ("cth_own", cth_own)):
+            _require(name, a, "float32", cuda=True)
+        self._after_torch()
+        self._check(self._L.octane_srsal_band_dev(self._h, _ptr(u_own), _ptr(v_own), _ptr(cth_own), nx, ny))
+        self._before_torch()
+        return u_own, v_own
+
     def oct_optical_flow(self, geo1, geo2, nav: Nav, t1: float, t2: float, p: Optional[Params] = None,
                          cth=None, upix=None, vpix=None, nc: int = 1, out=None):
         """Dispatcher (host arrays): returns dict(uPix, vPix, uVal, vVal, uVal2, vVal2, CTP, dT).
@@ -337,21 +347,24 @@ class Context:
 
     # ---- pipelined dispatcher over a sequence of pairs (host buffers, ideally pinned)
     def stream_submit(self, slot: int, geo1_band, geo2_band, nav: Nav, t1: float, t2: float, p: Params, out: dict,
-                      nx: int, ny: int, cth=None, nc: int = 1) -> int:
-        """enqueue copy-in -> solve -> navigation -> copy-out of one pair and return.  geo*_band: rows [in0,in1) of
-        band_plan() (the whole scene on one GPU); `out`: host arrays for rows [own0,own1) under the keys uVal, vVal,
-        uVal2, vVal2 (int16) and optionally uPix, vPix (float32), CTP (int16).  The arrays must stay alive and untouched
-        until stream_wait(slot)."""
+                      nx: int, ny: int, cth=None, nc: int = 1, *, fg_u_band=None, fg_v_band=None) -> int:
+        """enqueue copy-in -> solve -> navigation (-> -srsal) -> copy-out of one pair and return.  geo*_band: rows
+        [in0,in1) of band_plan() (the whole scene on one GPU); `out`: host arrays for rows [own0,own1) under the keys
+        uVal, vVal, uVal2, vVal2 (int16) and optionally uPix, vPix (float32), CTP (int16).  cth: rows [own0,own1) of the
+        cloud-top heights (doCTH, dosrsal; dosrsal also needs uPix / vPix).  fg_u_band / fg_v_band: rows [in0,in1) of a
+        first guess (p.first_guess), only read.  The arrays must stay alive and untouched until stream_wait(slot)."""
         for name, a in (("geo1_band", geo1_band), ("geo2_band", geo2_band), ("cth", cth), ("uPix", out.get("uPix")),
-                        ("vPix", out.get("vPix"))):
+                        ("vPix", out.get("vPix")), ("fg_u_band", fg_u_band), ("fg_v_band", fg_v_band)):
             _require(name, a, "float32", cuda=False)
         for name in ("uVal", "vVal", "uVal2", "vVal2"):
             _require(name, out[name], "int16", cuda=False)
         _require("CTP", out.get("CTP"), "int16", cuda=False)
-        return self._check(self._L.octane_stream_submit(self._h, slot, _ptr(geo1_band), _ptr(geo2_band), _ptr(cth), nx, ny, nc,
-                                                        C.byref(nav), t1, t2, C.byref(p), _ptr(out.get("uPix")),
-                                                        _ptr(out.get("vPix")), _ptr(out["uVal"]), _ptr(out["vVal"]),
-                                                        _ptr(out["uVal2"]), _ptr(out["vVal2"]), _ptr(out.get("CTP"))))
+        tail = (nx, ny, nc, C.byref(nav), t1, t2, C.byref(p), _ptr(out.get("uPix")), _ptr(out.get("vPix")),
+                _ptr(out["uVal"]), _ptr(out["vVal"]), _ptr(out["uVal2"]), _ptr(out["vVal2"]), _ptr(out.get("CTP")))
+        if fg_u_band is not None or fg_v_band is not None:
+            return self._check(self._L.octane_stream_submit_fg(self._h, slot, _ptr(geo1_band), _ptr(geo2_band),
+                                                               _ptr(fg_u_band), _ptr(fg_v_band), _ptr(cth), *tail))
+        return self._check(self._L.octane_stream_submit(self._h, slot, _ptr(geo1_band), _ptr(geo2_band), _ptr(cth), *tail))
 
     def stream_wait(self, slot: int):
         self._check(self._L.octane_stream_wait(self._h, slot))

@@ -188,6 +188,7 @@ struct octane_ctx {
     // small persistent device objects
     PcgScalars* d_scal = nullptr;
     double* d_pending = nullptr;
+    double* d_vote = nullptr;      // banded runs: one double for the all-ranks vote of octane_srsal_band_dev
     unsigned* d_ticket = nullptr;
     double* d_partials = nullptr;
     int partial_blocks = 0;
@@ -934,6 +935,7 @@ void octane_ctx_destroy(octane_ctx* c)
     if (c->stage) cudaFree(c->stage);
     if (c->d_scal) cudaFree(c->d_scal);
     if (c->d_pending) cudaFree(c->d_pending);
+    if (c->d_vote) cudaFree(c->d_vote);
     if (c->d_ticket) cudaFree(c->d_ticket);
     if (c->d_partials) cudaFree(c->d_partials);
     if (c->d_its) cudaFree(c->d_its);
@@ -1099,6 +1101,9 @@ int octane_pix2uv_band_dev(octane_ctx* c, const octane_nav* nav, double t1, doub
 namespace {
 constexpr int SRSAL_R = 18;    // radius of the -srsal window (src/oct_srsal_cuda.cu:78-79)
 int srsal_enqueue(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int nx, int ny, float* tmp_u, float* tmp_v);
+size_t srsal_band_stage_bytes(int nx, int ny, int own0, int own1);
+int srsal_band_enqueue(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int nx, int ny, int own0, int own1, char* stage);
+bool srsal_bands_ok(int ny, int world);
 bool srsal_args_ok(const octane_params* p, const void* cth, int nx, int ny)
 {
     if (!p->dosrsal) return true;
@@ -1483,7 +1488,7 @@ int srsal_enqueue(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int
     SrsalTaps t;
     srsal_taps(&t);
     const size_t fb = (size_t)nx * ny * sizeof(float);
-    launch_srsal(d_u, d_v, d_cth, nx, ny, t, tmp_u, tmp_v, c->stream);
+    launch_srsal(d_u, d_v, d_cth, nx, ny, 0, 0, ny, t, tmp_u, tmp_v, c->stream);
     c->launches++;
     CUDA_OK(cudaGetLastError());
     CUDA_OK(cudaMemcpyAsync(d_u, tmp_u, fb, cudaMemcpyDeviceToDevice, c->stream));
@@ -1501,6 +1506,100 @@ int octane_srsal_dev(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, 
     int rc = ensure_stage(c, 2 * fb);
     if (rc) return rc;
     return srsal_enqueue(c, d_u, d_v, d_cth, nx, ny, (float*)c->stage, (float*)(c->stage + fb));
+}
+
+// ---- -srsal on row bands ------------------------------------------------------------------------
+// Rank r owns rows [r*ny/world, (r+1)*ny/world), the finest level's rule of make_plan.  The 37 x 37 window of an owned
+// row reaches 18 rows into each neighbour's band; the window of a row near the scene edge reflects back into the scene
+// (rows 1..18 above row 0, ny-18..ny-1 below row ny-1).  With every band at least 18 rows high both come from this
+// band and the two adjacent ones only: each rank stages u, v, cth over rows [max(0, own0-18), min(ny, own1+18)) and
+// takes the 18 rows above and below from its neighbours in one NCCL exchange.
+namespace {
+void own_rows(int ny, int rank, int world, int* own0, int* own1)
+{
+    *own0 = (int)((long long)rank * ny / world);
+    *own1 = (int)((long long)(rank + 1) * ny / world);
+}
+
+// the same answer on every rank (it depends on ny and world only): all refuse together, none enters the exchange alone
+bool srsal_bands_ok(int ny, int world)
+{
+    for (int r = 0; r < world; r++) {
+        int a, b;
+        own_rows(ny, r, world, &a, &b);
+        if (b - a < SRSAL_R) return false;
+    }
+    return true;
+}
+
+// three planes (u, v, cth) of the extended rows
+size_t srsal_band_stage_bytes(int nx, int ny, int own0, int own1)
+{
+    const int e0 = own0 - SRSAL_R < 0 ? 0 : own0 - SRSAL_R, e1 = own1 + SRSAL_R > ny ? ny : own1 + SRSAL_R;
+    return 3 * align_up((size_t)(e1 - e0) * nx * sizeof(float));
+}
+
+// d_u, d_v, d_cth: the owned rows [own0,own1), dense; stage: srsal_band_stage_bytes.  Collective on the context's
+// communicator (nothing is exchanged at world 1); the result goes back into d_u, d_v.
+int srsal_band_enqueue(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int nx, int ny, int own0, int own1, char* stage)
+{
+    const int e0 = own0 - SRSAL_R < 0 ? 0 : own0 - SRSAL_R, e1 = own1 + SRSAL_R > ny ? ny : own1 + SRSAL_R;
+    const size_t pb = align_up((size_t)(e1 - e0) * nx * sizeof(float)), ob = (size_t)(own1 - own0) * nx * sizeof(float);
+    float* ext[3] = { (float*)stage, (float*)(stage + pb), (float*)(stage + 2 * pb) };
+    const float* own[3] = { d_u, d_v, d_cth };
+    const size_t at_own = (size_t)(own0 - e0) * nx;
+    for (int p = 0; p < 3; p++)
+        CUDA_OK(cudaMemcpyAsync(ext[p] + at_own, own[p], ob, cudaMemcpyDeviceToDevice, c->stream));
+    if (c->comm.world > 1) {
+        // interior cuts have 18 rows of staging on both sides (every band >= 18 rows); the outermost ranks have no
+        // neighbour there and comm_halo_exchange skips those pointers
+        const bool has_up = c->comm.rank > 0, has_dn = c->comm.rank + 1 < c->comm.world;
+        float *su[3], *ru[3], *sd[3], *rd[3];
+        for (int p = 0; p < 3; p++) {
+            su[p] = ext[p] + at_own;                                                // my first 18 rows -> rank-1
+            ru[p] = has_up ? ext[p] : nullptr;                                      // rank-1's last 18 rows (e0 = own0-18)
+            sd[p] = ext[p] + (size_t)(own1 - SRSAL_R - e0) * nx;                    // my last 18 rows -> rank+1
+            rd[p] = has_dn ? ext[p] + (size_t)(own1 - e0) * nx : nullptr;           // rank+1's first 18 rows
+        }
+        if (comm_halo_exchange(&c->comm, 3, su, ru, sd, rd, (size_t)SRSAL_R * nx, c->stream)) {
+            set_err("%s", comm_last_error());
+            return OCTANE_ECOMM;
+        }
+    }
+    SrsalTaps t;
+    srsal_taps(&t);
+    launch_srsal(ext[0], ext[1], ext[2], nx, ny, e0, own0, own1, t, d_u, d_v, c->stream);
+    c->launches++;
+    CUDA_OK(cudaGetLastError());
+    return OCTANE_OK;
+}
+}  // namespace
+
+int octane_srsal_band_dev(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int nx, int ny)
+{
+    if (!c || !d_u || !d_v || !d_cth || nx <= SRSAL_R || ny <= SRSAL_R) { set_err("null or invalid argument"); return OCTANE_EINVAL; }
+    const int world = c->comm.world;
+    if (world <= 1) return octane_srsal_dev(c, d_u, d_v, d_cth, nx, ny);
+    if (!srsal_bands_ok(ny, world)) {
+        set_err("-srsal on row bands needs every band at least 18 rows high: fewer ranks or a taller scene");
+        return OCTANE_EINVAL;
+    }
+    CUDA_OK(cudaSetDevice(c->device));
+    int own0, own1;
+    own_rows(ny, c->comm.rank, world, &own0, &own1);
+    // the staging is the only step that can fail on one rank alone: vote on it before the exchange, so that a rank
+    // without memory returns an error on every rank instead of leaving its peers waiting in the exchange
+    int local = ensure_stage(c, srsal_band_stage_bytes(nx, ny, own0, own1));
+    if (local) cudaGetLastError();          // a failed allocation is not a sticky error: keep it out of later checks
+    const double mine = local ? 0.0 : 1.0;
+    double all = 0.0;
+    CUDA_OK(cudaMemcpyAsync(c->d_vote, &mine, sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    if (comm_allreduce_f64(&c->comm, c->d_vote, 1, c->stream)) { set_err("%s", comm_last_error()); return OCTANE_ECOMM; }
+    CUDA_OK(cudaMemcpyAsync(&all, c->d_vote, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CUDA_OK(cudaStreamSynchronize(c->stream));
+    if (local) return local;
+    if (all != (double)world) { set_err("-srsal on row bands: a peer could not allocate its staging"); return OCTANE_ENOMEM; }
+    return srsal_band_enqueue(c, d_u, d_v, d_cth, nx, ny, own0, own1, c->stage);
 }
 
 int octane_srsal(octane_ctx* c, float* u, float* v, const float* cth, int nx, int ny)
@@ -1617,6 +1716,8 @@ int octane_comm_init(octane_ctx* c, const char id[128], int rank, int world)
     destroy_graphs(c);
     comm_destroy(&c->comm);
     if (world == 1) return OCTANE_OK;
+    // allocated once, before any collective: the vote of a later call must not itself need an allocation
+    if (!c->d_vote) CUDA_OK(cudaMalloc(&c->d_vote, sizeof(double)));
     if (comm_init(&c->comm, id, rank, world)) { set_err("%s", comm_last_error()); return OCTANE_ECOMM; }
     // per-iteration exchanges over peer memory when every rank can map its peers (else NCCL)
     if (comm_p2p_init(&c->comm, sizeof(P2PWindow), c->stream)) { set_err("%s", comm_last_error()); return OCTANE_ECOMM; }
@@ -1661,22 +1762,36 @@ int slot_prepare(octane_ctx* c, int k, size_t bytes)
 }
 }  // namespace
 
-int octane_stream_submit(octane_ctx* c, int k, const float* img1, const float* img2, const float* cth, int nx, int ny, int nc,
-                         const octane_nav* nav, double t1, double t2, const octane_params* p, float* upix, float* vpix,
-                         short* U, short* V, short* Ur, short* Vr, short* ctp)
+namespace {
+// octane_stream_submit and octane_stream_submit_fg: fg_u / fg_v are host rows [in0,in1) of the first guess, read only
+// when p->first_guess (the callers check which of the two may set it)
+int stream_submit(octane_ctx* c, int k, const float* img1, const float* img2, const float* fg_u, const float* fg_v,
+                  const float* cth, int nx, int ny, int nc, const octane_nav* nav, double t1, double t2,
+                  const octane_params* p, float* upix, float* vpix, short* U, short* V, short* Ur, short* Vr, short* ctp)
 {
     if (!c || (k != 0 && k != 1) || !img1 || !img2 || !nav || !p || !U || !V || !Ur || !Vr || (!upix != !vpix)) {
         set_err("null or invalid argument");
         return OCTANE_EINVAL;
     }
     if (p->doCTH && (!cth || !ctp)) { set_err("doCTH needs cth and ctp"); return OCTANE_EINVAL; }
-    if (p->first_guess || p->dosrsal) { set_err("the pipelined dispatcher takes neither a first guess nor -srsal"); return OCTANE_EINVAL; }
+    if (!srsal_args_ok(p, cth, nx, ny)) return OCTANE_EINVAL;
+    // -srsal changes the pixel displacements only (src/oct_optical_flow.cc:91-105): a submit that does not ask for them
+    // would smooth nothing it returns
+    if (p->dosrsal && !upix) { set_err("dosrsal smooths upix / vpix only: the pipelined dispatcher needs them"); return OCTANE_EINVAL; }
+    if (p->dosrsal && !srsal_bands_ok(ny, c->comm.world)) {
+        set_err("-srsal on row bands needs every band at least 18 rows high: fewer ranks or a taller scene");
+        return OCTANE_EINVAL;
+    }
     CUDA_OK(cudaSetDevice(c->device));
     int rc = prepare(c, nx, ny, nc, *p);
     if (rc) return rc;
     const Level& F = c->plan.lv.back();
+    const bool banded = c->comm.world > 1;
     const size_t nin = (size_t)F.g.rows * nx, nown = (size_t)(F.own1 - F.own0) * nx;
     const size_t ib = align_up(nin * nc * sizeof(float)), fb = align_up(nown * sizeof(float)), sb = align_up(nown * sizeof(short));
+    const size_t gb = p->first_guess ? align_up(nin * sizeof(float)) : 0;
+    // -srsal staging: two result planes on one GPU, the three extended planes of the band otherwise
+    const size_t rb = !p->dosrsal ? 0 : banded ? srsal_band_stage_bytes(nx, ny, F.own0, F.own1) : 2 * fb;
     auto& sl = c->slot[k];
     if (sl.busy) {                       // resubmitting a slot implies its previous pair is finished with
         rc = flush_copy_out(c, k, false);
@@ -1684,7 +1799,7 @@ int octane_stream_submit(octane_ctx* c, int k, const float* img1, const float* i
         CUDA_OK(cudaEventSynchronize(sl.done));
         sl.busy = false;
     }
-    rc = slot_prepare(c, k, 2 * ib + 3 * fb + 5 * sb);
+    rc = slot_prepare(c, k, 2 * ib + 3 * fb + 5 * sb + 2 * gb + rb);
     if (rc) return rc;
     // When does the copy-out of a pair run?  On one GPU right after its navigation, under the next pair's solve.
     // In a banded run the peer-memory exchanges of every PCG iteration end in system-scope fences, and those take
@@ -1693,7 +1808,7 @@ int octane_stream_submit(octane_ctx* c, int k, const float* img1, const float* i
     // long and the iterations under the copy are few -- not under the hundreds of short coarse-level iterations a
     // solve starts with.  wait() enqueues it at once if no later submit() has.
     static const int defer_env = getenv("OCTANE_STREAM_DEFER") ? atoi(getenv("OCTANE_STREAM_DEFER")) : -1;   // developer switch
-    const bool defer = defer_env >= 0 ? defer_env != 0 : c->comm.world > 1;
+    const bool defer = defer_env >= 0 ? defer_env != 0 : banded;
     c->copy_out_at_finest = (defer && c->slot[k ^ 1].copy_pending) ? (k ^ 1) : -1;
     char* q = sl.buf;
     float* d_i1 = (float*)q; q += ib;
@@ -1701,12 +1816,19 @@ int octane_stream_submit(octane_ctx* c, int k, const float* img1, const float* i
     float* d_u = (float*)q; q += fb;
     float* d_v = (float*)q; q += fb;
     float* d_cth = (float*)q; q += fb;
-    short* d_s = (short*)q;
+    short* d_s = (short*)q; q += 5 * sb;
+    float* d_fgu = p->first_guess ? (float*)q : nullptr; q += gb;
+    float* d_fgv = p->first_guess ? (float*)q : nullptr; q += gb;
+    char* d_srsal = q;
     const size_t sstride = sb / sizeof(short);
     // copy-in on its own stream: runs under the solve of the pair in the other slot
     CUDA_OK(cudaMemcpyAsync(d_i1, img1, nin * nc * sizeof(float), cudaMemcpyHostToDevice, c->h2d_stream));
     CUDA_OK(cudaMemcpyAsync(d_i2, img2, nin * nc * sizeof(float), cudaMemcpyHostToDevice, c->h2d_stream));
-    if (p->doCTH) CUDA_OK(cudaMemcpyAsync(d_cth, cth, nown * sizeof(float), cudaMemcpyHostToDevice, c->h2d_stream));
+    if (p->first_guess) {
+        CUDA_OK(cudaMemcpyAsync(d_fgu, fg_u, nin * sizeof(float), cudaMemcpyHostToDevice, c->h2d_stream));
+        CUDA_OK(cudaMemcpyAsync(d_fgv, fg_v, nin * sizeof(float), cudaMemcpyHostToDevice, c->h2d_stream));
+    }
+    if (p->doCTH || p->dosrsal) CUDA_OK(cudaMemcpyAsync(d_cth, cth, nown * sizeof(float), cudaMemcpyHostToDevice, c->h2d_stream));
     CUDA_OK(cudaEventRecord(sl.in_ready, c->h2d_stream));
     // solve + navigation on the context's stream
     begin_call(c);
@@ -1714,7 +1836,7 @@ int octane_stream_submit(octane_ctx* c, int k, const float* img1, const float* i
     CUDA_OK(cudaStreamWaitEvent(c->stream, sl.in_ready, 0));
     {
         Scope total(c, CAT_TOTAL);
-        rc = ingest(c, d_i1, d_i2, nullptr, nullptr);
+        rc = ingest(c, d_i1, d_i2, d_fgu, d_fgv);
         if (rc) return rc;
         CUDA_OK(cudaEventRecord(sl.in_free, c->stream));
         rc = run_levels(c);
@@ -1729,6 +1851,11 @@ int octane_stream_submit(octane_ctx* c, int k, const float* img1, const float* i
     const int nrc = pix2uv_dev_rows(c, nav, t1, t2, d_u, d_v, nx, F.own0, F.own1 - F.own0, p, d_s, d_s + sstride,
                                     d_s + 2 * sstride, d_s + 3 * sstride);
     if (nrc < 0) return nrc;
+    if (p->dosrsal) {      // src/oct_optical_flow.cc:100-105: after the navigation, so only uPix / vPix are smoothed
+        rc = banded ? srsal_band_enqueue(c, d_u, d_v, d_cth, nx, ny, F.own0, F.own1, d_srsal)
+                    : srsal_enqueue(c, d_u, d_v, d_cth, nx, ny, (float*)d_srsal, (float*)(d_srsal + fb));
+        if (rc) return rc;
+    }
     CUDA_OK(cudaEventRecord(sl.out_ready, c->stream));
     // copy-out
     sl.ncopy = 0;
@@ -1746,6 +1873,25 @@ int octane_stream_submit(octane_ctx* c, int k, const float* img1, const float* i
     }
     if (!defer) { rc = flush_copy_out(c, k, false); if (rc) return rc; }
     return nrc;
+}
+
+}  // namespace
+
+int octane_stream_submit(octane_ctx* c, int k, const float* img1, const float* img2, const float* cth, int nx, int ny, int nc,
+                         const octane_nav* nav, double t1, double t2, const octane_params* p, float* upix, float* vpix,
+                         short* U, short* V, short* Ur, short* Vr, short* ctp)
+{
+    if (p && p->first_guess) { set_err("the pipelined dispatcher takes a first guess through octane_stream_submit_fg"); return OCTANE_EINVAL; }
+    return stream_submit(c, k, img1, img2, nullptr, nullptr, cth, nx, ny, nc, nav, t1, t2, p, upix, vpix, U, V, Ur, Vr, ctp);
+}
+
+int octane_stream_submit_fg(octane_ctx* c, int k, const float* img1, const float* img2, const float* fg_u, const float* fg_v,
+                            const float* cth, int nx, int ny, int nc, const octane_nav* nav, double t1, double t2,
+                            const octane_params* p, float* upix, float* vpix, short* U, short* V, short* Ur, short* Vr, short* ctp)
+{
+    if (p && !p->first_guess) { set_err("octane_stream_submit_fg needs p->first_guess"); return OCTANE_EINVAL; }
+    if (!fg_u || !fg_v) { set_err("octane_stream_submit_fg: no first guess was given"); return OCTANE_EINVAL; }
+    return stream_submit(c, k, img1, img2, fg_u, fg_v, cth, nx, ny, nc, nav, t1, t2, p, upix, vpix, U, V, Ur, Vr, ctp);
 }
 
 int octane_stream_wait(octane_ctx* c, int k)

@@ -160,7 +160,9 @@ struct SrsalTaps {
     double gk[37];
     double sigpix2;
 };
-void launch_srsal(const float* u, const float* v, const float* cth, int nx, int ny, const SrsalTaps& t,
-                  float* u_out, float* v_out, cudaStream_t st);
+// u, v, cth: dense rows [e0, ...) of the scene; u_out, v_out: dense rows [o0, o1).  Every row the window of an
+// output row reads (after reflection at the scene edges 0 and ny) must be present in the inputs.
+void launch_srsal(const float* u, const float* v, const float* cth, int nx, int ny, int e0, int o0, int o1,
+                  const SrsalTaps& t, float* u_out, float* v_out, cudaStream_t st);
 
 }  // namespace octane

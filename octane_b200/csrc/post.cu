@@ -14,6 +14,10 @@
 // a1 = GK[kc]*GK[lc]*exp(d*d*sigpix2) with d the FLOAT difference of the two heights widened to
 // double (:52,56-57), default FMA contraction of `au += u * a1`, result narrowed to float by the
 // host copy-back (:139-143).  The taps are computed on the host like the reference's (glibc exp).
+//
+// Row window (banded runs): the input planes hold global rows [e0, ...), the output planes global rows
+// [o0, o1).  The reflecting index stays in global coordinates (the scene edges are the edges of the whole
+// scene, not of a band); e0 is subtracted only when addressing.  One GPU: e0 = o0 = 0, o1 = ny.
 #include "kernels.cuh"
 
 namespace octane {
@@ -33,22 +37,22 @@ __device__ __forceinline__ int reflect(int x, int nx)
 
 __global__ void __launch_bounds__(TX * TY)
 k_srsal(const float* __restrict__ u, const float* __restrict__ v, const float* __restrict__ cth, int nx, int ny,
-        SrsalTaps t, float* __restrict__ u_out, float* __restrict__ v_out)
+        int e0, int o0, int o1, SrsalTaps t, float* __restrict__ u_out, float* __restrict__ v_out)
 {
     __shared__ float s_c[SH][SW], s_u[SH][SW], s_v[SH][SW];
-    const int i0 = blockIdx.x * TX, j0 = blockIdx.y * TY;
+    const int i0 = blockIdx.x * TX, j0 = o0 + blockIdx.y * TY;
     for (int k = threadIdx.y * TX + threadIdx.x; k < SW * SH; k += TX * TY) {
         const int sy = k / SW, sx = k - sy * SW;
-        // pixels beyond the scene in a partial tile are never read by a thread that stores
-        const int gi = reflect(min(i0 + sx - SR, nx - 1 + SR), nx), gj = reflect(min(j0 + sy - SR, ny - 1 + SR), ny);
-        const size_t at = (size_t)gi + (size_t)gj * nx;
+        // pixels beyond the scene (the window) in a partial tile are never read by a thread that stores
+        const int gi = reflect(min(i0 + sx - SR, nx - 1 + SR), nx), gj = reflect(min(j0 + sy - SR, o1 - 1 + SR), ny);
+        const size_t at = (size_t)gi + (size_t)(gj - e0) * nx;
         s_c[sy][sx] = cth[at];
         s_u[sy][sx] = u[at];
         s_v[sy][sx] = v[at];
     }
     __syncthreads();
     const int ic = i0 + threadIdx.x, jc = j0 + threadIdx.y;
-    if (ic >= nx || jc >= ny) return;
+    if (ic >= nx || jc >= o1) return;
     const float pixc = s_c[threadIdx.y + SR][threadIdx.x + SR];
     double au = 0, av = 0, a2 = 0;
     for (int kc = 0; kc < 2 * SR + 1; kc++) {
@@ -61,17 +65,17 @@ k_srsal(const float* __restrict__ u, const float* __restrict__ v, const float* _
             av += (double)s_v[threadIdx.y + lc][threadIdx.x + kc] * a1;
         }
     }
-    const size_t at = (size_t)ic + (size_t)jc * nx;
+    const size_t at = (size_t)ic + (size_t)(jc - o0) * nx;
     u_out[at] = (au / a2);
     v_out[at] = (av / a2);
 }
 }  // namespace
 
-void launch_srsal(const float* u, const float* v, const float* cth, int nx, int ny, const SrsalTaps& t,
-                  float* u_out, float* v_out, cudaStream_t st)
+void launch_srsal(const float* u, const float* v, const float* cth, int nx, int ny, int e0, int o0, int o1,
+                  const SrsalTaps& t, float* u_out, float* v_out, cudaStream_t st)
 {
-    dim3 grid((nx + TX - 1) / TX, (ny + TY - 1) / TY), block(TX, TY);
-    k_srsal<<<grid, block, 0, st>>>(u, v, cth, nx, ny, t, u_out, v_out);
+    dim3 grid((nx + TX - 1) / TX, (o1 - o0 + TY - 1) / TY), block(TX, TY);
+    k_srsal<<<grid, block, 0, st>>>(u, v, cth, nx, ny, e0, o0, o1, t, u_out, v_out);
 }
 
 }  // namespace octane
