@@ -248,6 +248,23 @@ int octane_optical_flow_dev(octane_ctx* ctx, const float* d_img1, const float* d
                             int nx, int ny, int nc, const octane_nav* nav, double t1, double t2,
                             const octane_params* p, float* d_upix_inout, float* d_vpix_inout,
                             short* d_U, short* d_V, short* d_U_raw, short* d_V_raw, short* d_ctp);
+/* Many same-size pairs in one call: each pair is solved, its CTP packed and its flow navigated exactly as
+ * octane_optical_flow_dev does, with one launch per stage for the whole batch.  Arrays are dense and pair-major:
+ * images npairs x nc x ny x nx, d_cth and every output npairs x ny x nx; nav, t1 and t2 are host arrays of npairs.
+ * Small pyramid levels solve all pairs in one cooperative launch (each pair on its own group of blocks, with its own
+ * barrier and stop rule); a pair's result does not depend on the other pairs of the call.  Stream-ordered, no host
+ * synchronisation; moved_out (host, npairs, may be NULL) gets 1 for each pair whose sector moved (its four short
+ * planes are zero).  OCTANE_EINVAL for npairs < 1, a first guess, dosrsal or a banded context; OCTANE_ENOMEM when
+ * the npairs workspaces do not fit.  The context stays usable after either.  octane_get_stats then reports the
+ * call's kernel launches and pair 0's iteration counts. */
+int octane_optical_flow_batch_dev(octane_ctx* ctx, int npairs, const float* d_img1, const float* d_img2,
+                                  const float* d_cth, int nx, int ny, int nc, const octane_nav* nav,
+                                  const double* t1, const double* t2, const octane_params* p,
+                                  float* d_upix, float* d_vpix, short* d_U, short* d_V, short* d_U_raw,
+                                  short* d_V_raw, short* d_ctp, int* moved_out);
+/* PCG iterations of every solve of every pair of the last batched call: its[pair * n_solves + solve].  npairs must
+ * be that call's.  Synchronises the context's stream. */
+int octane_batch_cg_iterations(octane_ctx* ctx, int* its, int npairs);
 
 int octane_navcal_dev(octane_ctx* ctx, const short* d_rad, const short* d_x, const short* d_y, int nx, int ny,
                       const octane_nav* nav, const octane_cal* cal, float* d_data, float* d_lat, float* d_lon);

@@ -345,6 +345,41 @@ class Context:
             self._before_torch()
         return rc
 
+    def oct_optical_flow_batch_dev(self, geo1, geo2, nav_list, t1_list, t2_list, p: Params, out: dict, cth=None,
+                                   nc: int = 1):
+        """Many same-size pairs in one call, on torch CUDA tensors shaped [B, ny, nx] (or [B, nc, ny, nx] for the
+        images).  `out` holds [B, ny, nx] tensors under uPix, vPix (float32), uVal, vVal, uVal2, vVal2 and, with
+        doCTH, CTP (int16).  Stream-ordered like oct_optical_flow_dev.  Returns the list of pairs whose sector moved
+        (their four navigated planes are zero); cg_iterations() gives the per-pair iteration counts."""
+        B = int(geo1.shape[0])
+        ny, nx = geo1.shape[-2:]
+        for name, a in (("geo1", geo1), ("geo2", geo2), ("cth", cth), ("uPix", out.get("uPix")), ("vPix", out.get("vPix"))):
+            _require(name, a, "float32", cuda=True)
+        for name in ("uVal", "vVal", "uVal2", "vVal2", "CTP"):
+            _require(name, out.get(name), "int16", cuda=True)
+        shapes = {tuple(a.shape[-2:]) for a in (geo2, cth, *out.values()) if a is not None}
+        if shapes != {(ny, nx)} or any(int(a.shape[0]) != B for a in (geo2, cth, *out.values()) if a is not None):
+            raise ValueError("every array must be [B, ny, nx] (images [B, nc, ny, nx]) with the same B, ny, nx")
+        if not (len(nav_list) == len(t1_list) == len(t2_list) == B):
+            raise ValueError("nav_list, t1_list and t2_list need one entry per pair")
+        navs = (Nav * max(B, 1))(*nav_list)
+        t1 = (C.c_double * max(B, 1))(*t1_list)
+        t2 = (C.c_double * max(B, 1))(*t2_list)
+        moved = (C.c_int * max(B, 1))()
+        self._after_torch()
+        self._check(self._L.octane_optical_flow_batch_dev(
+            self._h, B, _ptr(geo1), _ptr(geo2), _ptr(cth), nx, ny, nc, navs, t1, t2, C.byref(p), _ptr(out["uPix"]),
+            _ptr(out["vPix"]), _ptr(out["uVal"]), _ptr(out["vVal"]), _ptr(out["uVal2"]), _ptr(out["vVal2"]),
+            _ptr(out.get("CTP")), moved))
+        self._before_torch()
+        return [b for b in range(B) if moved[b]]
+
+    def batch_cg_iterations(self, npairs: int, n_solves: int) -> np.ndarray:
+        """[npairs, n_solves] PCG iterations of the last batched call (synchronises the context's stream)"""
+        its = np.zeros((npairs, n_solves), np.int32)
+        self._check(self._L.octane_batch_cg_iterations(self._h, its.ctypes.data_as(C.POINTER(C.c_int)), npairs))
+        return its
+
     # ---- pipelined dispatcher over a sequence of pairs (host buffers, ideally pinned)
     def stream_submit(self, slot: int, geo1_band, geo2_band, nav: Nav, t1: float, t2: float, p: Params, out: dict,
                       nx: int, ny: int, cth=None, nc: int = 1, *, fg_u_band=None, fg_v_band=None) -> int:

@@ -75,7 +75,7 @@ enum { GNC_QUADRATIC = 0, GNC_BLEND = 1, GNC_ROBUST = 2 };
 
 template <int MODE, int OCC>
 __global__ void __launch_bounds__(256, OCC)
-k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, BuildParams bp, int halo_check)
+k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, BuildParams bp, int halo_check, size_t ps)
 {
     constexpr bool ROBUST = (MODE != GNC_QUADRATIC);   // robust terms needed
     constexpr bool QUAD = (MODE != GNC_ROBUST);        // quadratic terms needed
@@ -85,6 +85,7 @@ k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, Bui
     const double alpha = bp.alpha, ralpha = bp.ralpha, lambdadalpha = bp.lambdadalpha, al1 = bp.al1;
     const float lambdac = bp.lambdac;
     double acc[2] = { 0.0, 0.0 };
+    const size_t po = (size_t)blockIdx.z * ps;         // pair blockIdx.z: every plane is ps floats further on
 
     // a block covers 32 columns x BUILD_ROWS rows, 8 rows at a time
     for (int jt = 0; jt < BUILD_ROWS; jt += 8) {
@@ -95,7 +96,7 @@ k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, Bui
         const int ip = (ii == xi - 1) ? ii - 1 : ii + 1;
         const int jm = (jj == 0) ? jj + 1 : jj - 1;
         const int jp = (jj == yi - 1) ? jj - 1 : jj + 1;
-        const size_t r0 = g.at(0, jj);
+        const size_t r0 = g.at(0, jj) + po;
         const float* u0 = f.u + r0;
         const float* v0 = f.v + r0;
         const int dm = (jm - jj) * pitch, dp = (jp - jj) * pitch;     // +-pitch
@@ -145,7 +146,7 @@ k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, Bui
                 jv1 = min(max(jv1, g.jlo()), g.jhi() - 2);
             }
         }
-        const size_t c1 = g.at(iv1, jv1);
+        const size_t c1 = g.at(iv1, jv1) + po;
         const size_t l = r0 + ii;
         // bilinear weights, :57-65; x2-x1 == y2-y1 == 1.0f exactly, so the divisions are dropped
         const float x1 = iv1, x2 = iv1 + 1, y1 = jv1, y2 = jv1 + 1;
@@ -264,20 +265,23 @@ k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, Bui
     block_sum<2>(acc, red);
     if (threadIdx.x == 0 && threadIdx.y == 0) {
         const unsigned nblocks = gridDim.x * gridDim.y, bid = blockIdx.y * gridDim.x + blockIdx.x;
-        b.partials[bid] = acc[0];
-        b.partials[(size_t)nblocks + bid] = acc[1];
+        double* part = b.partials + (size_t)blockIdx.z * 2 * nblocks;   // one region per pair
+        part[bid] = acc[0];
+        part[(size_t)nblocks + bid] = acc[1];
     }
 }
 
 // second stage of the build's dot products (fixed order) + PCG scalar seeding:
-// residc = b.b, rkTzk = b.z; stop rule already true -> no iterations (:1131).
+// residc = b.b, rkTzk = b.z; stop rule already true -> no iterations (:1131).  Pair blockIdx.z: its partials and
+// its scalars b.scal[blockIdx.z].
 __global__ void __launch_bounds__(1024) k_build_finish(PcgBuffers b, unsigned nblocks, float tol)
 {
     __shared__ double red[2 * 32];
     double acc[2] = { 0.0, 0.0 };
+    const double* part = b.partials + (size_t)blockIdx.z * 2 * nblocks;
     for (unsigned i = threadIdx.x; i < nblocks; i += 1024) {
-        acc[0] += b.partials[i];
-        acc[1] += b.partials[(size_t)nblocks + i];
+        acc[0] += part[i];
+        acc[1] += part[(size_t)nblocks + i];
     }
     block_sum<2>(acc, red);
     if (b.p2p.world > 1) p2p_allreduce<2>(b.p2p, P2P_BUILD, acc, &b.scal->comm_err);
@@ -285,7 +289,7 @@ __global__ void __launch_bounds__(1024) k_build_finish(PcgBuffers b, unsigned nb
         b.pending[0] = acc[0];
         b.pending[1] = acc[1];
     } else if (threadIdx.x == 0) {
-        PcgScalars* s = b.scal;
+        PcgScalars* s = b.scal + blockIdx.z;
         s->rr = (float)acc[0];
         s->rz = (float)acc[1];
         s->rz_old = 0.f;
@@ -298,15 +302,15 @@ __global__ void __launch_bounds__(1024) k_build_finish(PcgBuffers b, unsigned nb
 }
 
 void launch_build(const LevelFields& f, const PcgBuffers& b, const Geom& g, int ja, int jb, int da, int db,
-                  const BuildParams& bp, int halo_check, cudaStream_t st)
+                  const BuildParams& bp, int halo_check, cudaStream_t st, int npairs, size_t ps)
 {
-    dim3 grid((g.nx + 31) / 32, (jb - ja + BUILD_ROWS - 1) / BUILD_ROWS), block(32, 8);
-#define LAUNCH_BUILD(MODE) k_build<MODE, OCTANE_BUILD_OCC><<<grid, block, 0, st>>>(f, b, g, ja, jb, da, db, bp, halo_check)
+    dim3 grid((g.nx + 31) / 32, (jb - ja + BUILD_ROWS - 1) / BUILD_ROWS, npairs), block(32, 8);
+#define LAUNCH_BUILD(MODE) k_build<MODE, OCTANE_BUILD_OCC><<<grid, block, 0, st>>>(f, b, g, ja, jb, da, db, bp, halo_check, ps)
     if (bp.al1 == 1.0)      LAUNCH_BUILD(GNC_QUADRATIC);
     else if (bp.al1 == 0.0) LAUNCH_BUILD(GNC_ROBUST);
     else                    LAUNCH_BUILD(GNC_BLEND);
 #undef LAUNCH_BUILD
-    k_build_finish<<<1, 1024, 0, st>>>(b, grid.x * grid.y, bp.tol);
+    k_build_finish<<<dim3(1, 1, npairs), 1024, 0, st>>>(b, grid.x * grid.y, bp.tol);
 }
 
 int build_partial_blocks(const Geom& g, int nrows)

@@ -181,6 +181,17 @@ struct octane_ctx {
     // workspace
     char* arena = nullptr;
     size_t arena_bytes = 0;
+    int arena_pairs = 0;           // copies of the plan's workspace (one per pair of a batch) cleared since the re-plan
+    // batched calls (octane_optical_flow_batch_dev): per-pair scalars, partial sums, group barriers, iteration
+    // counts and navigation parameters, for up to batch_cap pairs
+    PcgScalars* d_bscal = nullptr;
+    double* d_bpart = nullptr;
+    size_t bpart_doubles = 0;
+    unsigned* d_bbar = nullptr;
+    int* d_bits = nullptr;
+    NavParams* d_bnav = nullptr;
+    int batch_cap = 0;
+    int batch_npairs = 0, batch_nsolves = 0;   // of the last batched call
     Plan plan;
     bool plan_valid = false;
     Buffers buf;
@@ -372,6 +383,7 @@ int prepare(octane_ctx* c, int nx, int ny, int nc, const octane_params& p)
     c->buf.pcg.p2p.epoch = c->comm.d_epoch;
     c->buf.pcg.up_ru = c->buf.pcg.up_rv = c->buf.pcg.dn_ru = c->buf.pcg.dn_rv = nullptr;
     c->plan = pl;
+    c->arena_pairs = 1;
     c->pcg_graph.assign(2 * pl.lv.size(), nullptr);
     c->plan_valid = true;
     return OCTANE_OK;
@@ -440,9 +452,9 @@ bool level_fused(const octane_ctx* c, const Level& L)
 }
 
 // ---- the PCG loop of one solve (:1129-1182), enqueued or captured ----------------------
-int enqueue_pcg(octane_ctx* c, const Level& L, int level, int solve, int const_wn)
+int enqueue_pcg(octane_ctx* c, const Level& L, int level, int solve, int const_wn, const PcgBuffers& pb)
 {
-    PcgBuffers b = c->buf.pcg;
+    PcgBuffers b = pb;
     const int iters = c->plan.p.cgiters;
     const bool multi = c->comm.world > 1;
     const bool p2p = multi && c->comm.p2p;
@@ -508,13 +520,13 @@ int run_pcg(octane_ctx* c, const Level& L, int level, int solve, int const_wn)
         cudaGetLastError();                              // e.g. a device that cannot co-schedule the grid: per-iteration launches
         c->coop = false;
     }
-    if (!c->graphs || c->profile) return enqueue_pcg(c, L, level, solve, const_wn);
+    if (!c->graphs || c->profile) return enqueue_pcg(c, L, level, solve, const_wn, c->buf.pcg);
     const size_t slot = 2 * (size_t)level + (const_wn ? 1 : 0);
     if (!c->pcg_graph[slot]) {
         cudaGraph_t graph = nullptr;
         const long long before = c->launches;
         CUDA_OK(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-        int rc = enqueue_pcg(c, L, level, solve, const_wn);
+        int rc = enqueue_pcg(c, L, level, solve, const_wn, c->buf.pcg);
         cudaError_t e = cudaStreamEndCapture(c->stream, &graph);
         c->launches = before;
         if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
@@ -941,6 +953,8 @@ void octane_ctx_destroy(octane_ctx* c)
     if (c->d_its) cudaFree(c->d_its);
     if (c->d_gk) cudaFree(c->d_gk);
     if (c->d_navtab) cudaFree(c->d_navtab);
+    for (void* q : { (void*)c->d_bscal, (void*)c->d_bpart, (void*)c->d_bbar, (void*)c->d_bits, (void*)c->d_bnav })
+        if (q) cudaFree(q);
     for (auto& sl : c->slot) {
         if (sl.done) cudaEventSynchronize(sl.done);
         if (sl.buf) cudaFree(sl.buf);
@@ -1137,6 +1151,244 @@ int octane_optical_flow_dev(octane_ctx* c, const float* d_img1, const float* d_i
     if (nrc < 0 || !p->dosrsal) return nrc;
     rc = srsal_enqueue(c, d_u, d_v, d_cth, nx, ny, (float*)c->stage, (float*)(c->stage + fb));   // :100-105
     return rc ? rc : nrc;
+}
+
+// ---- batched calls: many same-size pairs, one launch per stage -----------------------------------------------------
+namespace {
+// B copies of the plan's workspace at a fixed stride; pair 0 is the single-pair workspace.  A failed allocation
+// leaves the context as it was.
+int ensure_batch(octane_ctx* c, int npairs, size_t* stride)
+{
+    const Plan& pl = c->plan;
+    const size_t S = arena_layout(pl, nullptr, nullptr);
+    *stride = S;
+    const size_t need = S * (size_t)npairs;
+    if (need > c->arena_bytes) {
+        char* na = nullptr;
+        if (cudaMalloc(&na, need) != cudaSuccess) {
+            cudaGetLastError();
+            set_err("cudaMalloc (batch workspace): out of device memory");
+            return OCTANE_ENOMEM;
+        }
+        CUDA_OK(cudaStreamSynchronize(c->stream));
+        cudaFree(c->arena);
+        c->arena = na; c->arena_bytes = need; c->arena_pairs = 0;
+        arena_layout(pl, &c->buf, c->arena);
+        destroy_graphs(c);                                   // the captured PCG loops point into the old workspace
+        c->pcg_graph.assign(2 * pl.lv.size(), nullptr);
+    }
+    if (npairs > c->arena_pairs) {                           // padding and unused rows must hold finite values
+        CUDA_OK(cudaMemsetAsync(c->arena + S * c->arena_pairs, 0, S * (size_t)(npairs - c->arena_pairs), c->stream));
+        c->arena_pairs = npairs;
+    }
+    int bb = 0;
+    for (const Level& L : pl.lv) { int t = build_partial_blocks(L.g, L.g.rows); if (t > bb) bb = t; }
+    const size_t pd = (size_t)npairs * (2 * (size_t)bb > 3 * 8 ? 2 * (size_t)bb : 3 * 8);
+    if (npairs > c->batch_cap || pd > c->bpart_doubles) {
+        CUDA_OK(cudaStreamSynchronize(c->stream));
+        for (void* q : { (void*)c->d_bscal, (void*)c->d_bpart, (void*)c->d_bbar, (void*)c->d_bits, (void*)c->d_bnav })
+            if (q) cudaFree(q);
+        c->d_bscal = nullptr; c->d_bpart = nullptr; c->d_bbar = nullptr; c->d_bits = nullptr; c->d_bnav = nullptr;
+        c->batch_cap = 0; c->bpart_doubles = 0;
+        const int n = npairs > c->batch_cap ? npairs : c->batch_cap;
+        if (cudaMalloc(&c->d_bscal, n * sizeof(PcgScalars)) != cudaSuccess ||
+            cudaMalloc(&c->d_bpart, pd * sizeof(double)) != cudaSuccess ||
+            cudaMalloc(&c->d_bbar, 2 * n * sizeof(unsigned)) != cudaSuccess ||
+            cudaMalloc(&c->d_bits, (size_t)n * OCTANE_MAX_SOLVES * sizeof(int)) != cudaSuccess ||
+            cudaMalloc(&c->d_bnav, n * sizeof(NavParams)) != cudaSuccess) {
+            cudaGetLastError();
+            set_err("cudaMalloc (batch buffers): out of device memory");
+            return OCTANE_ENOMEM;
+        }
+        CUDA_OK(cudaMemsetAsync(c->d_bscal, 0, n * sizeof(PcgScalars), c->stream));
+        c->batch_cap = n; c->bpart_doubles = pd;
+    }
+    return OCTANE_OK;
+}
+
+// pair b's view of the PCG planes (the large-level loop runs the single-pair kernels on it)
+PcgBuffers pair_buffers(const PcgBuffers& b0, int b, size_t ps)
+{
+    PcgBuffers q = b0;
+    const size_t po = (size_t)b * ps;
+    for (int i = 0; i < NCOEF; i++) q.coef[i] += po;
+    q.ru += po; q.rv += po; q.xu += po; q.xv += po;
+    q.pu[0] += po; q.pu[1] += po; q.pv[0] += po; q.pv[1] += po;
+    q.qu += po; q.qv += po; q.r2u += po; q.r2v += po;
+    return q;
+}
+
+// run_levels for npairs pairs in the batch workspace (pair stride ps floats); one GPU, no first guess.  Per-pixel
+// stages are one launch for all pairs; small levels solve all pairs in cooperative launches with one barrier per
+// pair (launch_pcg_coop_batch), large levels run the single-pair PCG kernels pair by pair.
+int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
+{
+    const Plan& pl = c->plan;
+    Buffers& B = c->buf;
+    const octane_params& p = pl.p;
+    const int K = p.kiters, nc = pl.nc;
+    const int nsol = K * 3 * p.liters;
+    cudaStream_t st = c->stream;
+    const float sf = (float)p.scaleF;
+    const size_t S = ps * sizeof(float);
+    PcgBuffers pb = B.pcg;                       // build and update: pair z uses d_bscal[z] (and partials region z)
+    pb.scal = c->d_bscal;
+    pb.partials = c->d_bpart;
+    int solve = 0;
+    for (int k = 0; k < K; k++) {
+        const Level& L = pl.lv[k];
+        const Geom& g = L.g;
+        const bool finest = (k == K - 1);
+        float *g1 = finest ? B.img1 : B.g1c, *g2 = finest ? B.img2 : B.g2c;
+        if (k > 0) {
+            const Level& Lc = pl.lv[k - 1];
+            launch_zoom_in(B.ut, Lc.g, B.u, g, L.own0, L.own1, sf, st, npairs, ps);
+            launch_zoom_in(B.vt, Lc.g, B.v, g, L.own0, L.own1, sf, st, npairs, ps);
+            c->launches += 2;
+        }
+        if (!finest) {
+            const Geom& gF = pl.lv[K - 1].g;
+            launch_fill_gk(c->d_gk, L.factor, L.R, st);
+            launch_blur_decimate(B.img1, gF, B.g1c, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, 1.f, nc, st, npairs, ps);
+            launch_blur_decimate(B.img2, gF, B.g2c, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, 1.f, nc, st, npairs, ps);
+            c->launches += 3;
+        }
+        if (k == 0) {
+            CUDA_OK(cudaMemset2DAsync(B.u, S, 0, (size_t)g.plane * sizeof(float), npairs, st));
+            CUDA_OK(cudaMemset2DAsync(B.v, S, 0, (size_t)g.plane * sizeof(float), npairs, st));
+        }
+        launch_gradient(g1, B.g1x, B.g1y, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
+        launch_gradient(g2, B.g2x, B.g2y, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
+        launch_gradient(B.g2x, B.g2xx, nullptr, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
+        launch_gradient(B.g2y, B.g2xy, B.g2yy, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
+        c->launches += 4;
+        LevelFields f;
+        f.g1 = g1; f.g1x = B.g1x; f.g1y = B.g1y;
+        f.g2 = g2; f.g2x = B.g2x; f.g2y = B.g2y; f.g2xx = B.g2xx; f.g2xy = B.g2xy; f.g2yy = B.g2yy;
+        f.u = B.u; f.v = B.v;
+        f.uh = nullptr; f.vh = nullptr;
+        BuildParams bp;
+        bp.alpha = p.alpha; bp.ralpha = 1.0 / p.alpha; bp.lambdadalpha = p.lambda / p.alpha; bp.lambdac = L.lambdac;
+        bp.dozim = p.dozim != 0; bp.nchan = nc; bp.tol = 0.0001 * 0.0001;
+        const bool fused = level_fused(c, L);
+        const bool small = !pcg_fused_usable(L.g, L.own1 - L.own0);
+        const int per_launch = small ? coop_batch_pairs_per_launch(g, L.own0, L.own1, c->sm_count) : 0;
+        for (int gnc = 0; gnc < 3; gnc++) {
+            bp.al1 = 1. - 0.5 * gnc;
+            for (int l = 0; l < p.liters; l++, solve++) {
+                launch_build(f, pb, g, L.own0, L.own1, L.own0, L.own1, bp, 0, st, npairs, ps);
+                c->launches += 2;
+                if (p.cgiters > 0 && small) {
+                    for (int p0 = 0; p0 < npairs; p0 += per_launch) {
+                        const int n = npairs - p0 < per_launch ? npairs - p0 : per_launch;
+                        if (launch_pcg_coop_batch(pb, g, L.own0, L.own1, p.cgiters, p0, n, ps, c->d_bpart, c->d_bbar, st)) {
+                            set_err("cooperative launch of the batched PCG solver: %s", cudaGetErrorString(cudaGetLastError()));
+                            return OCTANE_ECUDA;
+                        }
+                        c->launches++;
+                    }
+                } else if (p.cgiters > 0) {
+                    for (int b = 0; b < npairs; b++) {
+                        PcgBuffers q = pair_buffers(B.pcg, b, ps);
+                        q.scal = c->d_bscal + b;
+                        int rc = enqueue_pcg(c, L, k, solve, gnc == 0 ? 1 : 0, q);
+                        if (rc) return rc;
+                    }
+                }
+                if (fused) launch_update_uv_fused(B.u, B.v, pb, g, L.own0, L.own1, c->d_bits + solve, c->sm_count, st, npairs, ps, nsol);
+                else launch_update_uv(B.u, B.v, pb, g, L.own0, L.own1, c->d_bits + solve, c->sm_count, st, npairs, ps, nsol);
+                c->launches++;
+            }
+        }
+        if (!finest) {
+            CUDA_OK(cudaMemcpy2DAsync(B.ut, S, B.u, S, (size_t)g.plane * sizeof(float), npairs, cudaMemcpyDeviceToDevice, st));
+            CUDA_OK(cudaMemcpy2DAsync(B.vt, S, B.v, S, (size_t)g.plane * sizeof(float), npairs, cudaMemcpyDeviceToDevice, st));
+        }
+    }
+    // pair 0's counts and scalars for octane_get_stats
+    CUDA_OK(cudaMemcpyAsync(c->h_its, c->d_bits, sizeof(int) * nsol, cudaMemcpyDeviceToHost, st));
+    CUDA_OK(cudaMemcpyAsync(c->h_scal, c->d_bscal, sizeof(PcgScalars), cudaMemcpyDeviceToHost, st));
+    CUDA_OK(cudaGetLastError());
+    return OCTANE_OK;
+}
+}  // namespace
+
+int octane_optical_flow_batch_dev(octane_ctx* c, int npairs, const float* d_img1, const float* d_img2, const float* d_cth,
+                                  int nx, int ny, int nc, const octane_nav* nav, const double* t1, const double* t2,
+                                  const octane_params* p, float* d_upix, float* d_vpix, short* U, short* V, short* Ur,
+                                  short* Vr, short* d_ctp, int* moved_out)
+{
+    if (!c || !d_img1 || !d_img2 || !nav || !t1 || !t2 || !p || !d_upix || !d_vpix || !U || !V || !Ur || !Vr) {
+        set_err("null argument");
+        return OCTANE_EINVAL;
+    }
+    if (npairs < 1) { set_err("npairs must be at least 1"); return OCTANE_EINVAL; }
+    if (p->first_guess) { set_err("batched calls take no first guess"); return OCTANE_EINVAL; }
+    if (p->dosrsal) { set_err("batched calls do not run -srsal"); return OCTANE_EINVAL; }
+    if (p->doCTH && (!d_cth || !d_ctp)) { set_err("doCTH needs cth and ctp"); return OCTANE_EINVAL; }
+    if (c->comm.world > 1) { set_err("context is banded: batched calls are single-GPU"); return OCTANE_EINVAL; }
+    begin_call(c);
+    int rc = prepare(c, nx, ny, nc, *p);
+    if (rc) return rc;
+    if (p->kiters * 3 * p->liters > OCTANE_MAX_SOLVES) { set_err("too many solves"); return OCTANE_EINVAL; }
+    size_t S = 0;
+    rc = ensure_batch(c, npairs, &S);
+    if (rc) return rc;
+    const size_t ps = S / sizeof(float), n = (size_t)nx * ny;
+    cudaStream_t st = c->stream;
+    // dense pairs -> pitched finest-level planes of each pair's workspace
+    const Geom& g = c->plan.lv.back().g;
+    const size_t w = (size_t)nx * sizeof(float), dp = (size_t)g.pitch * sizeof(float);
+    for (int b = 0; b < npairs; b++)
+        for (int ch = 0; ch < nc; ch++) {
+            const size_t src = ((size_t)b * nc + ch) * n, dst = (size_t)b * ps + (size_t)ch * g.plane;
+            CUDA_OK(cudaMemcpy2DAsync(c->buf.img1 + dst, dp, d_img1 + src, w, w, ny, cudaMemcpyDeviceToDevice, st));
+            CUDA_OK(cudaMemcpy2DAsync(c->buf.img2 + dst, dp, d_img2 + src, w, w, ny, cudaMemcpyDeviceToDevice, st));
+        }
+    rc = run_levels_batch(c, npairs, ps);
+    if (rc) return rc;
+    for (int b = 0; b < npairs; b++) {
+        CUDA_OK(cudaMemcpy2DAsync(d_upix + b * n, w, c->buf.u + (size_t)b * ps, dp, w, ny, cudaMemcpyDeviceToDevice, st));
+        CUDA_OK(cudaMemcpy2DAsync(d_vpix + b * n, w, c->buf.v + (size_t)b * ps, dp, w, ny, cudaMemcpyDeviceToDevice, st));
+    }
+    if (p->doCTH) {                            // src/oct_optical_flow.cc:71-88, all pairs in one launch
+        launch_ctp_pack(d_cth, d_ctp, (size_t)npairs * n, p->ir == 1, st);
+        c->launches++;
+    }
+    std::vector<NavParams> np(npairs);
+    for (int b = 0; b < npairs; b++) fill_nav(np[b], &nav[b], t1[b], t2[b], p);
+    const size_t need = pix2uv_table_doubles(nx, ny) * (size_t)npairs;
+    if (need > c->navtab_doubles) {
+        CUDA_OK(cudaStreamSynchronize(st));
+        if (c->d_navtab) cudaFree(c->d_navtab);
+        c->d_navtab = nullptr; c->navtab_doubles = 0;
+        CUDA_OK(cudaMalloc(&c->d_navtab, need * sizeof(double)));
+        c->navtab_doubles = need;
+    }
+    CUDA_OK(cudaMemcpyAsync(c->d_bnav, np.data(), npairs * sizeof(NavParams), cudaMemcpyHostToDevice, st));
+    c->launches += launch_pix2uv_batch(np[0], c->d_bnav, npairs, d_upix, d_vpix, nx, ny, c->d_navtab, U, V, Ur, Vr, st);
+    for (int b = 0; b < npairs; b++) {        // sector-moved guard, src/oct_pix2uv_cuda.cu:295,358-368
+        const bool moved = sector_moved(&nav[b]);
+        if (moved_out) moved_out[b] = moved ? 1 : 0;
+        if (!moved) continue;
+        for (short* q : { U, V, Ur, Vr }) CUDA_OK(cudaMemsetAsync(q + b * n, 0, n * sizeof(short), st));
+    }
+    CUDA_OK(cudaGetLastError());
+    c->batch_npairs = npairs;
+    c->batch_nsolves = p->kiters * 3 * p->liters;
+    return OCTANE_OK;
+}
+
+int octane_batch_cg_iterations(octane_ctx* c, int* its, int npairs)
+{
+    if (!c || !its) { set_err("null argument"); return OCTANE_EINVAL; }
+    if (npairs != c->batch_npairs || npairs < 1) { set_err("npairs differs from the last batched call"); return OCTANE_EINVAL; }
+    CUDA_OK(cudaSetDevice(c->device));
+    CUDA_OK(cudaStreamSynchronize(c->stream));
+    const int ns = c->batch_nsolves;
+    for (int b = 0; b < npairs; b++)
+        CUDA_OK(cudaMemcpy(its + (size_t)b * ns, c->d_bits + (size_t)b * ns, ns * sizeof(int), cudaMemcpyDeviceToHost));
+    return OCTANE_OK;
 }
 
 int octane_pix2uv(octane_ctx* c, const octane_nav* nav, double t1, double t2, const float* u, const float* v,

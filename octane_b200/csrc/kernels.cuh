@@ -4,13 +4,17 @@
 
 namespace octane {
 
+// Batched launches: npairs pairs whose planes lie ps floats apart (one copy of the per-pair workspace each); the
+// kernels take the pair from blockIdx.z.  npairs = 1, ps = 0 is the single-pair call.
 // ---- pyramid.cu
 void launch_fill_gk(float* GK, float factor, int R, cudaStream_t st);
 void launch_blur_decimate(const float* src, const Geom& gs, float* dst, const Geom& gd, int ja, int jb,
-                          float factor, const float* GK, int R, float scale, int nc, cudaStream_t st);
-void launch_gradient(const float* f, float* gx, float* gy, const Geom& g, int ja, int jb, int nc, cudaStream_t st);
+                          float factor, const float* GK, int R, float scale, int nc, cudaStream_t st,
+                          int npairs = 1, size_t ps = 0);
+void launch_gradient(const float* f, float* gx, float* gy, const Geom& g, int ja, int jb, int nc, cudaStream_t st,
+                     int npairs = 1, size_t ps = 0);
 void launch_zoom_in(const float* flow, const Geom& gc, float* out, const Geom& gf, int ja, int jb, float sf,
-                    cudaStream_t st);
+                    cudaStream_t st, int npairs = 1, size_t ps = 0);
 
 // ---- build.cu
 struct LevelFields {           // device planes of one level, all sharing Geom g
@@ -59,9 +63,10 @@ struct BuildParams {
     int dozim, nchan;
     float tol;
 };
-// rows [ja,jb) get coefficients + rhs; dots (b.b, b.Minv b) over rows [da,db)
+// rows [ja,jb) get coefficients + rhs; dots (b.b, b.Minv b) over rows [da,db).  Batched: pair z seeds b.scal[z] and
+// uses partials region z (2 * build_partial_blocks doubles each).
 void launch_build(const LevelFields& f, const PcgBuffers& b, const Geom& g, int ja, int jb, int da, int db,
-                  const BuildParams& bp, int halo_check, cudaStream_t st);
+                  const BuildParams& bp, int halo_check, cudaStream_t st, int npairs = 1, size_t ps = 0);
 int build_partial_blocks(const Geom& g, int nrows);
 
 // shared memory one block of k_blur_decimate needs for a level (pyramid.cu); levels beyond the limit are refused
@@ -86,9 +91,17 @@ void launch_pcg_pass2(const PcgBuffers& b, const Geom& g, int ja, int jb, int sm
 // small levels on one GPU: the whole solve (up to `iters` iterations of the same two passes, same recurrence) in one
 // cooperative launch with grid-wide barriers instead of 2 x iters launches; returns 0, or -1 when the launch fails
 int launch_pcg_coop(const PcgBuffers& b, const Geom& g, int ja, int jb, int iters, int sm_count, cudaStream_t st);
-// u += x + alpha_last p_last, v likewise (:1185-1195 with the pending x term folded in)
+// small levels of a batch: pairs [pair0, pair0 + npairs) solved in one cooperative launch, coop_batch_blocks blocks
+// per pair, each group with its own partials (3 G doubles) and barrier (2 unsigned, zeroed here on the stream);
+// b.scal[pair] are the pairs' scalars.  Returns 0, or -1 when the launch fails.
+int coop_batch_blocks(const Geom& g, int ja, int jb);
+int coop_batch_pairs_per_launch(const Geom& g, int ja, int jb, int sm_count);
+int launch_pcg_coop_batch(const PcgBuffers& b, const Geom& g, int ja, int jb, int iters, int pair0, int npairs, size_t ps,
+                          double* partials, unsigned* bar, cudaStream_t st);
+// u += x + alpha_last p_last, v likewise (:1185-1195 with the pending x term folded in).  Batched: pair z reads
+// b.scal[z] and writes its_out[z * its_stride].
 void launch_update_uv(float* u, float* v, const PcgBuffers& b, const Geom& g, int ja, int jb,
-                      int* its_out, int sm_count, cudaStream_t st);
+                      int* its_out, int sm_count, cudaStream_t st, int npairs = 1, size_t ps = 0, int its_stride = 0);
 // ---- pcg_fused.cu: one launch and one reduction per iteration (merged recurrence; large levels)
 bool pcg_fused_usable(const Geom& g, int nrows);
 // banded runs: the neighbours' two r buffers [buffer][component] as mapped here (peer memory), shifted to this rank's
@@ -102,7 +115,7 @@ void launch_pcg_fused(const PcgBuffers& b, const Geom& g, int ja, int jb, int ki
                       int sm_count, cudaStream_t st, int const_wn);
 // u += x (+ the pending alpha p when the iteration count is odd), after a merged-reduction solve
 void launch_update_uv_fused(float* u, float* v, const PcgBuffers& b, const Geom& g, int ja, int jb,
-                            int* its_out, int sm_count, cudaStream_t st);
+                            int* its_out, int sm_count, cudaStream_t st, int npairs = 1, size_t ps = 0, int its_stride = 0);
 // test hooks: 5-plane storage <-> the reference's 7 boundary-merged entries
 void launch_expand_coef(const PcgBuffers& b, const Geom& g, float* a5, float* a6, float* a7, float* a8, cudaStream_t st);
 // dense (stride nx, rows [ja,jb) starting at src row 0) <-> pitched
@@ -121,6 +134,10 @@ struct NavParams {
 size_t pix2uv_table_doubles(int nx, int nrows);
 int launch_pix2uv(const NavParams& np, const float* u, const float* v, int nx, int row0, int nrows, double* tab,
                   short* U, short* V, short* Uraw, short* Vraw, cudaStream_t st);
+// npairs whole scenes: pair b has d_navs[b] (device; the grid kind of np0 for all), dense planes b * nx * ny values
+// on and its table at tab + b * pix2uv_table_doubles(nx, ny)
+int launch_pix2uv_batch(const NavParams& np0, const NavParams* d_navs, int npairs, const float* u, const float* v, int nx,
+                        int ny, double* tab, short* U, short* V, short* Uraw, short* Vraw, cudaStream_t st);
 void launch_ctp_pack(const float* cth, short* ctp, size_t n, int ir, cudaStream_t st);
 
 

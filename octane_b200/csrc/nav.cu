@@ -139,8 +139,13 @@ __device__ __forceinline__ double arc_meridional(float lat_a, float lat_b)
 }
 
 // ---- setup: constants and the per-column / per-row tables of the unmoved pixel -------------------
-__global__ void __launch_bounds__(128) k_nav_tables(NavParams nav, int nx, int row0, int nrows, double* __restrict__ tab)
+// BATCH: pair blockIdx.z, with navs[blockIdx.z] and its own table tstride doubles further on
+template <bool BATCH>
+__global__ void __launch_bounds__(128) k_nav_tables(NavParams nav0, int nx, int row0, int nrows, double* __restrict__ tab,
+                                                    const NavParams* __restrict__ navs, size_t tstride)
 {
+    const NavParams nav = BATCH ? navs[blockIdx.z] : nav0;
+    if (BATCH) tab += blockIdx.z * tstride;
     const int t = blockIdx.x * 128 + threadIdx.x;
     double* col = tab + NT_HEAD;
     double* row = col + (size_t)NT_COL * nx;
@@ -191,14 +196,21 @@ __global__ void __launch_bounds__(128) k_nav_tables(NavParams nav, int nx, int r
 // ---- per pixel: a block owns 128 columns x NAV_ROWS rows; a thread walks one column down --------
 constexpr int NAV_ROWS = 8;
 
-template <int GRID>     // 0 GOES fixed grid, 1 polar, 2 Mercator
+// BATCH: pair blockIdx.z, with navs[blockIdx.z], its table tstride doubles and its planes n values further on
+template <int GRID, bool BATCH>     // GRID: 0 GOES fixed grid, 1 polar, 2 Mercator
 __global__ void __launch_bounds__(128)
-k_pix2uv(NavParams nav, const float* __restrict__ u, const float* __restrict__ v, int nx, int row0, int nrows,
+k_pix2uv(NavParams nav0, const float* __restrict__ u, const float* __restrict__ v, int nx, int row0, int nrows,
          const double* __restrict__ tab, short* __restrict__ ur, short* __restrict__ vr, short* __restrict__ ur2,
-         short* __restrict__ vr2)
+         short* __restrict__ vr2, const NavParams* __restrict__ navs, size_t tstride, size_t n)
 {
     const int i = blockIdx.x * 128 + threadIdx.x;
     if (i >= nx) return;
+    const NavParams nav = BATCH ? navs[blockIdx.z] : nav0;
+    if (BATCH) {
+        const size_t po = blockIdx.z * n;
+        tab += blockIdx.z * tstride;
+        u += po; v += po; ur += po; vr += po; ur2 += po; vr2 += po;
+    }
     const double* col = tab + NT_HEAD;
     const double* row = col + (size_t)NT_COL * nx;
     const double dt = nav.t2 - nav.t1;
@@ -285,11 +297,24 @@ int launch_pix2uv(const NavParams& np, const float* u, const float* v, int nx, i
                   short* U, short* V, short* Uraw, short* Vraw, cudaStream_t st)
 {
     if (nx <= 0 || nrows <= 0) return 0;
-    k_nav_tables<<<(nx + nrows + 127) / 128, 128, 0, st>>>(np, nx, row0, nrows, tab);
+    k_nav_tables<false><<<(nx + nrows + 127) / 128, 128, 0, st>>>(np, nx, row0, nrows, tab, nullptr, 0);
     const dim3 grid((nx + 127) / 128, (nrows + NAV_ROWS - 1) / NAV_ROWS);
-    if (np.dp)      k_pix2uv<1><<<grid, 128, 0, st>>>(np, u, v, nx, row0, nrows, tab, U, V, Uraw, Vraw);
-    else if (np.dm) k_pix2uv<2><<<grid, 128, 0, st>>>(np, u, v, nx, row0, nrows, tab, U, V, Uraw, Vraw);
-    else            k_pix2uv<0><<<grid, 128, 0, st>>>(np, u, v, nx, row0, nrows, tab, U, V, Uraw, Vraw);
+    if (np.dp)      k_pix2uv<1, false><<<grid, 128, 0, st>>>(np, u, v, nx, row0, nrows, tab, U, V, Uraw, Vraw, nullptr, 0, 0);
+    else if (np.dm) k_pix2uv<2, false><<<grid, 128, 0, st>>>(np, u, v, nx, row0, nrows, tab, U, V, Uraw, Vraw, nullptr, 0, 0);
+    else            k_pix2uv<0, false><<<grid, 128, 0, st>>>(np, u, v, nx, row0, nrows, tab, U, V, Uraw, Vraw, nullptr, 0, 0);
+    return 2;
+}
+
+int launch_pix2uv_batch(const NavParams& np0, const NavParams* d_navs, int npairs, const float* u, const float* v, int nx,
+                        int ny, double* tab, short* U, short* V, short* Uraw, short* Vraw, cudaStream_t st)
+{
+    if (nx <= 0 || ny <= 0 || npairs <= 0) return 0;
+    const size_t ts = pix2uv_table_doubles(nx, ny), n = (size_t)nx * ny;
+    k_nav_tables<true><<<dim3((nx + ny + 127) / 128, 1, npairs), 128, 0, st>>>(np0, nx, 0, ny, tab, d_navs, ts);
+    const dim3 grid((nx + 127) / 128, (ny + NAV_ROWS - 1) / NAV_ROWS, npairs);
+    if (np0.dp)      k_pix2uv<1, true><<<grid, 128, 0, st>>>(np0, u, v, nx, 0, ny, tab, U, V, Uraw, Vraw, d_navs, ts, n);
+    else if (np0.dm) k_pix2uv<2, true><<<grid, 128, 0, st>>>(np0, u, v, nx, 0, ny, tab, U, V, Uraw, Vraw, d_navs, ts, n);
+    else             k_pix2uv<0, true><<<grid, 128, 0, st>>>(np0, u, v, nx, 0, ny, tab, U, V, Uraw, Vraw, d_navs, ts, n);
     return 2;
 }
 

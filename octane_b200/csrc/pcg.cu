@@ -120,10 +120,10 @@ __device__ __forceinline__ PRow compute_p(const P1Args& a, int cur, int j, int i
 __device__ __forceinline__ float mul_lo(int i, int n) { return i == 0 ? 0.f : (i == n - 1 ? 2.f : 1.f); }
 __device__ __forceinline__ float mul_hi(int i, int n) { return i == n - 1 ? 0.f : (i == 0 ? 2.f : 1.f); }
 
-// q = A p of this block's share of the (strip x row segment) tasks, p and x updated on the way; returns the
-// thread's partial p.q.  Shared by the per-iteration kernel and the whole-solve cooperative kernel.
+// q = A p of block `bid`'s share (of `nblk` blocks) of the (strip x row segment) tasks, p and x updated on the way;
+// returns the thread's partial p.q.  Shared by the per-iteration kernel and the whole-solve cooperative kernels.
 template <int XM>
-__device__ __forceinline__ double pass1_tasks(const P1Args& a, int cur, float beta, float alpha_prev)
+__device__ __forceinline__ double pass1_tasks(const P1Args& a, int cur, float beta, float alpha_prev, int bid, int nblk)
 {
     constexpr bool FIRST = (XM == XM_NONE);
     const Geom& g = a.g;
@@ -135,7 +135,7 @@ __device__ __forceinline__ double pass1_tasks(const P1Args& a, int cur, float be
     const float* N = a.b.coef[C_N];
     double dot[1] = { 0.0 };
 
-    for (int t = blockIdx.x * 8 + wib; t < ntasks; t += gridDim.x * 8) {
+    for (int t = bid * 8 + wib; t < ntasks; t += nblk * 8) {
         const int seg = t / a.nstrips, strip = t - seg * a.nstrips;
         const int i0 = strip * 128 + lane * 4;
         const int j_a = a.ja + seg * a.rs, j_b = min(a.jb, j_a + a.rs);
@@ -224,7 +224,7 @@ __global__ void __launch_bounds__(256, 2) k_pcg_pass1(P1Args a)
     if (s->done) return;
     const float beta = FIRST ? 0.f : s->rz / s->rz_old;      // Bk, :1144
     const float alpha_prev = FIRST ? 0.f : s->alpha;
-    double dot[1] = { pass1_tasks<XM>(a, a.cur, beta, alpha_prev) };
+    double dot[1] = { pass1_tasks<XM>(a, a.cur, beta, alpha_prev, blockIdx.x, gridDim.x) };
     block_sum<1>(dot, red);
     double tot[1];
     if (grid_sum_finish<1>(dot, a.b.partials, a.b.ticket, tot, red)) {
@@ -238,15 +238,15 @@ __global__ void __launch_bounds__(256, 2) k_pcg_pass1(P1Args a)
 
 typedef P1Args P2Args;       // pass 2 reads b, g, ja, jb of the same argument block
 
-// r -= alpha q over this block's share of the rows; acc += partial r.r and z.r.  Shared by the per-iteration kernel
-// and the whole-solve cooperative kernel.
-__device__ __forceinline__ void pass2_units(const P1Args& a, float alphak, bool p2p, double (&acc)[2])
+// r -= alpha q over block `bid`'s share (of `nblk` blocks) of the rows; acc += partial r.r and z.r.  Shared by the
+// per-iteration kernel and the whole-solve cooperative kernels.
+__device__ __forceinline__ void pass2_units(const P1Args& a, float alphak, bool p2p, double (&acc)[2], int bid, int nblk)
 {
     const float nalpha = -1. * alphak;                        // :1174
     const Geom& g = a.g;
     const int upr = g.pitch >> 2;                             // float4 units per row
     const long long nunits = (long long)(a.jb - a.ja) * upr;
-    for (long long t = (long long)blockIdx.x * 256 + threadIdx.x; t < nunits; t += (long long)gridDim.x * 256) {
+    for (long long t = (long long)bid * 256 + threadIdx.x; t < nunits; t += (long long)nblk * 256) {
         const int jr = (int)(t / upr), i0 = (int)(t - (long long)jr * upr) * 4;
         if (i0 >= g.nx) continue;
         const size_t off = g.at(i0, a.ja + jr);
@@ -291,7 +291,7 @@ __global__ void __launch_bounds__(256) k_pcg_pass2(P2Args a)
     const float alphak = s->rz / s->pAp;                      // :1169
     const bool p2p = a.b.p2p.world > 1;
     double acc[2] = { 0.0, 0.0 };
-    pass2_units(a, alphak, p2p, acc);
+    pass2_units(a, alphak, p2p, acc, blockIdx.x, gridDim.x);
     block_sum<2>(acc, red);
     double tot[2];
     if (grid_sum_finish<2>(acc, a.b.partials, a.b.ticket, tot, red, p2p)) {
@@ -363,14 +363,14 @@ __global__ void __launch_bounds__(256, 2) k_pcg_coop(P1Args a, int iters)
     for (int ki = 0; ki < iters && !done; ki++) {
         const int cur = ki & 1;
         double d1[1];
-        if (ki == 0)      d1[0] = pass1_tasks<XM_NONE>(a, cur, 0.f, 0.f);
-        else if (ki == 1) d1[0] = pass1_tasks<XM_INIT>(a, cur, rz / rz_old, alpha);       // Bk, :1144
-        else              d1[0] = pass1_tasks<XM_ACC>(a, cur, rz / rz_old, alpha);
+        if (ki == 0)      d1[0] = pass1_tasks<XM_NONE>(a, cur, 0.f, 0.f, blockIdx.x, gridDim.x);
+        else if (ki == 1) d1[0] = pass1_tasks<XM_INIT>(a, cur, rz / rz_old, alpha, blockIdx.x, gridDim.x);       // Bk, :1144
+        else              d1[0] = pass1_tasks<XM_ACC>(a, cur, rz / rz_old, alpha, blockIdx.x, gridDim.x);
         coop_sum<1>(d1, part1, red, grid);
         const float pAp = (float)d1[0];                                              // pkTApk, :1165
         const float alphak = rz / pAp;                                               // :1169
         double d2[2] = { 0.0, 0.0 };
-        pass2_units(a, alphak, false, d2);
+        pass2_units(a, alphak, false, d2, blockIdx.x, gridDim.x);
         coop_sum<2>(d2, part2, red, grid);
         alpha = alphak;
         rz_old = rz;
@@ -380,6 +380,130 @@ __global__ void __launch_bounds__(256, 2) k_pcg_coop(P1Args a, int iters)
         done = !(rr > tol);                                                          // :1131
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) {
+        s->alpha = alpha; s->rz_old = rz_old; s->rz = rz; s->rr = rr; s->its = its; s->done = done ? 1 : 0;
+    }
+}
+
+// ---- a whole solve of MANY pairs in one cooperative launch (small levels, batched calls) ------------------------
+// Pair `pair0 + k` of the launch is solved by the k-th group of G consecutive blocks, with its own partial sums, its
+// own barrier and its own scalars: a pair that meets its stop rule leaves without waiting for the others.  G and
+// the task partition depend only on the level geometry (coop_batch_blocks), so a pair's bits do not depend on how
+// many other pairs share the launch or where in the batch it sits.
+struct CoopBatch {
+    int G;                 // blocks per pair
+    int pair0;             // first pair of this launch (index into the batch)
+    size_t ps;             // pair stride of the workspace planes (floats)
+    double* partials;      // [launch pairs][3 G]: p.q, then r.r and z.r
+    unsigned* bar;         // [launch pairs][2]: arrive counter, generation -- zero before the launch
+};
+
+__device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p)
+{
+    unsigned v;
+    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_release_gpu(unsigned* p, unsigned v)
+{
+    asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ unsigned atom_add_acq_rel_gpu(unsigned* p, unsigned v)
+{
+    unsigned old;
+    asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], %2;" : "=r"(old) : "l"(p), "r"(v) : "memory");
+    return old;
+}
+
+// Barrier of one group of G blocks (all co-resident: the launch is cooperative).  Thread 0 reads the generation
+// (acquire) BEFORE it arrives, so the last arrival cannot advance it unseen; the last arrival resets the counter and
+// then releases the next generation, so a block that has seen the new generation also sees the counter at zero.
+// The fences make the writes of all the block's threads (ordered before thread 0 by __syncthreads) visible to the
+// group, as grid.sync() does for a whole grid.
+__device__ __forceinline__ void group_barrier(unsigned* bar, unsigned G)
+{
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const unsigned gen = ld_acquire_gpu(bar + 1);
+        __threadfence();
+        if (atom_add_acq_rel_gpu(bar, 1u) == G - 1) {
+            bar[0] = 0u;
+            st_release_gpu(bar + 1, gen + 1u);
+        } else {
+            while (ld_acquire_gpu(bar + 1) == gen) __nanosleep(20);
+        }
+        __threadfence();
+    }
+    __syncthreads();
+}
+
+// coop_sum over the blocks of one group: block lb of G writes its partials, then every block sums all G in the same
+// fixed order
+template <int NV>
+__device__ __forceinline__ void group_sum(double (&v)[NV], double* partials, double* red, unsigned* bar, int G, int lb)
+{
+    const int tid = threadIdx.x;
+    block_sum<NV>(v, red);
+    if (tid == 0) {
+#pragma unroll
+        for (int k = 0; k < NV; k++) partials[(size_t)k * G + lb] = v[k];
+    }
+    group_barrier(bar, (unsigned)G);
+#pragma unroll
+    for (int k = 0; k < NV; k++) {
+        double t = 0.0;
+        for (int b = tid; b < G; b += 256) t += __ldcg(&partials[(size_t)k * G + b]);
+        v[k] = t;
+    }
+    __syncthreads();
+    block_sum<NV>(v, red);
+    __shared__ double bc[NV];
+    if (tid == 0) {
+#pragma unroll
+        for (int k = 0; k < NV; k++) bc[k] = v[k];
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < NV; k++) v[k] = bc[k];
+}
+
+__global__ void __launch_bounds__(256, 2) k_pcg_coop_batch(P1Args a, CoopBatch cb, int iters)
+{
+    __shared__ double red[2 * 32];
+    const int grp = blockIdx.x / cb.G, lb = blockIdx.x - grp * cb.G, G = cb.G;
+    const int pair = cb.pair0 + grp;
+    const size_t po = (size_t)pair * cb.ps;
+    for (int i = 0; i < NCOEF; i++) a.b.coef[i] += po;
+    a.b.ru += po; a.b.rv += po; a.b.xu += po; a.b.xv += po;
+    a.b.pu[0] += po; a.b.pu[1] += po; a.b.pv[0] += po; a.b.pv[1] += po;
+    a.b.qu += po; a.b.qv += po;
+    PcgScalars* s = a.b.scal + pair;
+    double* part1 = cb.partials + (size_t)grp * 3 * G;       // p.q
+    double* part2 = part1 + G;                               // r.r, z.r
+    unsigned* bar = cb.bar + 2 * grp;
+    float rz = s->rz, rr = s->rr, rz_old = 0.f, alpha = 0.f;
+    const float tol = s->tol;
+    int its = 0;
+    bool done = s->done != 0;
+    for (int ki = 0; ki < iters && !done; ki++) {
+        const int cur = ki & 1;
+        double d1[1];
+        if (ki == 0)      d1[0] = pass1_tasks<XM_NONE>(a, cur, 0.f, 0.f, lb, G);
+        else if (ki == 1) d1[0] = pass1_tasks<XM_INIT>(a, cur, rz / rz_old, alpha, lb, G);       // Bk, :1144
+        else              d1[0] = pass1_tasks<XM_ACC>(a, cur, rz / rz_old, alpha, lb, G);
+        group_sum<1>(d1, part1, red, bar, G, lb);
+        const float pAp = (float)d1[0];                                              // pkTApk, :1165
+        const float alphak = rz / pAp;                                               // :1169
+        double d2[2] = { 0.0, 0.0 };
+        pass2_units(a, alphak, false, d2, lb, G);
+        group_sum<2>(d2, part2, red, bar, G, lb);
+        alpha = alphak;
+        rz_old = rz;
+        rz = (float)d2[1];
+        rr = (float)d2[0];
+        its++;
+        done = !(rr > tol);                                                          // :1131
+    }
+    if (lb == 0 && threadIdx.x == 0) {
         s->alpha = alpha; s->rz_old = rz_old; s->rz = rz; s->rr = rr; s->its = its; s->done = done ? 1 : 0;
     }
 }
@@ -423,11 +547,12 @@ void launch_finalize(const PcgBuffers& b, int kind, float tol, cudaStream_t st)
 // After `its` iterations x holds the terms of iterations 0 .. its-2 (none when its == 1) and
 // p[its & 1] is the search direction of iteration its-1.  Nothing happens when no iteration ran.
 __global__ void __launch_bounds__(256)
-k_update_uv(float* __restrict__ u, float* __restrict__ v, PcgBuffers b, Geom g, int ja, int jb, int* its_out)
+k_update_uv(float* __restrict__ u, float* __restrict__ v, PcgBuffers b, Geom g, int ja, int jb, int* its_out, size_t ps,
+            int its_stride)
 {
-    const PcgScalars* s = b.scal;
+    const PcgScalars* s = b.scal + blockIdx.z;                // pair blockIdx.z
     const int its = s->its;
-    if (blockIdx.x == 0 && threadIdx.x == 0 && its_out) *its_out = its;
+    if (blockIdx.x == 0 && threadIdx.x == 0 && its_out) its_out[(size_t)blockIdx.z * its_stride] = its;
     if (its == 0) return;
     const float alpha = s->alpha;
     const float* pu = b.pu[its & 1];
@@ -437,7 +562,7 @@ k_update_uv(float* __restrict__ u, float* __restrict__ v, PcgBuffers b, Geom g, 
     for (long long t = (long long)blockIdx.x * 256 + threadIdx.x; t < nunits; t += (long long)gridDim.x * 256) {
         const int jr = (int)(t / upr), i0 = (int)(t - (long long)jr * upr) * 4;
         if (i0 >= g.nx) continue;
-        const size_t off = g.at(i0, ja + jr);
+        const size_t off = g.at(i0, ja + jr) + (size_t)blockIdx.z * ps;
         float4 a = ld4(u + off), c = ld4(v + off);
         float4 xu = make_float4(0.f, 0.f, 0.f, 0.f), xv = xu;
         if (its > 1) { xu = ld4(b.xu + off); xv = ld4(b.xv + off); }
@@ -460,11 +585,12 @@ k_update_uv(float* __restrict__ u, float* __restrict__ v, PcgBuffers b, Geom g, 
 // second iteration on; iteration k leaves its p in pu[(k & 1) ^ 1], so the last one is in pu[its & 1] as for the
 // two-pass kernels.
 __global__ void __launch_bounds__(256)
-k_update_uv_fused(float* __restrict__ u, float* __restrict__ v, PcgBuffers b, Geom g, int ja, int jb, int* its_out)
+k_update_uv_fused(float* __restrict__ u, float* __restrict__ v, PcgBuffers b, Geom g, int ja, int jb, int* its_out, size_t ps,
+                  int its_stride)
 {
-    const PcgScalars* s = b.scal;
+    const PcgScalars* s = b.scal + blockIdx.z;                // pair blockIdx.z
     const int its = s->its;
-    if (blockIdx.x == 0 && threadIdx.x == 0 && its_out) *its_out = its;
+    if (blockIdx.x == 0 && threadIdx.x == 0 && its_out) its_out[(size_t)blockIdx.z * its_stride] = its;
     if (its == 0) return;
     const bool pending = (its & 1) != 0, havex = its >= 2;
     const float alpha = s->alpha;
@@ -473,7 +599,7 @@ k_update_uv_fused(float* __restrict__ u, float* __restrict__ v, PcgBuffers b, Ge
     for (long long t = (long long)blockIdx.x * 256 + threadIdx.x; t < nunits; t += (long long)gridDim.x * 256) {
         const int jr = (int)(t / upr), i0 = (int)(t - (long long)jr * upr) * 4;
         if (i0 >= g.nx) continue;
-        const size_t off = g.at(i0, ja + jr);
+        const size_t off = g.at(i0, ja + jr) + (size_t)blockIdx.z * ps;
         float4 a = ld4(u + off), c = ld4(v + off);
         float4 xu = make_float4(0.f, 0.f, 0.f, 0.f), xv = xu, p_u = xu, p_v = xu;
         if (havex) { xu = ld4(b.xu + off); xv = ld4(b.xv + off); }
@@ -579,21 +705,57 @@ void launch_pcg_pass2(const PcgBuffers& b, const Geom& g, int ja, int jb, int sm
 }
 
 void launch_update_uv(float* u, float* v, const PcgBuffers& b, const Geom& g, int ja, int jb,
-                      int* its_out, int sm_count, cudaStream_t st)
+                      int* its_out, int sm_count, cudaStream_t st, int npairs, size_t ps, int its_stride)
 {
     const long long nunits = (long long)(jb - ja) * (g.pitch >> 2);
     long long grid = (nunits + 255) / 256;
     if (grid > sm_count * 16) grid = sm_count * 16;
-    k_update_uv<<<(int)grid, 256, 0, st>>>(u, v, b, g, ja, jb, its_out);
+    k_update_uv<<<dim3((unsigned)grid, 1, npairs), 256, 0, st>>>(u, v, b, g, ja, jb, its_out, ps, its_stride);
 }
 
 void launch_update_uv_fused(float* u, float* v, const PcgBuffers& b, const Geom& g, int ja, int jb,
-                            int* its_out, int sm_count, cudaStream_t st)
+                            int* its_out, int sm_count, cudaStream_t st, int npairs, size_t ps, int its_stride)
 {
     const long long nunits = (long long)(jb - ja) * (g.pitch >> 2);
     long long grid = (nunits + 255) / 256;
     if (grid > sm_count * 16) grid = sm_count * 16;
-    k_update_uv_fused<<<(int)grid, 256, 0, st>>>(u, v, b, g, ja, jb, its_out);
+    k_update_uv_fused<<<dim3((unsigned)grid, 1, npairs), 256, 0, st>>>(u, v, b, g, ja, jb, its_out, ps, its_stride);
+}
+
+// Blocks per pair of the batched whole-solve kernel: one per 8 warp tasks of 8 rows each, at most 8 -- a function of
+// the level geometry alone.
+int coop_batch_blocks(const Geom& g, int ja, int jb)
+{
+    const int nstrips = (g.nx + 127) / 128, nsegs = (jb - ja + 7) / 8;
+    const int G = (nstrips * nsegs + 7) / 8;
+    return G < 1 ? 1 : (G > 8 ? 8 : G);
+}
+
+int coop_batch_pairs_per_launch(const Geom& g, int ja, int jb, int sm_count)
+{
+    static int per_sm = 0;
+    if (!per_sm) {
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_pcg_coop_batch, 256, 0) != cudaSuccess || per_sm < 1)
+            per_sm = 1;
+    }
+    const int n = sm_count * per_sm / coop_batch_blocks(g, ja, jb);
+    return n < 1 ? 1 : n;
+}
+
+int launch_pcg_coop_batch(const PcgBuffers& b, const Geom& g, int ja, int jb, int iters, int pair0, int npairs, size_t ps,
+                          double* partials, unsigned* bar, cudaStream_t st)
+{
+    P1Args a;
+    a.b = b; a.g = g; a.ja = ja; a.jb = jb; a.cur = 0; a.store_halo = 0;
+    a.nstrips = (g.nx + 127) / 128;
+    a.rs = 8;
+    a.nsegs = (jb - ja + a.rs - 1) / a.rs;
+    CoopBatch cb;
+    cb.G = coop_batch_blocks(g, ja, jb); cb.pair0 = pair0; cb.ps = ps; cb.partials = partials; cb.bar = bar;
+    if (cudaMemsetAsync(bar, 0, 2 * sizeof(unsigned) * npairs, st) != cudaSuccess) return -1;
+    void* args[] = { &a, &cb, &iters };
+    return cudaLaunchCooperativeKernel((const void*)k_pcg_coop_batch, dim3(cb.G * npairs), dim3(256), args, 0, st) == cudaSuccess
+               ? 0 : -1;
 }
 
 void launch_expand_coef(const PcgBuffers& b, const Geom& g, float* a5, float* a6, float* a7, float* a8, cudaStream_t st)

@@ -36,7 +36,7 @@ __global__ void k_fill_gk(float* GK, float factor, int R)
 template <int TX, int TY>
 __global__ void __launch_bounds__(TX* TY)
 k_blur_decimate(const float* __restrict__ src, Geom gs, float* __restrict__ dst, Geom gd,
-                int ja, int jb, float factor, const float* __restrict__ GK, int R, float scale, int nc)
+                int ja, int jb, float factor, const float* __restrict__ GK, int R, float scale, int nc, size_t ps)
 {
     extern __shared__ float sm[];
     float* gk = sm;                  // 2R+1 taps
@@ -47,7 +47,10 @@ k_blur_decimate(const float* __restrict__ src, Geom gs, float* __restrict__ dst,
     const int jj0 = ja + blockIdx.y * TY;
     // Reference quirk kept for parity: zoom_out reads the blurred plane without a channel
     // offset (:406), so every coarse-level channel is channel 0's blurred, decimated image.
-    dst += (size_t)blockIdx.z * gd.plane;
+    // blockIdx.z = pair * nc + channel; pairs are ps floats apart in both planes.
+    const unsigned pair = blockIdx.z / nc;
+    src += pair * ps;
+    dst += (size_t)(blockIdx.z - pair * nc) * gd.plane + pair * ps;
     const int i2 = (int)(ii / factor);                          // :369
     const int jj_last = min(jj0 + TY, jb) - 1;
     const int jsrc0 = (int)(jj0 / factor) - R;                  // first source row of the tile
@@ -125,13 +128,14 @@ __device__ __forceinline__ float4 grad_row(const float* __restrict__ f, const Ge
 template <bool VEC>
 __global__ void __launch_bounds__(256)
 k_gradient(const float* __restrict__ f, float* __restrict__ gx, float* __restrict__ gy, Geom g,
-           int ja, int jb, int nc)
+           int ja, int jb, int nc, size_t ps)
 {
     const int lane = threadIdx.x;
     const int i0 = (blockIdx.x * 32 + lane) * 4;
     const int js = ja + (blockIdx.y * 8 + threadIdx.y) * GRAD_ROWS;
     if (js >= jb) return;                                  // whole warp: js depends on threadIdx.y only
-    const size_t coff = (size_t)blockIdx.z * g.plane;
+    const unsigned pair = blockIdx.z / nc;            // blockIdx.z = pair * nc + channel
+    const size_t coff = (size_t)(blockIdx.z - pair * nc) * g.plane + pair * ps;
     f += coff; gx += coff;
     if (gy) gy += coff;
     const int lo = g.jlo(), hi = g.jhi() - 1;
@@ -221,13 +225,15 @@ __device__ __forceinline__ float bicubic(const float* __restrict__ in, const Geo
 __device__ __forceinline__ float zoom_u(int ii, float factorx) { return (float)((ii / factorx) - (0.5 - 0.5 / factorx)); }
 
 __global__ void __launch_bounds__(256)
-k_zoom_in(const float* __restrict__ flow, Geom gc, float* __restrict__ out, Geom gf, int ja, int jb, float sf)
+k_zoom_in(const float* __restrict__ flow, Geom gc, float* __restrict__ out, Geom gf, int ja, int jb, float sf, size_t ps)
 {
     __shared__ float V[8][ZOOM_VMAX];
     const int lane = threadIdx.x, wy = threadIdx.y;
     const int ibase = blockIdx.x * ZOOM_COLS;
     const int jj = ja + blockIdx.y * 8 + wy;
     if (jj >= jb || ibase >= gf.nx) return;                // whole warp
+    flow += blockIdx.z * ps;                               // pair blockIdx.z
+    out += blockIdx.z * ps;
     const float factorx = ((float)gf.nx / gc.nx);
     const float factory = ((float)gf.ny / gc.ny);
     const float vv = (float)((jj / factory) - (0.5 - 0.5 / factory));
@@ -287,34 +293,35 @@ size_t blur_decimate_smem_bytes(float factor, int R)
 }
 
 void launch_blur_decimate(const float* src, const Geom& gs, float* dst, const Geom& gd, int ja, int jb,
-                          float factor, const float* GK, int R, float scale, int nc, cudaStream_t st)
+                          float factor, const float* GK, int R, float scale, int nc, cudaStream_t st, int npairs, size_t ps)
 {
     if (jb <= ja) return;
     constexpr int TX = 32, TY = 8;
     const size_t smem = blur_decimate_smem_bytes(factor, R);
-    dim3 grid((gd.nx + TX - 1) / TX, (jb - ja + TY - 1) / TY, nc), block(TX, TY);
+    dim3 grid((gd.nx + TX - 1) / TX, (jb - ja + TY - 1) / TY, nc * npairs), block(TX, TY);
     static unsigned long long configured = 0;
     if (first_launch_on_device(&configured))
         cudaFuncSetAttribute(k_blur_decimate<TX, TY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BLUR_DECIMATE_SMEM_LIMIT);
-    k_blur_decimate<TX, TY><<<grid, block, smem, st>>>(src, gs, dst, gd, ja, jb, factor, GK, R, scale, nc);
+    k_blur_decimate<TX, TY><<<grid, block, smem, st>>>(src, gs, dst, gd, ja, jb, factor, GK, R, scale, nc, ps);
 }
 
-void launch_gradient(const float* f, float* gx, float* gy, const Geom& g, int ja, int jb, int nc, cudaStream_t st)
+void launch_gradient(const float* f, float* gx, float* gy, const Geom& g, int ja, int jb, int nc, cudaStream_t st,
+                     int npairs, size_t ps)
 {
     if (jb <= ja) return;
-    dim3 grid((g.nx + 127) / 128, (jb - ja + 8 * GRAD_ROWS - 1) / (8 * GRAD_ROWS), nc), block(32, 8);
+    dim3 grid((g.nx + 127) / 128, (jb - ja + 8 * GRAD_ROWS - 1) / (8 * GRAD_ROWS), nc * npairs), block(32, 8);
     const bool vec = (g.pitch & 3) == 0 && (g.plane & 3) == 0 &&
                      (((uintptr_t)f | (uintptr_t)gx | (uintptr_t)gy) & 15) == 0;
-    if (vec) k_gradient<true><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc);
-    else k_gradient<false><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc);
+    if (vec) k_gradient<true><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc, ps);
+    else k_gradient<false><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc, ps);
 }
 
 void launch_zoom_in(const float* flow, const Geom& gc, float* out, const Geom& gf, int ja, int jb, float sf,
-                    cudaStream_t st)
+                    cudaStream_t st, int npairs, size_t ps)
 {
     if (jb <= ja) return;
-    dim3 grid((gf.nx + ZOOM_COLS - 1) / ZOOM_COLS, (jb - ja + 7) / 8), block(32, 8);
-    k_zoom_in<<<grid, block, 0, st>>>(flow, gc, out, gf, ja, jb, sf);
+    dim3 grid((gf.nx + ZOOM_COLS - 1) / ZOOM_COLS, (jb - ja + 7) / 8, npairs), block(32, 8);
+    k_zoom_in<<<grid, block, 0, st>>>(flow, gc, out, gf, ja, jb, sf, ps);
 }
 
 }  // namespace octane
