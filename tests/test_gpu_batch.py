@@ -2,7 +2,12 @@
 
 A pair's result must not depend on the other pairs of the call (batch invariance), must meet the single-pair gates
 against the CPU oracle and the reference's fixtures, and must agree with the single-pair dispatcher up to the
-reordered dot-product sums of the per-pair PCG groups."""
+reordered dot-product sums of the per-pair PCG groups.
+
+Every pair of a batch is distinct where the oracle judges it: a kernel that reads pair 0's planes, navigation or
+heights for every pair cannot pass.  The cases reach every group size of the cooperative small-level solver
+(k_pcg_coop_batch), batches that need several waves and end with a one-pair wave, pairs that stop at the build next
+to pairs that reach the iteration cap, every navigation grid and the workspace state kept between calls."""
 import numpy as np
 import pytest
 
@@ -14,6 +19,7 @@ from octane_b200 import synthetic as S
 pytestmark = pytest.mark.gpu
 KEYS_F = ("uPix", "vPix")
 KEYS_S = ("uVal", "vVal", "uVal2", "vVal2", "CTP")
+COOP_PER_SM = 2        # k_pcg_coop_batch: __launch_bounds__(256, 2), 2 co-resident blocks per SM
 
 
 @pytest.fixture(scope="module")
@@ -26,6 +32,11 @@ def bctx():
 def tdev(a):
     import torch
     return torch.from_numpy(np.ascontiguousarray(a)).cuda()
+
+
+def sm_count():
+    import torch
+    return torch.cuda.get_device_properties(0).multi_processor_count
 
 
 def run_batch(ctx, img1, img2, navs, t1, t2, p, cth=None, nc=1):
@@ -55,6 +66,55 @@ def meso_inputs(npairs, n=500, seed0=100):
     return img1, img2, np.stack([cth] * npairs), [nav] * npairs, [0.0] * npairs, [dt] * npairs
 
 
+def distinct_inputs(npairs, nx, ny, seed0, nc=1):
+    """npairs distinct nx x ny pairs (nc channels: seeds + 100 ch, as cases.variational_inputs), each with its own
+    cloud-top heights and times, all on the 2 km mesoscale grid"""
+    xs, ys, xo, yo, dt = S.SECTORS["meso_2km"]
+    img1, img2 = [], []
+    for k in range(npairs):
+        chans = [S.make_pair(nx, ny, seed0 + k + 100 * ch)[:2] for ch in range(nc)]
+        img1.append(np.stack([a for a, _ in chans]) if nc > 1 else chans[0][0])
+        img2.append(np.stack([b for _, b in chans]) if nc > 1 else chans[0][1])
+    yy, xx = np.mgrid[0:ny, 0:nx].astype(np.float32)
+    cth = np.stack([(7500.0 + 7400.0 * np.sin(xx / (30.0 + k) + k) * np.cos(yy / 30.0)).astype(np.float32)
+                    for k in range(npairs)])
+    t1 = [100.0 * k for k in range(npairs)]
+    return (np.stack(img1).astype(np.float32), np.stack(img2).astype(np.float32), cth,
+            [ob.goes_nav(xs, ys, xo, yo)] * npairs, t1, [t + dt for t in t1])
+
+
+def check_vs_oracle(oracle, out, its, b, img1, img2, p_over, nc, tag, want=None):
+    """pair b of a batch against its own oracle run (or `want`, a stored one) with the gates of
+    test_flow_matches_oracle: mean |d| < 1e-4 px, max < 2e-3 px, equal iteration counts per solve"""
+    uo, vo, its_o = want if want is not None else oracle.variational_flow(img1, img2, oracle.params(**p_over), None, None,
+                                                                        nc=nc)
+    du, dv = np.abs(out["uPix"][b] - uo), np.abs(out["vPix"][b] - vo)
+    print(f"{tag} pair {b}: max |d u, v| vs the oracle = {max(du.max(), dv.max()):.3e} px, "
+          f"oracle iterations {int(its_o.min())}..{int(its_o.max())}")
+    assert du.mean() < 1e-4 and dv.mean() < 1e-4, (tag, b, du.mean(), dv.mean())
+    assert du.max() < 2e-3 and dv.max() < 2e-3, (tag, b, du.max(), dv.max())
+    bad = [s for s in range(len(its_o)) if its[b][s] != its_o[s]]
+    assert not bad, f"{tag} pair {b}: iterations differ at solves {bad}: batch {list(its[b][bad])}, oracle {list(its_o[bad])}"
+    return uo, vo, its_o
+
+
+# ---- small-level solver geometry (mirror of pcg.cu coop_batch_blocks and ctx.cu run_levels_batch) ----------------
+def coop_blocks(nx, rows):
+    """blocks per pair of k_pcg_coop_batch: one per 8 warp tasks of 128 columns x 8 rows, clamped to 1..8"""
+    g = ((nx + 127) // 128 * ((rows + 7) // 8) + 7) // 8
+    return min(max(g, 1), 8)
+
+
+def small_level(nx, rows):
+    """a level the batched call solves in cooperative launches (the merged-reduction kernels need nx >= 512 and
+    at least 64 rows); the others run the single-pair PCG kernels pair by pair"""
+    return nx < 512 or rows < 64
+
+
+def small_level_groups(oracle, nx, ny, p):
+    return [coop_blocks(a, b) for a, b in oracle.level_dims(nx, ny, kiters=p.kiters, scaleF=p.scaleF) if small_level(a, b)]
+
+
 def test_batch_invariance(bctx):
     """64 pairs of 500^2 with CTH: one call, a shuffled call and ragged sub-batches give the same bits per pair"""
     img1, img2, cth, navs, t1, t2 = meso_inputs(64)
@@ -76,28 +136,212 @@ def test_batch_invariance(bctx):
 
 VAR_CASES = sorted(k for k, c in cases.VARIATIONAL.items() if not c.get("first_guess") and
                    cases.variational_inputs(c)[2] is None)
+# judged by the oracle alone (no reference fixture): three channels, and the stop after one or two iterations
+# (k_pcg_coop_batch's XM_NONE-only and XM_INIT exits, k_update_uv with its = 1 and 2)
+EXTRA_VAR_CASES = {
+    "var_112x88_nc3": dict(nx=112, ny=88, seed=18, kind="vortex", nc=3),
+    "var_96x80_shift_cg1": dict(cases.VARIATIONAL["var_96x80_shift"], params=dict(cgiters=1)),
+    "var_96x80_shift_cg2": dict(cases.VARIATIONAL["var_96x80_shift"], params=dict(cgiters=2)),
+}
 
 
-@pytest.mark.parametrize("name", VAR_CASES)
+@pytest.mark.parametrize("name", VAR_CASES + sorted(EXTRA_VAR_CASES))
 def test_batch_matches_oracle_and_fixture(bctx, oracle, name):
-    """each of three copies of a pair meets the single-pair gates against the oracle and the reference fixture"""
-    c = cases.VARIATIONAL[name]
+    """four distinct pairs: pair 0 is the case's input, pairs 1-3 the case regenerated with seed + 1000 k; each meets
+    the single-pair gates against its own oracle run, and pair 0 also against the reference fixture"""
+    c = cases.VARIATIONAL.get(name) or EXTRA_VAR_CASES[name]
     nc = c.get("nc", 1)
-    img1, img2, _, _ = cases.variational_inputs(c)
+    ins = [cases.variational_inputs(dict(c, seed=c["seed"] + 1000 * k))[:2] for k in range(4)]
     p = ob.default_params(**c.get("params", {}))
     xs, ys, xo, yo, dt = S.SECTORS["meso_2km"]
-    navs = [ob.goes_nav(xs, ys, xo, yo)] * 3
-    out, _, its = run_batch(bctx, np.stack([img1] * 3), np.stack([img2] * 3), navs, [0.0] * 3, [dt] * 3, p, nc=nc)
-    uo, vo, its_o = oracle.variational_flow(img1, img2, oracle.params(**c.get("params", {})), None, None, nc=nc)
+    navs = [ob.goes_nav(xs, ys, xo, yo)] * 4
+    out, _, its = run_batch(bctx, np.stack([a for a, _ in ins]), np.stack([b for _, b in ins]), navs, [0.0] * 4, [dt] * 4,
+                            p, nc=nc)
+    for b, (i1, i2) in enumerate(ins):
+        check_vs_oracle(oracle, out, its, b, i1, i2, c.get("params", {}), nc, name)
+    if name not in cases.VARIATIONAL:
+        if "cgiters" in c.get("params", {}):                  # every solve stops at the cap
+            assert (its == c["params"]["cgiters"]).all()
+        return
     g = load_golden(name)
+    du, dv = np.abs(out["uPix"][0] - g["u"]), np.abs(out["vPix"][0] - g["v"])
+    assert du.mean() < 1e-3 and dv.mean() < 1e-3 and du.max() < 1e-2 and dv.max() < 1e-2
+    assert max(du.max(), dv.max()) < max(20 * float(g["spread"].max()), 2e-4)
+
+
+# (nx, ny): the small levels of these shapes use every group size 1..8 of k_pcg_coop_batch
+GROUP_SHAPES = [(120, 160), (200, 192), (256, 224), (264, 240), (300, 104)]
+
+
+def test_batch_shapes_cover_every_group_size(oracle):
+    p = ob.default_params()
+    per_shape = {s: small_level_groups(oracle, *s, p) for s in GROUP_SHAPES}
+    covered = sorted(set().union(*per_shape.values()))
+    print(f"group sizes per shape (coarsest first): {per_shape}; covered {covered}")
+    assert covered == list(range(1, 9))
+    assert any(nx % 128 == 0 for nx, _ in GROUP_SHAPES) and any(nx % 128 for nx, _ in GROUP_SHAPES)
+
+
+@pytest.mark.parametrize("shape", GROUP_SHAPES, ids=lambda s: f"{s[0]}x{s[1]}")
+def test_batch_group_sizes_match_oracle(bctx, oracle, shape):
+    """three distinct pairs per shape, each against its own oracle run"""
+    nx, ny = shape
+    p = ob.default_params()
+    img1, img2, _, navs, t1, t2 = distinct_inputs(3, nx, ny, seed0=400 + nx)
+    out, _, its = run_batch(bctx, img1, img2, navs, t1, t2, p)
+    tag = f"{nx}x{ny} G={small_level_groups(oracle, nx, ny, p)}"
     for b in range(3):
-        u, v = out["uPix"][b], out["vPix"][b]
-        assert np.abs(u - uo).mean() < 1e-4 and np.abs(v - vo).mean() < 1e-4
-        assert np.abs(u - uo).max() < 2e-3 and np.abs(v - vo).max() < 2e-3
-        assert list(its[b]) == list(its_o)
-        du, dv = np.abs(u - g["u"]), np.abs(v - g["v"])
-        assert du.mean() < 1e-3 and dv.mean() < 1e-3 and du.max() < 1e-2 and dv.max() < 1e-2
-        assert max(du.max(), dv.max()) < max(20 * float(g["spread"].max()), 2e-4)
+        check_vs_oracle(oracle, out, its, b, img1[b], img2[b], {}, 1, tag)
+
+
+def test_batch_waves_and_mixed_exits(bctx, oracle):
+    """2 floor(2 sm / 8) + 1 distinct 264x240 pairs: the finest level (8 blocks per pair) runs in three waves and
+    132x120 (4 blocks) in two, each ending with a one-pair wave.  Pairs with img1 == img2 (zero rhs: no iteration in
+    any solve) sit at index 0, at both sides of the first wave boundary and alone in the last wave; the others mostly
+    reach the 30-iteration cap"""
+    nx, ny = 264, 240
+    p = ob.default_params()
+    sms = sm_count()
+    per8 = sms * COOP_PER_SM // 8
+    B = 2 * per8 + 1
+    groups = small_level_groups(oracle, nx, ny, p)
+    assert groups[-1] == 8 and B % per8 == 1 and B % (sms * COOP_PER_SM // 4) == 1 and 4 in groups
+    img1, img2, _, navs, t1, t2 = distinct_inputs(B, nx, ny, seed0=500)
+    still = [0, per8 - 1, per8, B - 1]
+    for b in still:
+        img2[b] = img1[b]
+    run_batch(bctx, img1[1:2], img2[1:2], navs[:1], t1[:1], t2[:1], p)
+    one = bctx.stats().kernel_launches
+    out, _, its = run_batch(bctx, img1, img2, navs, t1, t2, p)
+    many = bctx.stats().kernel_launches
+    want = sum(3 * p.liters * (-(-B // max(1, sms * COOP_PER_SM // g)) - 1) for g in groups)
+    print(f"{B} pairs of {nx}x{ny} on {sms} SMs: group sizes {groups}, kernel launches 1 pair {one}, "
+          f"{B} pairs {many}, delta {many - one} (expected {want})")
+    assert many - one == want
+    capped = 0
+    for b in range(B):
+        uo, vo, its_o = check_vs_oracle(oracle, out, its, b, img1[b], img2[b], {}, 1, f"waves {nx}x{ny}")
+        if b in still:
+            assert its_o.max() == 0 and not uo.any() and not vo.any()
+            assert not out["uPix"][b].any() and not out["vPix"][b].any()
+        capped += int((its_o == p.cgiters).any())
+    assert capped > 0
+
+
+@pytest.fixture(scope="module")
+def large_pairs(oracle):
+    img1, img2, _, navs, t1, t2 = distinct_inputs(3, 768, 640, seed0=600)
+    want = [oracle.variational_flow(img1[b], img2[b], oracle.params()) for b in range(3)]
+    return img1, img2, navs, t1, t2, want
+
+
+@pytest.mark.parametrize("solver", [1, 0])
+def test_batch_large_levels_match_oracle(oracle, large_pairs, solver):
+    """three distinct 768x640 pairs: the finest level runs the single-pair PCG kernels pair by pair, the coarser ones
+    the cooperative solver with 2, 5 and 8 blocks per pair"""
+    img1, img2, navs, t1, t2, want = large_pairs
+    p = ob.default_params()
+    assert small_level_groups(oracle, 768, 640, p) == [2, 5, 8]
+    ctx = ob.Context(0)
+    try:
+        ctx.set_solver(solver)
+        out, _, its = run_batch(ctx, img1, img2, navs, t1, t2, p)
+        for b in range(3):
+            check_vs_oracle(oracle, out, its, b, img1[b], img2[b], {}, 1, f"768x640 solver {solver}", want=want[b])
+    finally:
+        ctx.close()
+
+
+def ctp_model(cth, ir):
+    """the reference's host packing of CTP (src/oct_optical_flow.cc:71-88): float arithmetic, conversion to int
+    (truncation), then to short (16-bit wrap)"""
+    f = np.float32
+    x = (cth.astype(f) - f(300)) * f(100) if ir else cth.astype(f)
+    return x.astype(np.int32).astype(np.int16)
+
+
+def grid_batch(grid):
+    """(navs, t1, t2, moved pairs, flags) of four pairs on one navigation grid, each with its own times"""
+    if grid in ("goes", "pixuv"):
+        cs = [cases.NAVIGATION[n] for n in ("nav_goes_meso", "nav_goes_limb", "nav_goes_2km_offset", "nav_moved")]
+        named = [cases.nav_constants(c) for c in cs]
+    elif grid == "polar":
+        named = [cases.nav_constants(cases.NAVIGATION[n]) for n in ("nav_polar", "nav_polar_pole")] * 2
+    else:
+        kw, extra, t1, t2, flags = cases.nav_constants(cases.NAVIGATION["nav_merc"])
+        kw2 = dict(kw, xOffset=kw["xOffset"] + 84000.0, yOffset=kw["yOffset"] - 1500000.0)
+        named = [(kw, extra, t1, t2, flags), (kw2, extra, t1, t2, flags)] * 2
+    navs, t1s, t2s = [], [], []
+    for b, (kw, extra, t1, t2, _) in enumerate(named):
+        nav = ob.goes_nav(**kw)
+        for k, val in extra.items():
+            setattr(nav, k, val)
+        navs.append(nav)
+        t1s.append(t1 + 37.0 * b)
+        t2s.append(t1 + 37.0 * b + (t2 - t1) * (1.0 + 0.5 * b))
+    flags = dict(pixuv=int(grid == "pixuv"), dopolar=int(grid == "polar"), domerc=int(grid == "merc"))
+    moved = [b for b, (kw, *_) in enumerate(named) if "g2xOffset" in kw]
+    return navs, t1s, t2s, moved, flags
+
+
+@pytest.mark.parametrize("ir", [0, 1])
+@pytest.mark.parametrize("grid", ["goes", "polar", "merc", "pixuv"])
+def test_batch_navigation_and_ctp_per_pair(bctx, grid, ir):
+    """every pair navigates with its own nav and times: its four short planes are, bit for bit, what the single-pair
+    navigation gives on the batch's own flow; CTP packs each pair's own heights as the reference's host code does"""
+    nx, ny = 120, 90
+    navs, t1, t2, want_moved, flags = grid_batch(grid)
+    B = len(navs)
+    img1, img2, cth, _, _, _ = distinct_inputs(B, nx, ny, seed0=700)
+    cth[:, 0, :12] = [-50.0, 0.0, 299.99, 300.0, 627.6, 627.7, 655.35, 12000.5, 19999.9, 32767.0, 32768.9, 65535.5]
+    cth[:, 1, :3] = [-32768.0, -32769.5, 40000.7]
+    p = ob.default_params(doCTH=1, ir=ir, **flags)
+    out, moved, _ = run_batch(bctx, img1, img2, navs, t1, t2, p, cth)
+    assert moved == want_moved
+    import torch
+    for b in range(B):
+        ref = [torch.full((ny, nx), 7, dtype=torch.int16, device="cuda") for _ in range(4)]
+        _, mv = bctx.oct_pix2uv_cuda(navs[b], t1[b], t2[b], tdev(out["uPix"][b]), tdev(out["vPix"][b]), *ref, p)
+        assert mv == (b in want_moved)
+        for k, r in zip(("uVal", "vVal", "uVal2", "vVal2"), ref):
+            assert np.array_equal(out[k][b], r.cpu().numpy()), (grid, b, k)
+        assert np.array_equal(out["CTP"][b], ctp_model(cth[b], ir)), (grid, ir, b)
+    # (the limb sector lies wholly beyond the limb cut: its speeds are zero)
+    assert sum(bool(out["uVal"][b].any() and out["vVal"][b].any()) for b in range(B) if b not in want_moved) >= 2
+
+
+def test_batch_state_across_calls():
+    """batches and single-pair calls of several sizes on one context (re-plans, a workspace that grows and drops the
+    captured PCG graphs, batch buffers sized by an earlier call) give what a fresh context gives, bit for bit"""
+    p = ob.default_params(doCTH=1)
+    batches = [distinct_inputs(16, 264, 240, seed0=800), distinct_inputs(5, 200, 192, seed0=820, nc=2),
+               distinct_inputs(40, 264, 240, seed0=840)]
+    ncs = [1, 2, 1]
+    i1, i2, cth, navs, t1, t2 = distinct_inputs(1, 768, 640, seed0=900)
+
+    def batch(ctx, k):
+        img1, img2, bcth, bnavs, bt1, bt2 = batches[k]
+        return run_batch(ctx, img1, img2, bnavs, bt1, bt2, p, bcth, nc=ncs[k])
+
+    def one(ctx):
+        return single(ctx, i1[0], i2[0], navs[0], t1[0], t2[0], p, cth[0])
+
+    ctx = ob.Context(0)
+    try:
+        got = [batch(ctx, 0), one(ctx), batch(ctx, 1), batch(ctx, 2), one(ctx)]
+    finally:
+        ctx.close()
+    for k, pos in ((0, 0), (1, 2), (2, 3)):
+        fresh = ob.Context(0)
+        try:
+            want = batch(fresh, k)
+        finally:
+            fresh.close()
+        for key in want[0]:
+            assert np.array_equal(got[pos][0][key], want[0][key]), (k, key)
+        assert got[pos][1] == want[1] and np.array_equal(got[pos][2], want[2]), k
+    for key in got[1]:
+        assert np.array_equal(got[4][key], got[1][key]), key
 
 
 def single(ctx, a, b, nav, t1, t2, p, cth):

@@ -172,7 +172,7 @@ def test_stage_zoom_in_bit_exact(ctx, oracle, dims):
 
 
 @pytest.mark.parametrize("gnc", [0, 1, 2])
-@pytest.mark.parametrize("nc", [1, 2])
+@pytest.mark.parametrize("nc", [1, 2, 3])
 def test_stage_build_and_pcg(ctx, oracle, gnc, nc):
     import torch
     nx, ny = 150, 110
