@@ -254,16 +254,35 @@ int octane_optical_flow_dev(octane_ctx* ctx, const float* d_img1, const float* d
  * Small pyramid levels solve all pairs in one cooperative launch (each pair on its own group of blocks, with its own
  * barrier and stop rule); a pair's result does not depend on the other pairs of the call.  Stream-ordered, no host
  * synchronisation; moved_out (host, npairs, may be NULL) gets 1 for each pair whose sector moved (its four short
- * planes are zero).  OCTANE_EINVAL for npairs < 1, a first guess, dosrsal or a banded context; OCTANE_ENOMEM when
- * the npairs workspaces do not fit.  The context stays usable after either.  octane_get_stats then reports the
- * call's kernel launches and pair 0's iteration counts. */
+ * planes are zero).  OCTANE_EINVAL for npairs < 1, a first guess, dosrsal or a banded context (a first guess and
+ * -srsal go through octane_optical_flow_batch_ex_dev, which shares this call's body); OCTANE_ENOMEM when the npairs
+ * workspaces do not fit.  The context stays usable after either.  octane_get_stats then reports the call's kernel
+ * launches and pair 0's iteration counts. */
 int octane_optical_flow_batch_dev(octane_ctx* ctx, int npairs, const float* d_img1, const float* d_img2,
                                   const float* d_cth, int nx, int ny, int nc, const octane_nav* nav,
                                   const double* t1, const double* t2, const octane_params* p,
                                   float* d_upix, float* d_vpix, short* d_U, short* d_V, short* d_U_raw,
                                   short* d_V_raw, short* d_ctp, int* moved_out);
-/* PCG iterations of every solve of every pair of the last batched call: its[pair * n_solves + solve].  npairs must
- * be that call's.  Synchronises the context's stream. */
+/* octane_optical_flow_batch_dev with a first guess and -srsal: per pair, what octane_optical_flow_dev does with the
+ * same flags.  With neither flag set the results are octane_optical_flow_batch_dev's, bit for bit.
+ * - p->first_guess: d_fg_u / d_fg_v (npairs x ny x nx, only read; NULL otherwise) are each pair's first guess.  They
+ *   may be d_upix / d_vpix themselves (octane_optical_flow_dev's in/out convention): they are copied into the
+ *   workspaces before any output is written.  The hint term is built on the levels with lambdac != 0.
+ * - p->dosrsal: each pair's d_upix / d_vpix is smoothed with its own heights d_cth (npairs x ny x nx), in one launch
+ *   for all pairs, after the CTP pack and the navigation: the short planes and CTP come from the unsmoothed flow.
+ *   A pair whose sector moved is smoothed too.
+ * OCTANE_EINVAL for npairs < 1, first_guess without both fg pointers, dosrsal without d_cth or with nx or ny <= 18,
+ * doCTH without d_cth / d_ctp and a banded context; OCTANE_ENOMEM when the workspaces or the -srsal staging
+ * (2 x npairs x ny x nx floats) do not fit.  Every allocation is made before anything is enqueued: the context stays
+ * usable after any refusal. */
+int octane_optical_flow_batch_ex_dev(octane_ctx* ctx, int npairs, const float* d_img1, const float* d_img2,
+                                     const float* d_fg_u, const float* d_fg_v, const float* d_cth,
+                                     int nx, int ny, int nc, const octane_nav* nav,
+                                     const double* t1, const double* t2, const octane_params* p,
+                                     float* d_upix, float* d_vpix, short* d_U, short* d_V, short* d_U_raw,
+                                     short* d_V_raw, short* d_ctp, int* moved_out);
+/* PCG iterations of every solve of every pair of the last batched call (either of the two above):
+ * its[pair * n_solves + solve].  npairs must be that call's.  Synchronises the context's stream. */
 int octane_batch_cg_iterations(octane_ctx* ctx, int* its, int npairs);
 
 int octane_navcal_dev(octane_ctx* ctx, const short* d_rad, const short* d_x, const short* d_y, int nx, int ny,

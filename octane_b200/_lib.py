@@ -71,7 +71,7 @@ EXPORTS = [
     "octane_band_plan", "octane_comm_unique_id", "octane_comm_init", "octane_comm_rank",
     "octane_variational_flow_band_dev", "octane_variational_flow_band_fg_dev", "octane_pix2uv_band_dev",
     "octane_srsal_band_dev", "octane_stream_submit", "octane_stream_submit_fg", "octane_stream_wait",
-    "octane_optical_flow_batch_dev", "octane_batch_cg_iterations",
+    "octane_optical_flow_batch_dev", "octane_optical_flow_batch_ex_dev", "octane_batch_cg_iterations",
 ]
 
 _lib = None
@@ -118,6 +118,8 @@ def load() -> C.CDLL:
     L.octane_optical_flow_dev.argtypes = [vp, vp, vp, vp, i, i, i, NP, d, d, PP, vp, vp, vp, vp, vp, vp, vp]
     L.octane_optical_flow_batch_dev.argtypes = [vp, i, vp, vp, vp, i, i, i, NP, C.POINTER(d), C.POINTER(d), PP,
                                                 vp, vp, vp, vp, vp, vp, vp, ip]
+    L.octane_optical_flow_batch_ex_dev.argtypes = [vp, i, vp, vp, vp, vp, vp, i, i, i, NP, C.POINTER(d), C.POINTER(d),
+                                                   PP, vp, vp, vp, vp, vp, vp, vp, ip]
     L.octane_batch_cg_iterations.argtypes = [vp, ip, i]
     CP = C.POINTER(Cal)
     L.octane_navcal.argtypes = [vp, vp, vp, vp, i, i, NP, CP, vp, vp, vp]

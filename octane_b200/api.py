@@ -345,20 +345,18 @@ class Context:
             self._before_torch()
         return rc
 
-    def oct_optical_flow_batch_dev(self, geo1, geo2, nav_list, t1_list, t2_list, p: Params, out: dict, cth=None,
-                                   nc: int = 1):
-        """Many same-size pairs in one call, on torch CUDA tensors shaped [B, ny, nx] (or [B, nc, ny, nx] for the
-        images).  `out` holds [B, ny, nx] tensors under uPix, vPix (float32), uVal, vVal, uVal2, vVal2 and, with
-        doCTH, CTP (int16).  Stream-ordered like oct_optical_flow_dev.  Returns the list of pairs whose sector moved
-        (their four navigated planes are zero); cg_iterations() gives the per-pair iteration counts."""
+    def _batch_args(self, geo1, geo2, nav_list, t1_list, t2_list, out: dict, cth, fg_u=None, fg_v=None):
+        """the checks and ctypes arguments both batched calls share: (B, nx, ny, navs, t1, t2, moved)"""
         B = int(geo1.shape[0])
         ny, nx = geo1.shape[-2:]
-        for name, a in (("geo1", geo1), ("geo2", geo2), ("cth", cth), ("uPix", out.get("uPix")), ("vPix", out.get("vPix"))):
+        for name, a in (("geo1", geo1), ("geo2", geo2), ("cth", cth), ("uPix", out.get("uPix")), ("vPix", out.get("vPix")),
+                        ("fg_u", fg_u), ("fg_v", fg_v)):
             _require(name, a, "float32", cuda=True)
         for name in ("uVal", "vVal", "uVal2", "vVal2", "CTP"):
             _require(name, out.get(name), "int16", cuda=True)
-        shapes = {tuple(a.shape[-2:]) for a in (geo2, cth, *out.values()) if a is not None}
-        if shapes != {(ny, nx)} or any(int(a.shape[0]) != B for a in (geo2, cth, *out.values()) if a is not None):
+        arrays = [a for a in (geo2, cth, fg_u, fg_v, *out.values()) if a is not None]
+        shapes = {tuple(a.shape[-2:]) for a in arrays}
+        if shapes != {(ny, nx)} or any(int(a.shape[0]) != B for a in arrays):
             raise ValueError("every array must be [B, ny, nx] (images [B, nc, ny, nx]) with the same B, ny, nx")
         if not (len(nav_list) == len(t1_list) == len(t2_list) == B):
             raise ValueError("nav_list, t1_list and t2_list need one entry per pair")
@@ -366,11 +364,34 @@ class Context:
         t1 = (C.c_double * max(B, 1))(*t1_list)
         t2 = (C.c_double * max(B, 1))(*t2_list)
         moved = (C.c_int * max(B, 1))()
+        return B, nx, ny, navs, t1, t2, moved
+
+    def oct_optical_flow_batch_dev(self, geo1, geo2, nav_list, t1_list, t2_list, p: Params, out: dict, cth=None,
+                                   nc: int = 1):
+        """Many same-size pairs in one call, on torch CUDA tensors shaped [B, ny, nx] (or [B, nc, ny, nx] for the
+        images).  `out` holds [B, ny, nx] tensors under uPix, vPix (float32), uVal, vVal, uVal2, vVal2 and, with
+        doCTH, CTP (int16).  Stream-ordered like oct_optical_flow_dev.  Returns the list of pairs whose sector moved
+        (their four navigated planes are zero); cg_iterations() gives the per-pair iteration counts."""
+        B, nx, ny, navs, t1, t2, moved = self._batch_args(geo1, geo2, nav_list, t1_list, t2_list, out, cth)
         self._after_torch()
         self._check(self._L.octane_optical_flow_batch_dev(
             self._h, B, _ptr(geo1), _ptr(geo2), _ptr(cth), nx, ny, nc, navs, t1, t2, C.byref(p), _ptr(out["uPix"]),
             _ptr(out["vPix"]), _ptr(out["uVal"]), _ptr(out["vVal"]), _ptr(out["uVal2"]), _ptr(out["vVal2"]),
             _ptr(out.get("CTP")), moved))
+        self._before_torch()
+        return [b for b in range(B) if moved[b]]
+
+    def oct_optical_flow_batch_ex_dev(self, geo1, geo2, nav_list, t1_list, t2_list, p: Params, out: dict, cth=None,
+                                      nc: int = 1, *, fg_u=None, fg_v=None):
+        """oct_optical_flow_batch_dev with a first guess (p.first_guess: fg_u / fg_v, [B, ny, nx] float32 CUDA
+        tensors, only read; they may be out["uPix"] / out["vPix"]) and -srsal (p.dosrsal: each pair's uPix / vPix
+        smoothed with its own heights cth after the navigation).  Returns the list of pairs whose sector moved."""
+        B, nx, ny, navs, t1, t2, moved = self._batch_args(geo1, geo2, nav_list, t1_list, t2_list, out, cth, fg_u, fg_v)
+        self._after_torch()
+        self._check(self._L.octane_optical_flow_batch_ex_dev(
+            self._h, B, _ptr(geo1), _ptr(geo2), _ptr(fg_u), _ptr(fg_v), _ptr(cth), nx, ny, nc, navs, t1, t2, C.byref(p),
+            _ptr(out["uPix"]), _ptr(out["vPix"]), _ptr(out["uVal"]), _ptr(out["vVal"]), _ptr(out["uVal2"]),
+            _ptr(out["vVal2"]), _ptr(out.get("CTP")), moved))
         self._before_torch()
         return [b for b in range(B) if moved[b]]
 

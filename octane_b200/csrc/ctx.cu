@@ -736,7 +736,12 @@ int ensure_stage(octane_ctx* c, size_t bytes)
     CUDA_OK(cudaStreamSynchronize(c->stream));
     if (c->stage) cudaFree(c->stage);
     c->stage = nullptr; c->stage_bytes = 0;
-    CUDA_OK(cudaMalloc(&c->stage, bytes));
+    if (cudaMalloc(&c->stage, bytes) != cudaSuccess) {
+        cudaGetLastError();                    // not sticky: later calls must not see it
+        c->stage = nullptr;
+        set_err("cudaMalloc (staging): out of device memory");
+        return OCTANE_ENOMEM;
+    }
     c->stage_bytes = bytes;
     return OCTANE_OK;
 }
@@ -1114,7 +1119,8 @@ int octane_pix2uv_band_dev(octane_ctx* c, const octane_nav* nav, double t1, doub
 
 namespace {
 constexpr int SRSAL_R = 18;    // radius of the -srsal window (src/oct_srsal_cuda.cu:78-79)
-int srsal_enqueue(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int nx, int ny, float* tmp_u, float* tmp_v);
+int srsal_enqueue(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int nx, int ny, float* tmp_u, float* tmp_v,
+                  int npairs = 1);
 size_t srsal_band_stage_bytes(int nx, int ny, int own0, int own1);
 int srsal_band_enqueue(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int nx, int ny, int own0, int own1, char* stage);
 bool srsal_bands_ok(int ny, int world);
@@ -1218,9 +1224,10 @@ PcgBuffers pair_buffers(const PcgBuffers& b0, int b, size_t ps)
     return q;
 }
 
-// run_levels for npairs pairs in the batch workspace (pair stride ps floats); one GPU, no first guess.  Per-pixel
-// stages are one launch for all pairs; small levels solve all pairs in cooperative launches with one barrier per
-// pair (launch_pcg_coop_batch), large levels run the single-pair PCG kernels pair by pair.
+// run_levels for npairs pairs in the batch workspace (pair stride ps floats); one GPU.  With a first guess, each
+// pair's hint is in its own uh / vh planes.  Per-pixel stages are one launch for all pairs; small levels solve all
+// pairs in cooperative launches with one barrier per pair (launch_pcg_coop_batch), large levels run the single-pair
+// PCG kernels pair by pair.
 int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
 {
     const Plan& pl = c->plan;
@@ -1240,6 +1247,7 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
         const Geom& g = L.g;
         const bool finest = (k == K - 1);
         float *g1 = finest ? B.img1 : B.g1c, *g2 = finest ? B.img2 : B.g2c;
+        const float *hu = nullptr, *hv = nullptr;
         if (k > 0) {
             const Level& Lc = pl.lv[k - 1];
             launch_zoom_in(B.ut, Lc.g, B.u, g, L.own0, L.own1, sf, st, npairs, ps);
@@ -1252,10 +1260,24 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
             launch_blur_decimate(B.img1, gF, B.g1c, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, 1.f, nc, st, npairs, ps);
             launch_blur_decimate(B.img2, gF, B.g2c, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, 1.f, nc, st, npairs, ps);
             c->launches += 3;
+            if (p.first_guess) {
+                launch_blur_decimate(B.uh, gF, B.hu, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, L.factor, 1, st, npairs, ps);
+                launch_blur_decimate(B.vh, gF, B.hv, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, L.factor, 1, st, npairs, ps);
+                c->launches += 2;
+                hu = B.hu; hv = B.hv;
+            }
+        } else if (p.first_guess) {
+            hu = B.uh; hv = B.vh;
         }
         if (k == 0) {
-            CUDA_OK(cudaMemset2DAsync(B.u, S, 0, (size_t)g.plane * sizeof(float), npairs, st));
-            CUDA_OK(cudaMemset2DAsync(B.v, S, 0, (size_t)g.plane * sizeof(float), npairs, st));
+            const size_t w = (size_t)g.plane * sizeof(float);
+            if (hu) {
+                CUDA_OK(cudaMemcpy2DAsync(B.u, S, hu, S, w, npairs, cudaMemcpyDeviceToDevice, st));
+                CUDA_OK(cudaMemcpy2DAsync(B.v, S, hv, S, w, npairs, cudaMemcpyDeviceToDevice, st));
+            } else {
+                CUDA_OK(cudaMemset2DAsync(B.u, S, 0, w, npairs, st));
+                CUDA_OK(cudaMemset2DAsync(B.v, S, 0, w, npairs, st));
+            }
         }
         launch_gradient(g1, B.g1x, B.g1y, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
         launch_gradient(g2, B.g2x, B.g2y, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
@@ -1266,7 +1288,8 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
         f.g1 = g1; f.g1x = B.g1x; f.g1y = B.g1y;
         f.g2 = g2; f.g2x = B.g2x; f.g2y = B.g2y; f.g2xx = B.g2xx; f.g2xy = B.g2xy; f.g2yy = B.g2yy;
         f.u = B.u; f.v = B.v;
-        f.uh = nullptr; f.vh = nullptr;
+        f.uh = (L.lambdac != 0.f) ? hu : nullptr;
+        f.vh = (L.lambdac != 0.f) ? hv : nullptr;
         BuildParams bp;
         bp.alpha = p.alpha; bp.ralpha = 1.0 / p.alpha; bp.lambdadalpha = p.lambda / p.alpha; bp.lambdac = L.lambdac;
         bp.dozim = p.dozim != 0; bp.nchan = nc; bp.tol = 0.0001 * 0.0001;
@@ -1311,21 +1334,21 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
     CUDA_OK(cudaGetLastError());
     return OCTANE_OK;
 }
-}  // namespace
 
-int octane_optical_flow_batch_dev(octane_ctx* c, int npairs, const float* d_img1, const float* d_img2, const float* d_cth,
-                                  int nx, int ny, int nc, const octane_nav* nav, const double* t1, const double* t2,
-                                  const octane_params* p, float* d_upix, float* d_vpix, short* U, short* V, short* Ur,
-                                  short* Vr, short* d_ctp, int* moved_out)
+// the body of octane_optical_flow_batch_ex_dev and octane_optical_flow_batch_dev (which passes no first guess)
+int optical_flow_batch(octane_ctx* c, int npairs, const float* d_img1, const float* d_img2, const float* d_fg_u,
+                       const float* d_fg_v, const float* d_cth, int nx, int ny, int nc, const octane_nav* nav,
+                       const double* t1, const double* t2, const octane_params* p, float* d_upix, float* d_vpix, short* U,
+                       short* V, short* Ur, short* Vr, short* d_ctp, int* moved_out)
 {
     if (!c || !d_img1 || !d_img2 || !nav || !t1 || !t2 || !p || !d_upix || !d_vpix || !U || !V || !Ur || !Vr) {
         set_err("null argument");
         return OCTANE_EINVAL;
     }
     if (npairs < 1) { set_err("npairs must be at least 1"); return OCTANE_EINVAL; }
-    if (p->first_guess) { set_err("batched calls take no first guess"); return OCTANE_EINVAL; }
-    if (p->dosrsal) { set_err("batched calls do not run -srsal"); return OCTANE_EINVAL; }
+    if (p->first_guess && (!d_fg_u || !d_fg_v)) { set_err("first_guess is set but no first guess was given"); return OCTANE_EINVAL; }
     if (p->doCTH && (!d_cth || !d_ctp)) { set_err("doCTH needs cth and ctp"); return OCTANE_EINVAL; }
+    if (!srsal_args_ok(p, d_cth, nx, ny)) return OCTANE_EINVAL;
     if (c->comm.world > 1) { set_err("context is banded: batched calls are single-GPU"); return OCTANE_EINVAL; }
     begin_call(c);
     int rc = prepare(c, nx, ny, nc, *p);
@@ -1336,15 +1359,40 @@ int octane_optical_flow_batch_dev(octane_ctx* c, int npairs, const float* d_img1
     if (rc) return rc;
     const size_t ps = S / sizeof(float), n = (size_t)nx * ny;
     cudaStream_t st = c->stream;
-    // dense pairs -> pitched finest-level planes of each pair's workspace
+    // every allocation of the call before its first copy or launch: a failed one leaves nothing half enqueued
+    const size_t need = pix2uv_table_doubles(nx, ny) * (size_t)npairs;
+    if (need > c->navtab_doubles) {
+        CUDA_OK(cudaStreamSynchronize(st));
+        if (c->d_navtab) cudaFree(c->d_navtab);
+        c->d_navtab = nullptr; c->navtab_doubles = 0;
+        if (cudaMalloc(&c->d_navtab, need * sizeof(double)) != cudaSuccess) {
+            cudaGetLastError();
+            c->d_navtab = nullptr;
+            set_err("cudaMalloc (navigation tables): out of device memory");
+            return OCTANE_ENOMEM;
+        }
+        c->navtab_doubles = need;
+    }
+    const size_t sfb = align_up((size_t)npairs * n * sizeof(float));      // -srsal: two result planes per pair
+    if (p->dosrsal) {
+        rc = ensure_stage(c, 2 * sfb);
+        if (rc) return rc;
+    }
+    // dense pairs -> pitched finest-level planes of each pair's workspace; the first guess is copied in before any
+    // output is written, so it may alias d_upix / d_vpix
     const Geom& g = c->plan.lv.back().g;
     const size_t w = (size_t)nx * sizeof(float), dp = (size_t)g.pitch * sizeof(float);
-    for (int b = 0; b < npairs; b++)
+    for (int b = 0; b < npairs; b++) {
         for (int ch = 0; ch < nc; ch++) {
             const size_t src = ((size_t)b * nc + ch) * n, dst = (size_t)b * ps + (size_t)ch * g.plane;
             CUDA_OK(cudaMemcpy2DAsync(c->buf.img1 + dst, dp, d_img1 + src, w, w, ny, cudaMemcpyDeviceToDevice, st));
             CUDA_OK(cudaMemcpy2DAsync(c->buf.img2 + dst, dp, d_img2 + src, w, w, ny, cudaMemcpyDeviceToDevice, st));
         }
+        if (p->first_guess) {
+            CUDA_OK(cudaMemcpy2DAsync(c->buf.uh + (size_t)b * ps, dp, d_fg_u + b * n, w, w, ny, cudaMemcpyDeviceToDevice, st));
+            CUDA_OK(cudaMemcpy2DAsync(c->buf.vh + (size_t)b * ps, dp, d_fg_v + b * n, w, w, ny, cudaMemcpyDeviceToDevice, st));
+        }
+    }
     rc = run_levels_batch(c, npairs, ps);
     if (rc) return rc;
     for (int b = 0; b < npairs; b++) {
@@ -1357,14 +1405,6 @@ int octane_optical_flow_batch_dev(octane_ctx* c, int npairs, const float* d_img1
     }
     std::vector<NavParams> np(npairs);
     for (int b = 0; b < npairs; b++) fill_nav(np[b], &nav[b], t1[b], t2[b], p);
-    const size_t need = pix2uv_table_doubles(nx, ny) * (size_t)npairs;
-    if (need > c->navtab_doubles) {
-        CUDA_OK(cudaStreamSynchronize(st));
-        if (c->d_navtab) cudaFree(c->d_navtab);
-        c->d_navtab = nullptr; c->navtab_doubles = 0;
-        CUDA_OK(cudaMalloc(&c->d_navtab, need * sizeof(double)));
-        c->navtab_doubles = need;
-    }
     CUDA_OK(cudaMemcpyAsync(c->d_bnav, np.data(), npairs * sizeof(NavParams), cudaMemcpyHostToDevice, st));
     c->launches += launch_pix2uv_batch(np[0], c->d_bnav, npairs, d_upix, d_vpix, nx, ny, c->d_navtab, U, V, Ur, Vr, st);
     for (int b = 0; b < npairs; b++) {        // sector-moved guard, src/oct_pix2uv_cuda.cu:295,358-368
@@ -1373,10 +1413,36 @@ int octane_optical_flow_batch_dev(octane_ctx* c, int npairs, const float* d_img1
         if (!moved) continue;
         for (short* q : { U, V, Ur, Vr }) CUDA_OK(cudaMemsetAsync(q + b * n, 0, n * sizeof(short), st));
     }
+    if (p->dosrsal) {      // src/oct_optical_flow.cc:100-105: after the navigation, so only uPix / vPix are smoothed
+        rc = srsal_enqueue(c, d_upix, d_vpix, d_cth, nx, ny, (float*)c->stage, (float*)(c->stage + sfb), npairs);
+        if (rc) return rc;
+    }
     CUDA_OK(cudaGetLastError());
     c->batch_npairs = npairs;
     c->batch_nsolves = p->kiters * 3 * p->liters;
     return OCTANE_OK;
+}
+}  // namespace
+
+int octane_optical_flow_batch_ex_dev(octane_ctx* c, int npairs, const float* d_img1, const float* d_img2,
+                                     const float* d_fg_u, const float* d_fg_v, const float* d_cth, int nx, int ny, int nc,
+                                     const octane_nav* nav, const double* t1, const double* t2, const octane_params* p,
+                                     float* d_upix, float* d_vpix, short* U, short* V, short* Ur, short* Vr, short* d_ctp,
+                                     int* moved_out)
+{
+    return optical_flow_batch(c, npairs, d_img1, d_img2, d_fg_u, d_fg_v, d_cth, nx, ny, nc, nav, t1, t2, p, d_upix, d_vpix,
+                              U, V, Ur, Vr, d_ctp, moved_out);
+}
+
+int octane_optical_flow_batch_dev(octane_ctx* c, int npairs, const float* d_img1, const float* d_img2, const float* d_cth,
+                                  int nx, int ny, int nc, const octane_nav* nav, const double* t1, const double* t2,
+                                  const octane_params* p, float* d_upix, float* d_vpix, short* U, short* V, short* Ur,
+                                  short* Vr, short* d_ctp, int* moved_out)
+{
+    if (p && p->first_guess) { set_err("batched calls take no first guess: use octane_optical_flow_batch_ex_dev"); return OCTANE_EINVAL; }
+    if (p && p->dosrsal) { set_err("octane_optical_flow_batch_dev does not run -srsal: use octane_optical_flow_batch_ex_dev"); return OCTANE_EINVAL; }
+    return optical_flow_batch(c, npairs, d_img1, d_img2, nullptr, nullptr, d_cth, nx, ny, nc, nav, t1, t2, p, d_upix, d_vpix,
+                              U, V, Ur, Vr, d_ctp, moved_out);
 }
 
 int octane_batch_cg_iterations(octane_ctx* c, int* its, int npairs)
@@ -1734,13 +1800,15 @@ void srsal_taps(SrsalTaps* t)
     for (int i = 0; i < 2 * filtsize + 1; ++i) t->gk[i] /= sum;
 }
 
-// u, v -> tmp (filtered) -> back into u, v, all on the context's stream
-int srsal_enqueue(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int nx, int ny, float* tmp_u, float* tmp_v)
+// u, v -> tmp (filtered) -> back into u, v, all on the context's stream.  npairs dense pair-major scenes (u, v, cth
+// and each tmp plane npairs x ny x nx), filtered in one launch, each pair with its own heights.
+int srsal_enqueue(octane_ctx* c, float* d_u, float* d_v, const float* d_cth, int nx, int ny, float* tmp_u, float* tmp_v,
+                  int npairs)
 {
     SrsalTaps t;
     srsal_taps(&t);
-    const size_t fb = (size_t)nx * ny * sizeof(float);
-    launch_srsal(d_u, d_v, d_cth, nx, ny, 0, 0, ny, t, tmp_u, tmp_v, c->stream);
+    const size_t n = (size_t)nx * ny, fb = (size_t)npairs * n * sizeof(float);
+    launch_srsal(d_u, d_v, d_cth, nx, ny, 0, 0, ny, t, tmp_u, tmp_v, c->stream, npairs, n);
     c->launches++;
     CUDA_OK(cudaGetLastError());
     CUDA_OK(cudaMemcpyAsync(d_u, tmp_u, fb, cudaMemcpyDeviceToDevice, c->stream));

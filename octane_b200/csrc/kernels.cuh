@@ -178,8 +178,9 @@ struct SrsalTaps {
     double sigpix2;
 };
 // u, v, cth: dense rows [e0, ...) of the scene; u_out, v_out: dense rows [o0, o1).  Every row the window of an
-// output row reads (after reflection at the scene edges 0 and ny) must be present in the inputs.
+// output row reads (after reflection at the scene edges 0 and ny) must be present in the inputs.  Batched: npairs
+// pairs, every input and output plane of pair z ps floats after pair 0's.
 void launch_srsal(const float* u, const float* v, const float* cth, int nx, int ny, int e0, int o0, int o1,
-                  const SrsalTaps& t, float* u_out, float* v_out, cudaStream_t st);
+                  const SrsalTaps& t, float* u_out, float* v_out, cudaStream_t st, int npairs = 1, size_t ps = 0);
 
 }  // namespace octane

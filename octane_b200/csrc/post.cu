@@ -18,6 +18,11 @@
 // Row window (banded runs): the input planes hold global rows [e0, ...), the output planes global rows
 // [o0, o1).  The reflecting index stays in global coordinates (the scene edges are the edges of the whole
 // scene, not of a band); e0 is subtracted only when addressing.  One GPU: e0 = o0 = 0, o1 = ny.
+//
+// Batches (octane_optical_flow_batch_ex_dev): pair blockIdx.z reads and writes planes ps floats further on, each pair
+// filtered with its own heights; one launch covers every pair.  The offset enters the staging loads and the two
+// stores only, so the 37 x 37 loop, which reads shared memory only, is the single-pair loop instruction for
+// instruction.
 #include "kernels.cuh"
 
 namespace octane {
@@ -37,9 +42,11 @@ __device__ __forceinline__ int reflect(int x, int nx)
 
 __global__ void __launch_bounds__(TX * TY)
 k_srsal(const float* __restrict__ u, const float* __restrict__ v, const float* __restrict__ cth, int nx, int ny,
-        int e0, int o0, int o1, SrsalTaps t, float* __restrict__ u_out, float* __restrict__ v_out)
+        int e0, int o0, int o1, SrsalTaps t, float* __restrict__ u_out, float* __restrict__ v_out, size_t ps)
 {
     __shared__ float s_c[SH][SW], s_u[SH][SW], s_v[SH][SW];
+    const size_t po = (size_t)blockIdx.z * ps;
+    u += po; v += po; cth += po;
     const int i0 = blockIdx.x * TX, j0 = o0 + blockIdx.y * TY;
     for (int k = threadIdx.y * TX + threadIdx.x; k < SW * SH; k += TX * TY) {
         const int sy = k / SW, sx = k - sy * SW;
@@ -65,17 +72,21 @@ k_srsal(const float* __restrict__ u, const float* __restrict__ v, const float* _
             av += (double)s_v[threadIdx.y + lc][threadIdx.x + kc] * a1;
         }
     }
-    const size_t at = (size_t)ic + (size_t)(jc - o0) * nx;
+    // the pair index is read again rather than kept from the staging loop: a value live across the filter loop moves
+    // the loop's uniform registers and its schedule
+    unsigned z;
+    asm volatile("mov.u32 %0, %%ctaid.z;" : "=r"(z));
+    const size_t at = (size_t)z * ps + (size_t)ic + (size_t)(jc - o0) * nx;
     u_out[at] = (au / a2);
     v_out[at] = (av / a2);
 }
 }  // namespace
 
 void launch_srsal(const float* u, const float* v, const float* cth, int nx, int ny, int e0, int o0, int o1,
-                  const SrsalTaps& t, float* u_out, float* v_out, cudaStream_t st)
+                  const SrsalTaps& t, float* u_out, float* v_out, cudaStream_t st, int npairs, size_t ps)
 {
-    dim3 grid((nx + TX - 1) / TX, (o1 - o0 + TY - 1) / TY), block(TX, TY);
-    k_srsal<<<grid, block, 0, st>>>(u, v, cth, nx, ny, e0, o0, o1, t, u_out, v_out);
+    dim3 grid((nx + TX - 1) / TX, (o1 - o0 + TY - 1) / TY, npairs), block(TX, TY);
+    k_srsal<<<grid, block, 0, st>>>(u, v, cth, nx, ny, e0, o0, o1, t, u_out, v_out, ps);
 }
 
 }  // namespace octane

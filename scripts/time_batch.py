@@ -4,7 +4,12 @@ Two workloads: 64 x 500^2 with cloud-top heights and m/s output (BASELINE config
 8 x 2000^2, whose finest levels run the single-pair PCG kernels pair by pair.  Arms, alternated on the same inputs in
 one run: one batched call per step, and the contexts-in-flight loop of bench.py's batch_arm with K = 8 and 16
 contexts.  Reports device ms per step (CUDA events), Mpix/s and kernel launches per step, with the card's name and
-power limit.  Writes --out (JSON)."""
+power limit.  Writes --out (JSON).
+
+--first-guess (with lambda_c = 0.5) and --srsal time the same workloads with those flags: the batch arm calls
+octane_optical_flow_batch_ex_dev, the contexts arms pass the same flags to octane_optical_flow_dev, and with --srsal a
+second batch arm without -srsal gives the cost of the smoother.  The default output is then
+profiles/r03_batch_fg_srsal_n1.json."""
 import argparse
 import json
 import os
@@ -23,7 +28,7 @@ def card():
     return r.stdout.strip().splitlines()[0] if r.returncode == 0 and r.stdout.strip() else "unknown"
 
 
-def workload(n, npairs, seed0, rounds, steps, warmup):
+def workload(n, npairs, seed0, rounds, steps, warmup, fg=False, srsal=False):
     import torch
 
     import octane_b200 as ob
@@ -32,7 +37,8 @@ def workload(n, npairs, seed0, rounds, steps, warmup):
     dev = torch.device("cuda", 0)
     xs, ys, xo, yo, dt = S.SECTORS["meso_2km"]
     nav = ob.goes_nav(xs, ys, xo, yo)
-    p = ob.default_params(doCTH=1)
+    flags = dict(first_guess=1, lambdac=0.5) if fg else {}
+    p = ob.default_params(doCTH=1, dosrsal=int(srsal), **flags)
     yy, xx = np.mgrid[0:n, 0:n].astype(np.float32)
     cth1 = torch.from_numpy((7500.0 + 7400.0 * np.sin(xx / 40.0) * np.cos(yy / 30.0)).astype(np.float32)).to(dev)
     pairs = [S.make_pair_torch(n, n, seed0 + k, dev) for k in range(npairs)]
@@ -43,11 +49,25 @@ def workload(n, npairs, seed0, rounds, steps, warmup):
     for k in ("uVal", "vVal", "uVal2", "vVal2", "CTP"):
         bout[k] = torch.zeros((npairs, n, n), dtype=torch.int16, device=dev)
     bctx = ob.Context(0)
+    if fg:                                       # a smooth first guess, scaled per pair
+        u0 = torch.from_numpy(0.6 + 0.3 * np.sin(xx / 23.0) * np.cos(yy / 31.0)).to(dev)
+        v0 = torch.from_numpy(-0.3 + 0.2 * np.cos(xx / 19.0 + yy / 29.0)).to(dev)
+        scale = torch.linspace(0.8, 1.2, npairs, device=dev).view(npairs, 1, 1)
+        fgu, fgv = (u0 * scale).contiguous(), (v0 * scale).contiguous()
+    ex = dict(fg_u=fgu, fg_v=fgv) if fg else {}
 
-    def batch_step():
-        bctx.oct_optical_flow_batch_dev(img1, img2, [nav] * npairs, [0.0] * npairs, [dt] * npairs, p, bout, cth=cth)
+    def batch_step(p=p, bout=bout):
+        if fg or srsal:
+            bctx.oct_optical_flow_batch_ex_dev(img1, img2, [nav] * npairs, [0.0] * npairs, [dt] * npairs, p, bout,
+                                               cth=cth, **ex)
+        else:
+            bctx.oct_optical_flow_batch_dev(img1, img2, [nav] * npairs, [0.0] * npairs, [dt] * npairs, p, bout, cth=cth)
 
     arms = {"batch": ([bctx], batch_step)}
+    if srsal:                                    # the same call without -srsal, on its own outputs
+        p0 = ob.default_params(doCTH=1, **flags)
+        bout0 = {k: torch.zeros_like(a) for k, a in bout.items()}
+        arms["batch_no_srsal"] = ([bctx], lambda: batch_step(p0, bout0))
     for K in (8, 16):
         ctxs = [ob.Context(0) for _ in range(K)]
         outs = [dict(u=torch.zeros((n, n), device=dev), v=torch.zeros((n, n), device=dev),
@@ -56,6 +76,10 @@ def workload(n, npairs, seed0, rounds, steps, warmup):
         def step(ctxs=ctxs, outs=outs, K=K):
             for i, (a, b) in enumerate(pairs):
                 o = outs[i]
+                if fg:                           # octane_optical_flow_dev reads its first guess from uPix / vPix
+                    with torch.cuda.stream(ctxs[i % K]._ext_stream()):
+                        o["u"].copy_(fgu[i])
+                        o["v"].copy_(fgv[i])
                 ctxs[i % K].oct_optical_flow_dev(a, b, nav, 0.0, dt, p, o["u"], o["v"], *o["s"][:4], cth=cth1,
                                                  ctp=o["s"][4], sync_torch=False)
         arms[f"contexts_{K}"] = (ctxs, step)
@@ -90,8 +114,10 @@ def workload(n, npairs, seed0, rounds, steps, warmup):
     res = {}
     mpix = npairs * n * n / 1e6
     for k, (ctxs, fn) in arms.items():
+        if srsal and k.startswith("batch"):      # the two batch arms share a context: its counters hold the last call
+            fn()
         launches = sum(int(c.stats().kernel_launches) for c in ctxs)
-        if k != "batch":
+        if k.startswith("contexts"):
             used = min(len(ctxs), npairs)                 # every used context's last call was one pair
             launches = launches // used * npairs
         best = min(ms[k])
@@ -101,24 +127,39 @@ def workload(n, npairs, seed0, rounds, steps, warmup):
     torch.cuda.synchronize()
     u8 = torch.stack([o["u"] for o in outs8])
     res["batch_vs_contexts_max_abs_px"] = float((bout["uPix"] - u8).abs().max())
+    if fg or srsal:
+        v8 = torch.stack([o["v"] for o in outs8])
+        res["batch_vs_contexts_max_abs_px_v"] = float((bout["vPix"] - v8).abs().max())
     for name, (ctxs, _) in arms.items():
-        if name != "batch":
+        if name.startswith("contexts"):
             for c in ctxs:
                 c.close()
     bctx.close()
-    return {"pairs": npairs, "size": n, "doCTH": 1, "output": "m/s", **res}
+    if srsal:
+        res["srsal_ms_per_step"] = res["batch"]["ms_per_step"] - res["batch_no_srsal"]["ms_per_step"]
+    if fg:
+        res["first_guess_note"] = ("the contexts arms copy each pair's first guess into its uPix / vPix on the "
+                                   "context's stream before each call (two device copies per pair, timed); the batch "
+                                   "arm reads fg_u / fg_v directly")
+    return {"pairs": npairs, "size": n, "doCTH": 1, "output": "m/s", **({"first_guess": 1, "lambdac": 0.5} if fg else {}),
+            **({"dosrsal": 1} if srsal else {}), **res}
 
 
 def main():
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_batch_n1.json"))
+    ap.add_argument("--out", default=None)
     ap.add_argument("--steps", type=int, default=3)
     ap.add_argument("--warmup", type=int, default=1)
     ap.add_argument("--rounds", type=int, default=3)
+    ap.add_argument("--first-guess", action="store_true", help="solve with a first guess and lambda_c = 0.5")
+    ap.add_argument("--srsal", action="store_true", help="run the -srsal post-smoother")
     a = ap.parse_args()
+    name = "r03_batch_fg_srsal_n1.json" if a.first_guess or a.srsal else "r03_batch_n1.json"
+    a.out = a.out or os.path.join(ROOT, "profiles", name)
+    flags = dict(fg=a.first_guess, srsal=a.srsal)
     res = {"card": card(), "what": "device ms per step over CUDA events, best of the alternated rounds",
-           "workloads": [workload(500, 64, 100, a.rounds, a.steps, a.warmup),
-                         workload(2000, 8, 300, a.rounds, a.steps, a.warmup)]}
+           "workloads": [workload(500, 64, 100, a.rounds, a.steps, a.warmup, **flags),
+                         workload(2000, 8, 300, a.rounds, a.steps, a.warmup, **flags)]}
     os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
     with open(a.out, "w") as f:
         json.dump(res, f, indent=1)
