@@ -252,7 +252,11 @@ int octane_optical_flow_dev(octane_ctx* ctx, const float* d_img1, const float* d
  * octane_optical_flow_dev does, with one launch per stage for the whole batch.  Arrays are dense and pair-major:
  * images npairs x nc x ny x nx, d_cth and every output npairs x ny x nx; nav, t1 and t2 are host arrays of npairs.
  * Small pyramid levels solve all pairs in one cooperative launch (each pair on its own group of blocks, with its own
- * barrier and stop rule); a pair's result does not depend on the other pairs of the call.  Stream-ordered, no host
+ * barrier and stop rule).  Large levels (nx >= 512, >= 64 rows) under the default solver (octane_ctx_set_solver 1)
+ * run one PCG launch per iteration for all pairs, each pair on the grid and tiling it would get alone, with its own
+ * reductions and stop rule (a converged pair's blocks exit at once), replayed from a CUDA graph; under solver 0 they
+ * run the two-pass kernels pair by pair.  A pair's result does not depend on the other pairs of the call, nor on
+ * their number.  Stream-ordered, no host
  * synchronisation; moved_out (host, npairs, may be NULL) gets 1 for each pair whose sector moved (its four short
  * planes are zero).  OCTANE_EINVAL for npairs < 1, a first guess, dosrsal or a banded context (a first guess and
  * -srsal go through octane_optical_flow_batch_ex_dev, which shares this call's body); OCTANE_ENOMEM when the npairs

@@ -188,6 +188,7 @@ struct octane_ctx {
     double* d_bpart = nullptr;
     size_t bpart_doubles = 0;
     unsigned* d_bbar = nullptr;
+    unsigned* d_bticket = nullptr;       // one grid-reduction ticket per pair (large levels, merged-reduction solver)
     int* d_bits = nullptr;
     NavParams* d_bnav = nullptr;
     int batch_cap = 0;
@@ -196,6 +197,9 @@ struct octane_ctx {
     bool plan_valid = false;
     Buffers buf;
     std::vector<cudaGraphExec_t> pcg_graph;   // two per level: [2 * level + (constant W / N variant)]
+    // batched calls: the large levels' PCG loop of all pairs, same slots; captured for batch_graph_pairs[slot] pairs
+    std::vector<cudaGraphExec_t> batch_graph;
+    std::vector<int> batch_graph_pairs;
     // small persistent device objects
     PcgScalars* d_scal = nullptr;
     double* d_pending = nullptr;
@@ -237,10 +241,18 @@ struct octane_ctx {
 
 namespace {
 
+void destroy_batch_graphs(octane_ctx* c)
+{
+    for (auto g : c->batch_graph) if (g) cudaGraphExecDestroy(g);
+    c->batch_graph.clear();
+    c->batch_graph_pairs.clear();
+}
+
 void destroy_graphs(octane_ctx* c)
 {
     for (auto g : c->pcg_graph) if (g) cudaGraphExecDestroy(g);
     c->pcg_graph.clear();
+    destroy_batch_graphs(c);
 }
 
 size_t align_up(size_t x) { return (x + 255) & ~(size_t)255; }
@@ -507,6 +519,25 @@ bool level_coop(const octane_ctx* c, const Level& L)
     return c->coop && c->comm.world <= 1 && !pcg_fused_usable(L.g, L.own1 - L.own0);
 }
 
+// Capture what enqueue() puts on the stream as an executable graph (*exec); the launches it counts are not counted
+// here (the caller counts each replay).
+template <class F>
+int capture_graph(octane_ctx* c, F enqueue, cudaGraphExec_t* exec)
+{
+    cudaGraph_t graph = nullptr;
+    const long long before = c->launches;
+    CUDA_OK(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
+    int rc = enqueue();
+    cudaError_t e = cudaStreamEndCapture(c->stream, &graph);
+    c->launches = before;
+    if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
+    if (e != cudaSuccess) { set_err("cudaStreamEndCapture: %s", cudaGetErrorString(e)); return OCTANE_ECUDA; }
+    e = cudaGraphInstantiate(exec, graph, 0);
+    cudaGraphDestroy(graph);
+    if (e != cudaSuccess) { *exec = nullptr; set_err("cudaGraphInstantiate: %s", cudaGetErrorString(e)); return OCTANE_ECUDA; }
+    return OCTANE_OK;
+}
+
 // const_wn: the system was built in the first GNC stage (W = N = -1 everywhere)
 int run_pcg(octane_ctx* c, const Level& L, int level, int solve, int const_wn)
 {
@@ -523,19 +554,8 @@ int run_pcg(octane_ctx* c, const Level& L, int level, int solve, int const_wn)
     if (!c->graphs || c->profile) return enqueue_pcg(c, L, level, solve, const_wn, c->buf.pcg);
     const size_t slot = 2 * (size_t)level + (const_wn ? 1 : 0);
     if (!c->pcg_graph[slot]) {
-        cudaGraph_t graph = nullptr;
-        const long long before = c->launches;
-        CUDA_OK(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-        int rc = enqueue_pcg(c, L, level, solve, const_wn, c->buf.pcg);
-        cudaError_t e = cudaStreamEndCapture(c->stream, &graph);
-        c->launches = before;
-        if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-        if (e != cudaSuccess) { set_err("cudaStreamEndCapture: %s", cudaGetErrorString(e)); return OCTANE_ECUDA; }
-        cudaGraphExec_t exec = nullptr;
-        e = cudaGraphInstantiate(&exec, graph, 0);
-        cudaGraphDestroy(graph);
-        if (e != cudaSuccess) { set_err("cudaGraphInstantiate: %s", cudaGetErrorString(e)); return OCTANE_ECUDA; }
-        c->pcg_graph[slot] = exec;
+        int rc = capture_graph(c, [&] { return enqueue_pcg(c, L, level, solve, const_wn, c->buf.pcg); }, &c->pcg_graph[slot]);
+        if (rc) return rc;
     }
     CUDA_OK(cudaGraphLaunch(c->pcg_graph[slot], c->stream));
     if (level_fused(c, L)) c->launches += (long long)c->plan.p.cgiters + 1;
@@ -958,7 +978,8 @@ void octane_ctx_destroy(octane_ctx* c)
     if (c->d_its) cudaFree(c->d_its);
     if (c->d_gk) cudaFree(c->d_gk);
     if (c->d_navtab) cudaFree(c->d_navtab);
-    for (void* q : { (void*)c->d_bscal, (void*)c->d_bpart, (void*)c->d_bbar, (void*)c->d_bits, (void*)c->d_bnav })
+    for (void* q : { (void*)c->d_bscal, (void*)c->d_bpart, (void*)c->d_bbar, (void*)c->d_bticket, (void*)c->d_bits,
+                     (void*)c->d_bnav })
         if (q) cudaFree(q);
     for (auto& sl : c->slot) {
         if (sl.done) cudaEventSynchronize(sl.done);
@@ -1187,19 +1208,27 @@ int ensure_batch(octane_ctx* c, int npairs, size_t* stride)
         CUDA_OK(cudaMemsetAsync(c->arena + S * c->arena_pairs, 0, S * (size_t)(npairs - c->arena_pairs), c->stream));
         c->arena_pairs = npairs;
     }
+    // partials: one region per pair, large enough for the build, a cooperative group and a merged-reduction launch
+    // (2 * partial_blocks doubles, the single-pair budget: a pair's grid is never capped below its single-pair one)
     int bb = 0;
     for (const Level& L : pl.lv) { int t = build_partial_blocks(L.g, L.g.rows); if (t > bb) bb = t; }
-    const size_t pd = (size_t)npairs * (2 * (size_t)bb > 3 * 8 ? 2 * (size_t)bb : 3 * 8);
+    size_t per = 2 * (size_t)bb > 3 * 8 ? 2 * (size_t)bb : 3 * 8;
+    if (2 * (size_t)c->partial_blocks > per) per = 2 * (size_t)c->partial_blocks;
+    const size_t pd = (size_t)npairs * per;
     if (npairs > c->batch_cap || pd > c->bpart_doubles) {
         CUDA_OK(cudaStreamSynchronize(c->stream));
-        for (void* q : { (void*)c->d_bscal, (void*)c->d_bpart, (void*)c->d_bbar, (void*)c->d_bits, (void*)c->d_bnav })
+        for (void* q : { (void*)c->d_bscal, (void*)c->d_bpart, (void*)c->d_bbar, (void*)c->d_bticket, (void*)c->d_bits,
+                         (void*)c->d_bnav })
             if (q) cudaFree(q);
-        c->d_bscal = nullptr; c->d_bpart = nullptr; c->d_bbar = nullptr; c->d_bits = nullptr; c->d_bnav = nullptr;
+        c->d_bscal = nullptr; c->d_bpart = nullptr; c->d_bbar = nullptr; c->d_bticket = nullptr; c->d_bits = nullptr;
+        c->d_bnav = nullptr;
         c->batch_cap = 0; c->bpart_doubles = 0;
+        destroy_batch_graphs(c);                             // the captured batched PCG loops point into the old buffers
         const int n = npairs > c->batch_cap ? npairs : c->batch_cap;
         if (cudaMalloc(&c->d_bscal, n * sizeof(PcgScalars)) != cudaSuccess ||
             cudaMalloc(&c->d_bpart, pd * sizeof(double)) != cudaSuccess ||
             cudaMalloc(&c->d_bbar, 2 * n * sizeof(unsigned)) != cudaSuccess ||
+            cudaMalloc(&c->d_bticket, n * sizeof(unsigned)) != cudaSuccess ||
             cudaMalloc(&c->d_bits, (size_t)n * OCTANE_MAX_SOLVES * sizeof(int)) != cudaSuccess ||
             cudaMalloc(&c->d_bnav, n * sizeof(NavParams)) != cudaSuccess) {
             cudaGetLastError();
@@ -1207,6 +1236,7 @@ int ensure_batch(octane_ctx* c, int npairs, size_t* stride)
             return OCTANE_ENOMEM;
         }
         CUDA_OK(cudaMemsetAsync(c->d_bscal, 0, n * sizeof(PcgScalars), c->stream));
+        CUDA_OK(cudaMemsetAsync(c->d_bticket, 0, n * sizeof(unsigned), c->stream));      // each launch leaves it at 0
         c->batch_cap = n; c->bpart_doubles = pd;
     }
     return OCTANE_OK;
@@ -1224,10 +1254,54 @@ PcgBuffers pair_buffers(const PcgBuffers& b0, int b, size_t ps)
     return q;
 }
 
+// The PCG loop of one solve of every pair on a large level, merged-reduction solver: one launch per iteration (+ the
+// one that forms the first alpha) for all pairs.  pb: pair 0's planes, the pairs' scalars, partials and tickets.
+int enqueue_pcg_batch(octane_ctx* c, const Level& L, int level, int solve, int const_wn, const PcgBuffers& pb, int npairs,
+                      size_t ps)
+{
+    for (int ki = -1; ki < c->plan.p.cgiters; ki++) {
+        Scope s(c, CAT_P1, level, solve, ki);
+        if (launch_pcg_fused(pb, L.g, L.own0, L.own1, ki, L.fp, c->sm_count, c->stream, const_wn, npairs, ps)) {
+            set_err("batched merged-reduction launch refused");
+            return OCTANE_EINVAL;
+        }
+        c->launches++;
+    }
+    return OCTANE_OK;
+}
+
+// enqueue_pcg_batch replayed from a graph per (level, constant-W/N variant), re-captured when npairs changes;
+// without graphs or with profiling on, enqueued directly
+int run_pcg_batch(octane_ctx* c, const Level& L, int level, int solve, int const_wn, const PcgBuffers& pb, int npairs,
+                  size_t ps)
+{
+    if (!c->graphs || c->profile) return enqueue_pcg_batch(c, L, level, solve, const_wn, pb, npairs, ps);
+    const size_t slot = 2 * (size_t)level + (const_wn ? 1 : 0);
+    if (c->batch_graph.size() != 2 * c->plan.lv.size()) {
+        destroy_batch_graphs(c);
+        c->batch_graph.assign(2 * c->plan.lv.size(), nullptr);
+        c->batch_graph_pairs.assign(2 * c->plan.lv.size(), 0);
+    }
+    cudaGraphExec_t& exec = c->batch_graph[slot];
+    if (exec && c->batch_graph_pairs[slot] != npairs) {
+        CUDA_OK(cudaGraphExecDestroy(exec));
+        exec = nullptr;
+    }
+    if (!exec) {
+        int rc = capture_graph(c, [&] { return enqueue_pcg_batch(c, L, level, solve, const_wn, pb, npairs, ps); }, &exec);
+        if (rc) return rc;
+        c->batch_graph_pairs[slot] = npairs;
+    }
+    CUDA_OK(cudaGraphLaunch(exec, c->stream));
+    c->launches += (long long)c->plan.p.cgiters + 1;
+    return OCTANE_OK;
+}
+
 // run_levels for npairs pairs in the batch workspace (pair stride ps floats); one GPU.  With a first guess, each
 // pair's hint is in its own uh / vh planes.  Per-pixel stages are one launch for all pairs; small levels solve all
-// pairs in cooperative launches with one barrier per pair (launch_pcg_coop_batch), large levels run the single-pair
-// PCG kernels pair by pair.
+// pairs in cooperative launches with one barrier per pair (launch_pcg_coop_batch); large levels under the
+// merged-reduction solver run one launch per iteration for all pairs (run_pcg_batch), under the two-pass solver the
+// single-pair PCG kernels pair by pair.
 int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
 {
     const Plan& pl = c->plan;
@@ -1241,6 +1315,7 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
     PcgBuffers pb = B.pcg;                       // build and update: pair z uses d_bscal[z] (and partials region z)
     pb.scal = c->d_bscal;
     pb.partials = c->d_bpart;
+    pb.ticket = c->d_bticket;
     int solve = 0;
     for (int k = 0; k < K; k++) {
         const Level& L = pl.lv[k];
@@ -1310,6 +1385,9 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
                         }
                         c->launches++;
                     }
+                } else if (p.cgiters > 0 && fused) {
+                    int rc = run_pcg_batch(c, L, k, solve, gnc == 0 ? 1 : 0, pb, npairs, ps);
+                    if (rc) return rc;
                 } else if (p.cgiters > 0) {
                     for (int b = 0; b < npairs; b++) {
                         PcgBuffers q = pair_buffers(B.pcg, b, ps);

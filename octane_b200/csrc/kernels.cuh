@@ -111,8 +111,13 @@ struct FusedPeers {
 };
 // ki = -1: forms the first alpha (q0 = A z0, no writes); ki >= 0: iteration ki.  Reads r[ki & 1], p[ki & 1]
 // (r[0] = ru / rv as the build leaves it), writes the other buffer of each pair.
-void launch_pcg_fused(const PcgBuffers& b, const Geom& g, int ja, int jb, int ki, const FusedPeers& peers,
-                      int sm_count, cudaStream_t st, int const_wn);
+// Batched: npairs pairs in one launch, the pair from blockIdx.z; pair z uses b.scal[z], its own ticket b.ticket[z] and
+// partials region z (2 * b.max_partial_blocks doubles each), and its planes ps floats after pair z - 1's.  Every pair
+// gets the tiling and grid of a single-pair launch, so its bits are those of a launch of that pair alone; npairs = 1 runs
+// the single-pair kernels, npairs > 1 kernels compiled apart with the pair addressing.  Returns 0,
+// or -1 (nothing launched) when npairs < 1 or npairs > 1 comes with banded peers.
+int launch_pcg_fused(const PcgBuffers& b, const Geom& g, int ja, int jb, int ki, const FusedPeers& peers,
+                     int sm_count, cudaStream_t st, int const_wn, int npairs = 1, size_t ps = 0);
 // u += x (+ the pending alpha p when the iteration count is odd), after a merged-reduction solve
 void launch_update_uv_fused(float* u, float* v, const PcgBuffers& b, const Geom& g, int ja, int jb,
                             int* its_out, int sm_count, cudaStream_t st, int npairs = 1, size_t ps = 0, int its_stride = 0);
