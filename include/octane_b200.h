@@ -285,7 +285,24 @@ int octane_optical_flow_batch_ex_dev(octane_ctx* ctx, int npairs, const float* d
                                      const double* t1, const double* t2, const octane_params* p,
                                      float* d_upix, float* d_vpix, short* d_U, short* d_V, short* d_U_raw,
                                      short* d_V_raw, short* d_ctp, int* moved_out);
-/* PCG iterations of every solve of every pair of the last batched call (either of the two above):
+/* A sequence of nframes same-size frames (d_frames: nframes x nc x ny x nx, dense), solved as its nframes - 1
+ * consecutive pairs: pair k is (frame k, frame k + 1) with t1 = t[k], t2 = t[k + 1] (t: host array of nframes).
+ * Per pair, the results are octane_optical_flow_batch_ex_dev's on those pairs, bit for bit, with the same flags,
+ * refusals (OCTANE_EINVAL also for nframes < 2) and guarantees; nav (host) and moved_out have one entry per pair (pair
+ * k's nav carries frame k + 1's g2xOffset / g2yOffset), and d_fg_u, d_fg_v, d_cth (image 1's heights of each pair) and
+ * every output are (nframes - 1) x ny x nx.  Each frame is copied in, blurred, decimated and differentiated once
+ * instead of twice, in a workspace of nframes instead of 2 (nframes - 1) image slots (octane_batch_workspace_bytes).
+ * octane_batch_cg_iterations (npairs = nframes - 1) and octane_get_stats work afterwards as after a batch. */
+int octane_optical_flow_sequence_dev(octane_ctx* ctx, int nframes, const float* d_frames,
+                                     const float* d_fg_u, const float* d_fg_v, const float* d_cth,
+                                     int nx, int ny, int nc, const octane_nav* nav, const double* t,
+                                     const octane_params* p, float* d_upix, float* d_vpix, short* d_U, short* d_V,
+                                     short* d_U_raw, short* d_V_raw, short* d_ctp, int* moved_out);
+/* Device bytes a batched call (sequence = 0) or a sequence call (sequence = 1) of npairs pairs allocates on a fresh
+ * context of a 148-SM B200: the workspace, the per-pair scalars, partial sums and iteration counts, the navigation
+ * tables and, with p->dosrsal, the -srsal staging.  Host arithmetic, no device needed; 0 for invalid arguments. */
+size_t octane_batch_workspace_bytes(int npairs, int sequence, int nx, int ny, int nc, const octane_params* p);
+/* PCG iterations of every solve of every pair of the last batched call (any of the three above):
  * its[pair * n_solves + solve].  npairs must be that call's.  Synchronises the context's stream. */
 int octane_batch_cg_iterations(octane_ctx* ctx, int* its, int npairs);
 

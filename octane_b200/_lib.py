@@ -72,6 +72,7 @@ EXPORTS = [
     "octane_variational_flow_band_dev", "octane_variational_flow_band_fg_dev", "octane_pix2uv_band_dev",
     "octane_srsal_band_dev", "octane_stream_submit", "octane_stream_submit_fg", "octane_stream_wait",
     "octane_optical_flow_batch_dev", "octane_optical_flow_batch_ex_dev", "octane_batch_cg_iterations",
+    "octane_optical_flow_sequence_dev", "octane_batch_workspace_bytes",
 ]
 
 _lib = None
@@ -121,6 +122,10 @@ def load() -> C.CDLL:
     L.octane_optical_flow_batch_ex_dev.argtypes = [vp, i, vp, vp, vp, vp, vp, i, i, i, NP, C.POINTER(d), C.POINTER(d),
                                                    PP, vp, vp, vp, vp, vp, vp, vp, ip]
     L.octane_batch_cg_iterations.argtypes = [vp, ip, i]
+    L.octane_optical_flow_sequence_dev.argtypes = [vp, i, vp, vp, vp, vp, i, i, i, NP, C.POINTER(d), PP,
+                                                   vp, vp, vp, vp, vp, vp, vp, ip]
+    L.octane_batch_workspace_bytes.argtypes = [i, i, i, i, i, PP]
+    L.octane_batch_workspace_bytes.restype = C.c_size_t
     CP = C.POINTER(Cal)
     L.octane_navcal.argtypes = [vp, vp, vp, vp, i, i, NP, CP, vp, vp, vp]
     L.octane_navcal_dev.argtypes = [vp, vp, vp, vp, i, i, NP, CP, vp, vp, vp]

@@ -84,6 +84,14 @@ def level_dims(nx: int, ny: int, p: Optional[Params] = None):
     return out
 
 
+def batch_workspace_bytes(npairs: int, nx: int, ny: int, nc: int = 1, p: Optional[Params] = None,
+                          sequence: bool = False) -> int:
+    """device bytes a batched call (or, with sequence=True, a sequence call) of npairs pairs allocates on a fresh
+    context (octane_batch_workspace_bytes); 0 for invalid arguments"""
+    p = p or default_params()
+    return int(_lib.load().octane_batch_workspace_bytes(npairs, int(sequence), nx, ny, nc, C.byref(p)))
+
+
 def zoom_out_size(nx: int, ny: int, factor: float):
     """(nxx, nyy) of oct_zoom_size, src/oct_zoom.cc:12"""
     L = _lib.load()
@@ -390,6 +398,29 @@ class Context:
         self._after_torch()
         self._check(self._L.octane_optical_flow_batch_ex_dev(
             self._h, B, _ptr(geo1), _ptr(geo2), _ptr(fg_u), _ptr(fg_v), _ptr(cth), nx, ny, nc, navs, t1, t2, C.byref(p),
+            _ptr(out["uPix"]), _ptr(out["vPix"]), _ptr(out["uVal"]), _ptr(out["vVal"]), _ptr(out["uVal2"]),
+            _ptr(out["vVal2"]), _ptr(out.get("CTP")), moved))
+        self._before_torch()
+        return [b for b in range(B) if moved[b]]
+
+    def oct_optical_flow_sequence_dev(self, frames, nav_list, t_list, p: Params, out: dict, cth=None, nc: int = 1, *,
+                                      fg_u=None, fg_v=None):
+        """The consecutive pairs (frames[k], frames[k + 1]) of a sequence of N + 1 frames ([N + 1, ny, nx] or
+        [N + 1, nc, ny, nx] float32 CUDA tensor, t_list: N + 1 times, nav_list: N navigations) in one call, each frame
+        prepared once.  `out`, cth, fg_u and fg_v are [N, ny, nx] as in oct_optical_flow_batch_ex_dev, whose results
+        this gives bit for bit on frames[:-1], frames[1:].  Returns the list of pairs whose sector moved."""
+        nframes = int(frames.shape[0])
+        if len(t_list) != nframes:
+            raise ValueError(f"t_list needs one time per frame: {len(t_list)} for {nframes} frames")
+        if len(nav_list) != nframes - 1:
+            raise ValueError(f"nav_list needs one entry per pair: {len(nav_list)} for {nframes} frames")
+        _require("frames", frames, "float32", cuda=True)
+        B, nx, ny, navs, _, _, moved = self._batch_args(frames[:-1], frames[1:], nav_list, t_list[:-1], t_list[1:], out,
+                                                        cth, fg_u, fg_v)
+        t = (C.c_double * nframes)(*t_list)
+        self._after_torch()
+        self._check(self._L.octane_optical_flow_sequence_dev(
+            self._h, nframes, _ptr(frames), _ptr(fg_u), _ptr(fg_v), _ptr(cth), nx, ny, nc, navs, t, C.byref(p),
             _ptr(out["uPix"]), _ptr(out["vPix"]), _ptr(out["uVal"]), _ptr(out["vVal"]), _ptr(out["uVal2"]),
             _ptr(out["vVal2"]), _ptr(out.get("CTP")), moved))
         self._before_torch()

@@ -73,9 +73,12 @@ __device__ __forceinline__ float gather(const float* __restrict__ q, int pitch, 
 // because psi(x) = 1/sqrt(x + 1e-6) with x >= 0).
 enum { GNC_QUADRATIC = 0, GNC_BLEND = 1, GNC_ROBUST = 2 };
 
-template <int MODE, int OCC>
+// SPLIT: the batched instance, whose six image fields (g1, g1x, g1y, g2, g2x, g2y) of pair blockIdx.z lie `is` floats
+// after pair 0's, every other plane ps floats; the single-pair instance ignores `is`.
+template <int MODE, int OCC, bool SPLIT>
 __global__ void __launch_bounds__(256, OCC)
-k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, BuildParams bp, int halo_check, size_t ps)
+k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, BuildParams bp, int halo_check, size_t ps,
+        size_t is)
 {
     constexpr bool ROBUST = (MODE != GNC_QUADRATIC);   // robust terms needed
     constexpr bool QUAD = (MODE != GNC_ROBUST);        // quadratic terms needed
@@ -86,6 +89,7 @@ k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, Bui
     const float lambdac = bp.lambdac;
     double acc[2] = { 0.0, 0.0 };
     const size_t po = (size_t)blockIdx.z * ps;         // pair blockIdx.z: every plane is ps floats further on
+    const size_t pi = SPLIT ? (size_t)blockIdx.z * is : po;   // ... every image field pi floats
 
     // a block covers 32 columns x BUILD_ROWS rows, 8 rows at a time
     for (int jt = 0; jt < BUILD_ROWS; jt += 8) {
@@ -147,7 +151,9 @@ k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, Bui
             }
         }
         const size_t c1 = g.at(iv1, jv1) + po;
+        const size_t c1i = SPLIT ? g.at(iv1, jv1) + pi : c1;
         const size_t l = r0 + ii;
+        const size_t li = SPLIT ? g.at(0, jj) + pi + ii : l;
         // bilinear weights, :57-65; x2-x1 == y2-y1 == 1.0f exactly, so the divisions are dropped
         const float x1 = iv1, x2 = iv1 + 1, y1 = jv1, y2 = jv1 + 1;
         const float p1 = x2 - iv;
@@ -156,10 +162,10 @@ k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, Bui
         const float p4 = jv - y1;
         for (int c = 0; c < bp.nchan; c++) {
             const size_t off = (size_t)c * g.plane;
-            const size_t oc = off + c1;
-            float g2 = gather(f.g2 + oc, pitch, p1, p2, p3, p4);
-            float Ix = gather(f.g2x + oc, pitch, p1, p2, p3, p4);
-            float Iy = gather(f.g2y + oc, pitch, p1, p2, p3, p4);
+            const size_t oc = off + c1, oci = off + c1i;
+            float g2 = gather(f.g2 + oci, pitch, p1, p2, p3, p4);
+            float Ix = gather(f.g2x + oci, pitch, p1, p2, p3, p4);
+            float Iy = gather(f.g2y + oci, pitch, p1, p2, p3, p4);
             float Ixx = gather(f.g2xx + oc, pitch, p1, p2, p3, p4);
             float Ixy = gather(f.g2xy + oc, pitch, p1, p2, p3, p4);
             float Iyy = gather(f.g2yy + oc, pitch, p1, p2, p3, p4);
@@ -167,9 +173,9 @@ k_build(LevelFields f, PcgBuffers b, Geom g, int ja, int jb, int da, int db, Bui
             if (bc2) { Ix = 0.; Ixx = 0.; Ixy = 0.; }
             if (bc3) { Iy = 0.; Ixy = 0.; Iyy = 0.; }
             // :782-828
-            float It = g2 - __ldg(f.g1 + off + l);
-            float Ixt = Ix - __ldg(f.g1x + off + l);
-            float Iyt = Iy - __ldg(f.g1y + off + l);
+            float It = g2 - __ldg(f.g1 + off + li);
+            float Ixt = Ix - __ldg(f.g1x + off + li);
+            float Iyt = Iy - __ldg(f.g1y + off + li);
             float IxIx = Ix * Ix;
             float IyIy = Iy * Iy;
             float IxxIxx = Ixx * Ixx;
@@ -302,10 +308,14 @@ __global__ void __launch_bounds__(1024) k_build_finish(PcgBuffers b, unsigned nb
 }
 
 void launch_build(const LevelFields& f, const PcgBuffers& b, const Geom& g, int ja, int jb, int da, int db,
-                  const BuildParams& bp, int halo_check, cudaStream_t st, int npairs, size_t ps)
+                  const BuildParams& bp, int halo_check, cudaStream_t st, int npairs, size_t ps, size_t is)
 {
     dim3 grid((g.nx + 31) / 32, (jb - ja + BUILD_ROWS - 1) / BUILD_ROWS, npairs), block(32, 8);
-#define LAUNCH_BUILD(MODE) k_build<MODE, OCTANE_BUILD_OCC><<<grid, block, 0, st>>>(f, b, g, ja, jb, da, db, bp, halo_check, ps)
+#define LAUNCH_BUILD(MODE)                                                                                               \
+    do {                                                                                                                 \
+        if (npairs > 1) k_build<MODE, OCTANE_BUILD_OCC, true><<<grid, block, 0, st>>>(f, b, g, ja, jb, da, db, bp, halo_check, ps, is); \
+        else k_build<MODE, OCTANE_BUILD_OCC, false><<<grid, block, 0, st>>>(f, b, g, ja, jb, da, db, bp, halo_check, ps, is); \
+    } while (0)
     if (bp.al1 == 1.0)      LAUNCH_BUILD(GNC_QUADRATIC);
     else if (bp.al1 == 0.0) LAUNCH_BUILD(GNC_ROBUST);
     else                    LAUNCH_BUILD(GNC_BLEND);

@@ -181,9 +181,11 @@ struct octane_ctx {
     // workspace
     char* arena = nullptr;
     size_t arena_bytes = 0;
-    int arena_pairs = 0;           // copies of the plan's workspace (one per pair of a batch) cleared since the re-plan
-    // batched calls (octane_optical_flow_batch_dev): per-pair scalars, partial sums, group barriers, iteration
-    // counts and navigation parameters, for up to batch_cap pairs
+    // the layout (image slots, per-pair states; arena_layout) the workspace was last cleared for: a call with another
+    // layout clears it again, so that padding and unused rows hold finite values
+    int arena_slots = 0, arena_states = 0;
+    // batched calls (octane_optical_flow_batch_dev, octane_optical_flow_sequence_dev): per-pair scalars, partial sums,
+    // group barriers, iteration counts and navigation parameters, for up to batch_cap pairs
     PcgScalars* d_bscal = nullptr;
     double* d_bpart = nullptr;
     size_t bpart_doubles = 0;
@@ -197,9 +199,9 @@ struct octane_ctx {
     bool plan_valid = false;
     Buffers buf;
     std::vector<cudaGraphExec_t> pcg_graph;   // two per level: [2 * level + (constant W / N variant)]
-    // batched calls: the large levels' PCG loop of all pairs, same slots; captured for batch_graph_pairs[slot] pairs
+    // batched calls: the large levels' PCG loop of all pairs, same slots; captured for the workspace layout
+    // (arena_slots, arena_states) and destroyed when it changes
     std::vector<cudaGraphExec_t> batch_graph;
-    std::vector<int> batch_graph_pairs;
     // small persistent device objects
     PcgScalars* d_scal = nullptr;
     double* d_pending = nullptr;
@@ -245,7 +247,6 @@ void destroy_batch_graphs(octane_ctx* c)
 {
     for (auto g : c->batch_graph) if (g) cudaGraphExecDestroy(g);
     c->batch_graph.clear();
-    c->batch_graph_pairs.clear();
 }
 
 void destroy_graphs(octane_ctx* c)
@@ -257,7 +258,13 @@ void destroy_graphs(octane_ctx* c)
 
 size_t align_up(size_t x) { return (x + 255) & ~(size_t)255; }
 
-size_t arena_layout(const Plan& pl, Buffers* b, char* base)
+// The workspace: nslots image slots `is` floats apart (an image at the finest level, its current coarse level and that
+// level's gradients, nc planes each), then npairs per-pair states `ps` floats apart (second derivatives, flow, hint and
+// PCG planes).  b gets slot 0's fields as image 1's, slot 1's as image 2's and pair 0's state.  A single-pair call is
+// nslots = 2, npairs = 1; a batch of N pairs has 2N slots (pair z: slots 2z, 2z + 1), a sequence of N pairs N + 1
+// (pair z: slots z, z + 1).  Returns the bytes.
+size_t arena_layout(const Plan& pl, Buffers* b, char* base, int nslots = 2, int npairs = 1, size_t* is = nullptr,
+                    size_t* ps = nullptr)
 {
     size_t off = 0;
     auto take = [&](size_t nfloats) -> float* {
@@ -268,9 +275,11 @@ size_t arena_layout(const Plan& pl, Buffers* b, char* base)
     const size_t P = pl.P, Pc = pl.Pc, nc = pl.nc;
     Buffers tmp;
     Buffers& B = b ? *b : tmp;
-    B.img1 = take(P * nc); B.img2 = take(P * nc);
-    B.g1c = take(Pc * nc); B.g2c = take(Pc * nc);
-    B.g1x = take(P * nc); B.g1y = take(P * nc); B.g2x = take(P * nc); B.g2y = take(P * nc);
+    B.img1 = take(P * nc); B.g1c = take(Pc * nc); B.g1x = take(P * nc); B.g1y = take(P * nc);
+    const size_t slot = off;
+    B.img2 = take(P * nc); B.g2c = take(Pc * nc); B.g2x = take(P * nc); B.g2y = take(P * nc);
+    off = slot * nslots;
+    const size_t state0 = off;
     B.g2xx = take(P * nc); B.g2xy = take(P * nc); B.g2yy = take(P * nc);
     B.u = take(P); B.v = take(P); B.ut = take(Pc); B.vt = take(Pc);
     if (pl.p.first_guess) { B.uh = take(P); B.vh = take(P); B.hu = take(Pc); B.hv = take(Pc); }
@@ -280,7 +289,9 @@ size_t arena_layout(const Plan& pl, Buffers* b, char* base)
     B.pcg.pu[0] = take(P); B.pcg.pu[1] = take(P); B.pcg.pv[0] = take(P); B.pcg.pv[1] = take(P);
     B.pcg.qu = take(P); B.pcg.qv = take(P);
     B.pcg.r2u = B.pcg.qu; B.pcg.r2v = B.pcg.qv;           // the merged-reduction solver never stores q: r's second buffer
-    return off;
+    if (is) *is = slot / sizeof(float);
+    if (ps) *ps = (off - state0) / sizeof(float);
+    return state0 + (off - state0) * npairs;
 }
 
 int ensure_small(octane_ctx* c, int partial_blocks)
@@ -308,11 +319,18 @@ int ensure_small(octane_ctx* c, int partial_blocks)
     return OCTANE_OK;
 }
 
-// (re)build plan + workspace for this problem; cached across calls
-int prepare(octane_ctx* c, int nx, int ny, int nc, const octane_params& p)
+// (re)build plan + workspace for this problem; cached across calls.  batched: the caller lays the workspace out itself
+// (ensure_batch); otherwise it is made the single-pair layout c->buf describes.
+int prepare(octane_ctx* c, int nx, int ny, int nc, const octane_params& p, bool batched = false)
 {
     CUDA_OK(cudaSetDevice(c->device));
-    if (c->plan_valid && c->plan.same(nx, ny, nc, p, c->comm.rank, c->comm.world)) return OCTANE_OK;
+    if (c->plan_valid && c->plan.same(nx, ny, nc, p, c->comm.rank, c->comm.world)) {
+        if (!batched && (c->arena_slots != 2 || c->arena_states != 1)) {     // after a batched call
+            CUDA_OK(cudaMemsetAsync(c->arena, 0, arena_layout(c->plan, nullptr, nullptr), c->stream));
+            c->arena_slots = 2; c->arena_states = 1;
+        }
+        return OCTANE_OK;
+    }
     c->plan_valid = false;
     destroy_graphs(c);
     Plan pl;
@@ -395,7 +413,7 @@ int prepare(octane_ctx* c, int nx, int ny, int nc, const octane_params& p)
     c->buf.pcg.p2p.epoch = c->comm.d_epoch;
     c->buf.pcg.up_ru = c->buf.pcg.up_rv = c->buf.pcg.dn_ru = c->buf.pcg.dn_rv = nullptr;
     c->plan = pl;
-    c->arena_pairs = 1;
+    c->arena_slots = 2; c->arena_states = 1;
     c->pcg_graph.assign(2 * pl.lv.size(), nullptr);
     c->plan_valid = true;
     return OCTANE_OK;
@@ -1182,14 +1200,32 @@ int octane_optical_flow_dev(octane_ctx* c, const float* d_img1, const float* d_i
 
 // ---- batched calls: many same-size pairs, one launch per stage -----------------------------------------------------
 namespace {
-// B copies of the plan's workspace at a fixed stride; pair 0 is the single-pair workspace.  A failed allocation
-// leaves the context as it was.
-int ensure_batch(octane_ctx* c, int npairs, size_t* stride)
+// doubles of partial sums per pair of a batched call: large enough for the build, a cooperative group and a
+// merged-reduction launch (2 * partial_blocks doubles, the single-pair budget: a pair's grid is never capped below its
+// single-pair one)
+size_t batch_partials_per_pair(const Plan& pl, int partial_blocks)
+{
+    int bb = 0;
+    for (const Level& L : pl.lv) { int t = build_partial_blocks(L.g, L.g.rows); if (t > bb) bb = t; }
+    size_t per = 2 * (size_t)bb > 3 * 8 ? 2 * (size_t)bb : 3 * 8;
+    if (2 * (size_t)partial_blocks > per) per = 2 * (size_t)partial_blocks;
+    return per;
+}
+
+// bytes of ensure_batch's per-pair buffers for n pairs
+size_t batch_buffer_bytes(int n, size_t partials_per_pair)
+{
+    return n * (sizeof(PcgScalars) + partials_per_pair * sizeof(double) + 3 * sizeof(unsigned) +
+                OCTANE_MAX_SOLVES * sizeof(int) + sizeof(NavParams));
+}
+
+// The workspace of a batched call laid out with nslots image slots and npairs per-pair states (arena_layout) into *B
+// (image strides *is, pair stride *ps floats), plus the per-pair buffers.  A failed allocation leaves the context as
+// it was.
+int ensure_batch(octane_ctx* c, int nslots, int npairs, Buffers* B, size_t* is, size_t* ps)
 {
     const Plan& pl = c->plan;
-    const size_t S = arena_layout(pl, nullptr, nullptr);
-    *stride = S;
-    const size_t need = S * (size_t)npairs;
+    const size_t need = arena_layout(pl, nullptr, nullptr, nslots, npairs);
     if (need > c->arena_bytes) {
         char* na = nullptr;
         if (cudaMalloc(&na, need) != cudaSuccess) {
@@ -1199,22 +1235,12 @@ int ensure_batch(octane_ctx* c, int npairs, size_t* stride)
         }
         CUDA_OK(cudaStreamSynchronize(c->stream));
         cudaFree(c->arena);
-        c->arena = na; c->arena_bytes = need; c->arena_pairs = 0;
+        c->arena = na; c->arena_bytes = need; c->arena_slots = 0; c->arena_states = 0;
         arena_layout(pl, &c->buf, c->arena);
         destroy_graphs(c);                                   // the captured PCG loops point into the old workspace
         c->pcg_graph.assign(2 * pl.lv.size(), nullptr);
     }
-    if (npairs > c->arena_pairs) {                           // padding and unused rows must hold finite values
-        CUDA_OK(cudaMemsetAsync(c->arena + S * c->arena_pairs, 0, S * (size_t)(npairs - c->arena_pairs), c->stream));
-        c->arena_pairs = npairs;
-    }
-    // partials: one region per pair, large enough for the build, a cooperative group and a merged-reduction launch
-    // (2 * partial_blocks doubles, the single-pair budget: a pair's grid is never capped below its single-pair one)
-    int bb = 0;
-    for (const Level& L : pl.lv) { int t = build_partial_blocks(L.g, L.g.rows); if (t > bb) bb = t; }
-    size_t per = 2 * (size_t)bb > 3 * 8 ? 2 * (size_t)bb : 3 * 8;
-    if (2 * (size_t)c->partial_blocks > per) per = 2 * (size_t)c->partial_blocks;
-    const size_t pd = (size_t)npairs * per;
+    const size_t pd = (size_t)npairs * batch_partials_per_pair(pl, c->partial_blocks);
     if (npairs > c->batch_cap || pd > c->bpart_doubles) {
         CUDA_OK(cudaStreamSynchronize(c->stream));
         for (void* q : { (void*)c->d_bscal, (void*)c->d_bpart, (void*)c->d_bbar, (void*)c->d_bticket, (void*)c->d_bits,
@@ -1239,6 +1265,13 @@ int ensure_batch(octane_ctx* c, int npairs, size_t* stride)
         CUDA_OK(cudaMemsetAsync(c->d_bticket, 0, n * sizeof(unsigned), c->stream));      // each launch leaves it at 0
         c->batch_cap = n; c->bpart_doubles = pd;
     }
+    if (nslots != c->arena_slots || npairs != c->arena_states) {     // padding and unused rows must hold finite values
+        CUDA_OK(cudaMemsetAsync(c->arena, 0, need, c->stream));
+        c->arena_slots = nslots; c->arena_states = npairs;
+        destroy_batch_graphs(c);                             // the captured batched PCG loops point into the old layout
+    }
+    *B = c->buf;                                             // the scalars, partials and flags; the planes follow
+    arena_layout(pl, B, c->arena, nslots, npairs, is, ps);
     return OCTANE_OK;
 }
 
@@ -1270,8 +1303,8 @@ int enqueue_pcg_batch(octane_ctx* c, const Level& L, int level, int solve, int c
     return OCTANE_OK;
 }
 
-// enqueue_pcg_batch replayed from a graph per (level, constant-W/N variant), re-captured when npairs changes;
-// without graphs or with profiling on, enqueued directly
+// enqueue_pcg_batch replayed from a graph per (level, constant-W/N variant), captured for the workspace layout of the
+// call (ensure_batch destroys the graphs when it changes); without graphs or with profiling on, enqueued directly
 int run_pcg_batch(octane_ctx* c, const Level& L, int level, int solve, int const_wn, const PcgBuffers& pb, int npairs,
                   size_t ps)
 {
@@ -1280,38 +1313,37 @@ int run_pcg_batch(octane_ctx* c, const Level& L, int level, int solve, int const
     if (c->batch_graph.size() != 2 * c->plan.lv.size()) {
         destroy_batch_graphs(c);
         c->batch_graph.assign(2 * c->plan.lv.size(), nullptr);
-        c->batch_graph_pairs.assign(2 * c->plan.lv.size(), 0);
     }
     cudaGraphExec_t& exec = c->batch_graph[slot];
-    if (exec && c->batch_graph_pairs[slot] != npairs) {
-        CUDA_OK(cudaGraphExecDestroy(exec));
-        exec = nullptr;
-    }
     if (!exec) {
         int rc = capture_graph(c, [&] { return enqueue_pcg_batch(c, L, level, solve, const_wn, pb, npairs, ps); }, &exec);
         if (rc) return rc;
-        c->batch_graph_pairs[slot] = npairs;
     }
     CUDA_OK(cudaGraphLaunch(exec, c->stream));
     c->launches += (long long)c->plan.p.cgiters + 1;
     return OCTANE_OK;
 }
 
-// run_levels for npairs pairs in the batch workspace (pair stride ps floats); one GPU.  With a first guess, each
-// pair's hint is in its own uh / vh planes.  Per-pixel stages are one launch for all pairs; small levels solve all
-// pairs in cooperative launches with one barrier per pair (launch_pcg_coop_batch); large levels under the
-// merged-reduction solver run one launch per iteration for all pairs (run_pcg_batch), under the two-pass solver the
-// single-pair PCG kernels pair by pair.
-int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
+// run_levels for npairs pairs in the workspace B of ensure_batch (image slots is floats apart, per-pair states ps
+// floats apart); one GPU.  A batch's pair z reads slots 2z and 2z + 1, a sequence's slots z and z + 1.  With a first
+// guess, each pair's hint is in its own uh / vh planes.  Per-pixel stages are one launch for all pairs or all slots;
+// small levels solve all pairs in cooperative launches with one barrier per pair (launch_pcg_coop_batch); large levels
+// under the merged-reduction solver run one launch per iteration for all pairs (run_pcg_batch), under the two-pass
+// solver the single-pair PCG kernels pair by pair.
+int run_levels_batch(octane_ctx* c, int npairs, bool sequence, const Buffers& B, size_t is, size_t ps)
 {
     const Plan& pl = c->plan;
-    Buffers& B = c->buf;
     const octane_params& p = pl.p;
     const int K = p.kiters, nc = pl.nc;
     const int nsol = K * 3 * p.liters;
     cudaStream_t st = c->stream;
     const float sf = (float)p.scaleF;
     const size_t S = ps * sizeof(float);
+    // pair z's image 1 is B's image-1 fields + z * istep, its image 2 the image-2 fields + z * istep.  The per-image
+    // stages visit every slot once: a sequence's npairs + 1 slots in one launch, a batch's image-1 slots and its
+    // image-2 slots in one launch each.
+    const size_t istep = sequence ? is : 2 * is;
+    const int runs = sequence ? 1 : 2, run_slots = sequence ? npairs + 1 : npairs;
     PcgBuffers pb = B.pcg;                       // build and update: pair z uses d_bscal[z] (and partials region z)
     pb.scal = c->d_bscal;
     pb.partials = c->d_bpart;
@@ -1332,9 +1364,10 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
         if (!finest) {
             const Geom& gF = pl.lv[K - 1].g;
             launch_fill_gk(c->d_gk, L.factor, L.R, st);
-            launch_blur_decimate(B.img1, gF, B.g1c, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, 1.f, nc, st, npairs, ps);
-            launch_blur_decimate(B.img2, gF, B.g2c, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, 1.f, nc, st, npairs, ps);
-            c->launches += 3;
+            for (int r = 0; r < runs; r++)
+                launch_blur_decimate(r ? B.img2 : B.img1, gF, r ? B.g2c : B.g1c, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R,
+                                     1.f, nc, st, run_slots, istep);
+            c->launches += 1 + runs;
             if (p.first_guess) {
                 launch_blur_decimate(B.uh, gF, B.hu, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, L.factor, 1, st, npairs, ps);
                 launch_blur_decimate(B.vh, gF, B.hv, g, g.jlo(), g.jhi(), L.factor, c->d_gk, L.R, L.factor, 1, st, npairs, ps);
@@ -1354,11 +1387,12 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
                 CUDA_OK(cudaMemset2DAsync(B.v, S, 0, w, npairs, st));
             }
         }
-        launch_gradient(g1, B.g1x, B.g1y, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
-        launch_gradient(g2, B.g2x, B.g2y, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
-        launch_gradient(B.g2x, B.g2xx, nullptr, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
-        launch_gradient(B.g2y, B.g2xy, B.g2yy, g, g.jlo(), g.jhi(), nc, st, npairs, ps);
-        c->launches += 4;
+        for (int r = 0; r < runs; r++)
+            launch_gradient(r ? g2 : g1, r ? B.g2x : B.g1x, r ? B.g2y : B.g1y, g, g.jlo(), g.jhi(), nc, st, run_slots, istep,
+                            istep);
+        launch_gradient(B.g2x, B.g2xx, nullptr, g, g.jlo(), g.jhi(), nc, st, npairs, ps, istep);
+        launch_gradient(B.g2y, B.g2xy, B.g2yy, g, g.jlo(), g.jhi(), nc, st, npairs, ps, istep);
+        c->launches += runs + 2;
         LevelFields f;
         f.g1 = g1; f.g1x = B.g1x; f.g1y = B.g1y;
         f.g2 = g2; f.g2x = B.g2x; f.g2y = B.g2y; f.g2xx = B.g2xx; f.g2xy = B.g2xy; f.g2yy = B.g2yy;
@@ -1374,7 +1408,7 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
         for (int gnc = 0; gnc < 3; gnc++) {
             bp.al1 = 1. - 0.5 * gnc;
             for (int l = 0; l < p.liters; l++, solve++) {
-                launch_build(f, pb, g, L.own0, L.own1, L.own0, L.own1, bp, 0, st, npairs, ps);
+                launch_build(f, pb, g, L.own0, L.own1, L.own0, L.own1, bp, 0, st, npairs, ps, istep);
                 c->launches += 2;
                 if (p.cgiters > 0 && small) {
                     for (int p0 = 0; p0 < npairs; p0 += per_launch) {
@@ -1413,13 +1447,14 @@ int run_levels_batch(octane_ctx* c, int npairs, size_t ps)
     return OCTANE_OK;
 }
 
-// the body of octane_optical_flow_batch_ex_dev and octane_optical_flow_batch_dev (which passes no first guess)
-int optical_flow_batch(octane_ctx* c, int npairs, const float* d_img1, const float* d_img2, const float* d_fg_u,
-                       const float* d_fg_v, const float* d_cth, int nx, int ny, int nc, const octane_nav* nav,
-                       const double* t1, const double* t2, const octane_params* p, float* d_upix, float* d_vpix, short* U,
-                       short* V, short* Ur, short* Vr, short* d_ctp, int* moved_out)
+// the body of octane_optical_flow_batch_ex_dev, octane_optical_flow_batch_dev (which passes no first guess) and
+// octane_optical_flow_sequence_dev (sequence: d_img1 holds the npairs + 1 frames, d_img2 is unused and t2 = t1 + 1)
+int optical_flow_batch(octane_ctx* c, int npairs, bool sequence, const float* d_img1, const float* d_img2,
+                       const float* d_fg_u, const float* d_fg_v, const float* d_cth, int nx, int ny, int nc,
+                       const octane_nav* nav, const double* t1, const double* t2, const octane_params* p, float* d_upix,
+                       float* d_vpix, short* U, short* V, short* Ur, short* Vr, short* d_ctp, int* moved_out)
 {
-    if (!c || !d_img1 || !d_img2 || !nav || !t1 || !t2 || !p || !d_upix || !d_vpix || !U || !V || !Ur || !Vr) {
+    if (!c || !d_img1 || (!sequence && !d_img2) || !nav || !t1 || !t2 || !p || !d_upix || !d_vpix || !U || !V || !Ur || !Vr) {
         set_err("null argument");
         return OCTANE_EINVAL;
     }
@@ -1429,13 +1464,15 @@ int optical_flow_batch(octane_ctx* c, int npairs, const float* d_img1, const flo
     if (!srsal_args_ok(p, d_cth, nx, ny)) return OCTANE_EINVAL;
     if (c->comm.world > 1) { set_err("context is banded: batched calls are single-GPU"); return OCTANE_EINVAL; }
     begin_call(c);
-    int rc = prepare(c, nx, ny, nc, *p);
+    int rc = prepare(c, nx, ny, nc, *p, true);
     if (rc) return rc;
     if (p->kiters * 3 * p->liters > OCTANE_MAX_SOLVES) { set_err("too many solves"); return OCTANE_EINVAL; }
-    size_t S = 0;
-    rc = ensure_batch(c, npairs, &S);
+    const int nslots = sequence ? npairs + 1 : 2 * npairs;
+    Buffers B;
+    size_t is = 0, ps = 0;
+    rc = ensure_batch(c, nslots, npairs, &B, &is, &ps);
     if (rc) return rc;
-    const size_t ps = S / sizeof(float), n = (size_t)nx * ny;
+    const size_t n = (size_t)nx * ny;
     cudaStream_t st = c->stream;
     // every allocation of the call before its first copy or launch: a failed one leaves nothing half enqueued
     const size_t need = pix2uv_table_doubles(nx, ny) * (size_t)npairs;
@@ -1456,26 +1493,27 @@ int optical_flow_batch(octane_ctx* c, int npairs, const float* d_img1, const flo
         rc = ensure_stage(c, 2 * sfb);
         if (rc) return rc;
     }
-    // dense pairs -> pitched finest-level planes of each pair's workspace; the first guess is copied in before any
-    // output is written, so it may alias d_upix / d_vpix
+    // dense images -> pitched finest-level planes of the image slots (each frame of a sequence once); the first guess
+    // is copied in before any output is written, so it may alias d_upix / d_vpix
     const Geom& g = c->plan.lv.back().g;
     const size_t w = (size_t)nx * sizeof(float), dp = (size_t)g.pitch * sizeof(float);
-    for (int b = 0; b < npairs; b++) {
-        for (int ch = 0; ch < nc; ch++) {
-            const size_t src = ((size_t)b * nc + ch) * n, dst = (size_t)b * ps + (size_t)ch * g.plane;
-            CUDA_OK(cudaMemcpy2DAsync(c->buf.img1 + dst, dp, d_img1 + src, w, w, ny, cudaMemcpyDeviceToDevice, st));
-            CUDA_OK(cudaMemcpy2DAsync(c->buf.img2 + dst, dp, d_img2 + src, w, w, ny, cudaMemcpyDeviceToDevice, st));
-        }
-        if (p->first_guess) {
-            CUDA_OK(cudaMemcpy2DAsync(c->buf.uh + (size_t)b * ps, dp, d_fg_u + b * n, w, w, ny, cudaMemcpyDeviceToDevice, st));
-            CUDA_OK(cudaMemcpy2DAsync(c->buf.vh + (size_t)b * ps, dp, d_fg_v + b * n, w, w, ny, cudaMemcpyDeviceToDevice, st));
+    for (int k = 0; k < nslots; k++) {
+        const float* src = sequence ? d_img1 + (size_t)k * nc * n : (k & 1 ? d_img2 : d_img1) + (size_t)(k >> 1) * nc * n;
+        for (int ch = 0; ch < nc; ch++)
+            CUDA_OK(cudaMemcpy2DAsync(B.img1 + (size_t)k * is + (size_t)ch * g.plane, dp, src + (size_t)ch * n, w, w, ny,
+                                      cudaMemcpyDeviceToDevice, st));
+    }
+    if (p->first_guess) {
+        for (int b = 0; b < npairs; b++) {
+            CUDA_OK(cudaMemcpy2DAsync(B.uh + (size_t)b * ps, dp, d_fg_u + b * n, w, w, ny, cudaMemcpyDeviceToDevice, st));
+            CUDA_OK(cudaMemcpy2DAsync(B.vh + (size_t)b * ps, dp, d_fg_v + b * n, w, w, ny, cudaMemcpyDeviceToDevice, st));
         }
     }
-    rc = run_levels_batch(c, npairs, ps);
+    rc = run_levels_batch(c, npairs, sequence, B, is, ps);
     if (rc) return rc;
     for (int b = 0; b < npairs; b++) {
-        CUDA_OK(cudaMemcpy2DAsync(d_upix + b * n, w, c->buf.u + (size_t)b * ps, dp, w, ny, cudaMemcpyDeviceToDevice, st));
-        CUDA_OK(cudaMemcpy2DAsync(d_vpix + b * n, w, c->buf.v + (size_t)b * ps, dp, w, ny, cudaMemcpyDeviceToDevice, st));
+        CUDA_OK(cudaMemcpy2DAsync(d_upix + b * n, w, B.u + (size_t)b * ps, dp, w, ny, cudaMemcpyDeviceToDevice, st));
+        CUDA_OK(cudaMemcpy2DAsync(d_vpix + b * n, w, B.v + (size_t)b * ps, dp, w, ny, cudaMemcpyDeviceToDevice, st));
     }
     if (p->doCTH) {                            // src/oct_optical_flow.cc:71-88, all pairs in one launch
         launch_ctp_pack(d_cth, d_ctp, (size_t)npairs * n, p->ir == 1, st);
@@ -1508,8 +1546,34 @@ int octane_optical_flow_batch_ex_dev(octane_ctx* c, int npairs, const float* d_i
                                      float* d_upix, float* d_vpix, short* U, short* V, short* Ur, short* Vr, short* d_ctp,
                                      int* moved_out)
 {
-    return optical_flow_batch(c, npairs, d_img1, d_img2, d_fg_u, d_fg_v, d_cth, nx, ny, nc, nav, t1, t2, p, d_upix, d_vpix,
-                              U, V, Ur, Vr, d_ctp, moved_out);
+    return optical_flow_batch(c, npairs, false, d_img1, d_img2, d_fg_u, d_fg_v, d_cth, nx, ny, nc, nav, t1, t2, p, d_upix,
+                              d_vpix, U, V, Ur, Vr, d_ctp, moved_out);
+}
+
+int octane_optical_flow_sequence_dev(octane_ctx* c, int nframes, const float* d_frames, const float* d_fg_u,
+                                     const float* d_fg_v, const float* d_cth, int nx, int ny, int nc,
+                                     const octane_nav* nav, const double* t, const octane_params* p, float* d_upix,
+                                     float* d_vpix, short* U, short* V, short* Ur, short* Vr, short* d_ctp, int* moved_out)
+{
+    if (nframes < 2) { set_err("a sequence needs at least 2 frames"); return OCTANE_EINVAL; }
+    return optical_flow_batch(c, nframes - 1, true, d_frames, nullptr, d_fg_u, d_fg_v, d_cth, nx, ny, nc, nav, t,
+                              t ? t + 1 : nullptr, p, d_upix, d_vpix, U, V, Ur, Vr, d_ctp, moved_out);
+}
+
+size_t octane_batch_workspace_bytes(int npairs, int sequence, int nx, int ny, int nc, const octane_params* p)
+{
+    Plan pl;
+    if (!p || npairs < 1 || make_plan(pl, nx, ny, nc, *p, 0, 1)) return 0;
+    const int nslots = sequence ? npairs + 1 : 2 * npairs;
+    // the partial-sum budget prepare gives a context on a 148-SM B200
+    int pb = 148 * 16;
+    for (const Level& L : pl.lv) { int t = build_partial_blocks(L.g, L.g.rows); if (t > pb) pb = t; }
+    const size_t n = (size_t)nx * ny;
+    size_t bytes = arena_layout(pl, nullptr, nullptr, nslots, npairs) +
+                   batch_buffer_bytes(npairs, batch_partials_per_pair(pl, pb)) +
+                   pix2uv_table_doubles(nx, ny) * (size_t)npairs * sizeof(double);
+    if (p->dosrsal) bytes += 2 * align_up((size_t)npairs * n * sizeof(float));
+    return bytes;
 }
 
 int octane_optical_flow_batch_dev(octane_ctx* c, int npairs, const float* d_img1, const float* d_img2, const float* d_cth,
@@ -1519,8 +1583,8 @@ int octane_optical_flow_batch_dev(octane_ctx* c, int npairs, const float* d_img1
 {
     if (p && p->first_guess) { set_err("batched calls take no first guess: use octane_optical_flow_batch_ex_dev"); return OCTANE_EINVAL; }
     if (p && p->dosrsal) { set_err("octane_optical_flow_batch_dev does not run -srsal: use octane_optical_flow_batch_ex_dev"); return OCTANE_EINVAL; }
-    return optical_flow_batch(c, npairs, d_img1, d_img2, nullptr, nullptr, d_cth, nx, ny, nc, nav, t1, t2, p, d_upix, d_vpix,
-                              U, V, Ur, Vr, d_ctp, moved_out);
+    return optical_flow_batch(c, npairs, false, d_img1, d_img2, nullptr, nullptr, d_cth, nx, ny, nc, nav, t1, t2, p, d_upix,
+                              d_vpix, U, V, Ur, Vr, d_ctp, moved_out);
 }
 
 int octane_batch_cg_iterations(octane_ctx* c, int* its, int npairs)

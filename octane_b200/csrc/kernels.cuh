@@ -11,8 +11,9 @@ void launch_fill_gk(float* GK, float factor, int R, cudaStream_t st);
 void launch_blur_decimate(const float* src, const Geom& gs, float* dst, const Geom& gd, int ja, int jb,
                           float factor, const float* GK, int R, float scale, int nc, cudaStream_t st,
                           int npairs = 1, size_t ps = 0);
+// batched: pair z reads f + z * ps_in and writes gx, gy + z * ps
 void launch_gradient(const float* f, float* gx, float* gy, const Geom& g, int ja, int jb, int nc, cudaStream_t st,
-                     int npairs = 1, size_t ps = 0);
+                     int npairs = 1, size_t ps = 0, size_t ps_in = 0);
 void launch_zoom_in(const float* flow, const Geom& gc, float* out, const Geom& gf, int ja, int jb, float sf,
                     cudaStream_t st, int npairs = 1, size_t ps = 0);
 
@@ -64,9 +65,10 @@ struct BuildParams {
     float tol;
 };
 // rows [ja,jb) get coefficients + rhs; dots (b.b, b.Minv b) over rows [da,db).  Batched: pair z seeds b.scal[z] and
-// uses partials region z (2 * build_partial_blocks doubles each).
+// uses partials region z (2 * build_partial_blocks doubles each); its image fields g1, g1x, g1y, g2, g2x, g2y lie
+// z * is floats after pair 0's, every other plane z * ps.
 void launch_build(const LevelFields& f, const PcgBuffers& b, const Geom& g, int ja, int jb, int da, int db,
-                  const BuildParams& bp, int halo_check, cudaStream_t st, int npairs = 1, size_t ps = 0);
+                  const BuildParams& bp, int halo_check, cudaStream_t st, int npairs = 1, size_t ps = 0, size_t is = 0);
 int build_partial_blocks(const Geom& g, int nrows);
 
 // shared memory one block of k_blur_decimate needs for a level (pyramid.cu); levels beyond the limit are refused

@@ -124,11 +124,13 @@ __device__ __forceinline__ float4 grad_row(const float* __restrict__ f, const Ge
     return c;
 }
 
-// VEC: rows start on 16-byte boundaries (every plane of a plan does; the dense arrays of the stage entry point need not)
-template <bool VEC>
+// VEC: rows start on 16-byte boundaries (every plane of a plan does; the dense arrays of the stage entry point need not).
+// SPLIT: the batched instance, whose input planes of pair p lie p * ps_in floats after pair 0's and its outputs p * ps
+// (a sequence's second derivatives read image slots and write per-pair planes); the single-pair instance ignores ps_in.
+template <bool VEC, bool SPLIT>
 __global__ void __launch_bounds__(256)
 k_gradient(const float* __restrict__ f, float* __restrict__ gx, float* __restrict__ gy, Geom g,
-           int ja, int jb, int nc, size_t ps)
+           int ja, int jb, int nc, size_t ps, size_t ps_in)
 {
     const int lane = threadIdx.x;
     const int i0 = (blockIdx.x * 32 + lane) * 4;
@@ -136,7 +138,8 @@ k_gradient(const float* __restrict__ f, float* __restrict__ gx, float* __restric
     if (js >= jb) return;                                  // whole warp: js depends on threadIdx.y only
     const unsigned pair = blockIdx.z / nc;            // blockIdx.z = pair * nc + channel
     const size_t coff = (size_t)(blockIdx.z - pair * nc) * g.plane + pair * ps;
-    f += coff; gx += coff;
+    f += SPLIT ? (size_t)(blockIdx.z - pair * nc) * g.plane + pair * ps_in : coff;
+    gx += coff;
     if (gy) gy += coff;
     const int lo = g.jlo(), hi = g.jhi() - 1;
     float4 w0 = grad_row<VEC>(f, g, i0, js - 2), w1 = grad_row<VEC>(f, g, i0, js - 1), w2 = grad_row<VEC>(f, g, i0, js),
@@ -306,14 +309,19 @@ void launch_blur_decimate(const float* src, const Geom& gs, float* dst, const Ge
 }
 
 void launch_gradient(const float* f, float* gx, float* gy, const Geom& g, int ja, int jb, int nc, cudaStream_t st,
-                     int npairs, size_t ps)
+                     int npairs, size_t ps, size_t ps_in)
 {
     if (jb <= ja) return;
     dim3 grid((g.nx + 127) / 128, (jb - ja + 8 * GRAD_ROWS - 1) / (8 * GRAD_ROWS), nc * npairs), block(32, 8);
     const bool vec = (g.pitch & 3) == 0 && (g.plane & 3) == 0 &&
                      (((uintptr_t)f | (uintptr_t)gx | (uintptr_t)gy) & 15) == 0;
-    if (vec) k_gradient<true><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc, ps);
-    else k_gradient<false><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc, ps);
+    if (npairs > 1) {
+        if (vec) k_gradient<true, true><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc, ps, ps_in);
+        else k_gradient<false, true><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc, ps, ps_in);
+    } else {
+        if (vec) k_gradient<true, false><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc, ps, ps_in);
+        else k_gradient<false, false><<<grid, block, 0, st>>>(f, gx, gy, g, ja, jb, nc, ps, ps_in);
+    }
 }
 
 void launch_zoom_in(const float* flow, const Geom& gc, float* out, const Geom& gf, int ja, int jb, float sf,

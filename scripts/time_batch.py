@@ -9,7 +9,13 @@ power limit.  Writes --out (JSON).
 --first-guess (with lambda_c = 0.5) and --srsal time the same workloads with those flags: the batch arm calls
 octane_optical_flow_batch_ex_dev, the contexts arms pass the same flags to octane_optical_flow_dev, and with --srsal a
 second batch arm without -srsal gives the cost of the smoother.  The default output is then
-profiles/r03_batch_fg_srsal_n1.json."""
+profiles/r03_batch_fg_srsal_n1.json.
+
+--sequence times octane_optical_flow_sequence_dev on npairs + 1 frames against octane_optical_flow_batch_ex_dev on
+the same pairs (frames[:-1], frames[1:]), alternated, for 64 x 500^2 (65 frames) and 8 x 2000^2 (9 frames).  The
+frames alternate the two images of a synthetic pair, so every pair has real motion.  It also reports the device
+bytes each call allocates (octane_batch_workspace_bytes) and whether the two arms' outputs are bit-identical.  The
+default output is then profiles/r04_sequence_n1.json."""
 import argparse
 import json
 import os
@@ -145,6 +151,74 @@ def workload(n, npairs, seed0, rounds, steps, warmup, fg=False, srsal=False):
             **({"dosrsal": 1} if srsal else {}), **res}
 
 
+def sequence_workload(n, npairs, seed, rounds, steps, warmup):
+    import torch
+
+    import octane_b200 as ob
+    from octane_b200 import synthetic as S
+
+    dev = torch.device("cuda", 0)
+    xs, ys, xo, yo, dt = S.SECTORS["meso_2km"]
+    nav = ob.goes_nav(xs, ys, xo, yo)
+    p = ob.default_params(doCTH=1)
+    a, b = S.make_pair_torch(n, n, seed, dev)
+    frames = torch.stack([a if k % 2 == 0 else b for k in range(npairs + 1)]).contiguous()
+    t = [dt * k for k in range(npairs + 1)]
+    yy, xx = np.mgrid[0:n, 0:n].astype(np.float32)
+    cth1 = torch.from_numpy((7500.0 + 7400.0 * np.sin(xx / 40.0) * np.cos(yy / 30.0)).astype(np.float32)).to(dev)
+    cth = cth1.expand(npairs, n, n).contiguous()
+
+    def outputs():
+        o = {k: torch.zeros((npairs, n, n), device=dev) for k in ("uPix", "vPix")}
+        for k in ("uVal", "vVal", "uVal2", "vVal2", "CTP"):
+            o[k] = torch.zeros((npairs, n, n), dtype=torch.int16, device=dev)
+        return o
+
+    ctx = ob.Context(0)
+    outs = {"sequence": outputs(), "batch": outputs()}
+    navs = [nav] * npairs
+    arms = {
+        "sequence": lambda: ctx.oct_optical_flow_sequence_dev(frames, navs, t, p, outs["sequence"], cth=cth),
+        "batch": lambda: ctx.oct_optical_flow_batch_ex_dev(frames[:-1], frames[1:], navs, t[:-1], t[1:], p,
+                                                           outs["batch"], cth=cth),
+    }
+
+    def timed(fn):
+        ctx.synchronize()
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        ctx._after_torch()
+        for _ in range(steps):
+            fn()
+        ctx._before_torch()
+        e1.record()
+        ctx.synchronize()
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) / steps
+
+    for fn in arms.values():
+        for _ in range(warmup):
+            fn()
+    ms = {k: [] for k in arms}
+    for _ in range(rounds):                       # alternate the arms
+        for k, fn in arms.items():
+            ms[k].append(timed(fn))
+    res = {}
+    mpix = npairs * n * n / 1e6
+    for k, fn in arms.items():
+        fn()
+        best = min(ms[k])
+        res[k] = {"ms_per_step": best, "ms_per_step_all": ms[k], "mpix_per_s": mpix / (best / 1e3),
+                  "kernel_launches_per_step": int(ctx.stats().kernel_launches)}
+    torch.cuda.synchronize()
+    res["outputs_bit_identical"] = all(torch.equal(outs["sequence"][k], outs["batch"][k]) for k in outs["batch"])
+    res["workspace_bytes"] = {"sequence": ob.batch_workspace_bytes(npairs, n, n, 1, p, sequence=True),
+                              "batch": ob.batch_workspace_bytes(npairs, n, n, 1, p)}
+    ctx.close()
+    return {"pairs": npairs, "frames": npairs + 1, "size": n, "doCTH": 1, "output": "m/s", **res}
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("--out", default=None)
@@ -153,13 +227,21 @@ def main():
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--first-guess", action="store_true", help="solve with a first guess and lambda_c = 0.5")
     ap.add_argument("--srsal", action="store_true", help="run the -srsal post-smoother")
+    ap.add_argument("--sequence", action="store_true", help="time the sequence call against the batch on the same frames")
     a = ap.parse_args()
-    name = "r03_batch_fg_srsal_n1.json" if a.first_guess or a.srsal else "r03_batch_n1.json"
+    if a.sequence and (a.first_guess or a.srsal):
+        ap.error("--sequence times the plain call")
+    name = ("r04_sequence_n1.json" if a.sequence else
+            "r03_batch_fg_srsal_n1.json" if a.first_guess or a.srsal else "r03_batch_n1.json")
     a.out = a.out or os.path.join(ROOT, "profiles", name)
     flags = dict(fg=a.first_guess, srsal=a.srsal)
-    res = {"card": card(), "what": "device ms per step over CUDA events, best of the alternated rounds",
-           "workloads": [workload(500, 64, 100, a.rounds, a.steps, a.warmup, **flags),
-                         workload(2000, 8, 300, a.rounds, a.steps, a.warmup, **flags)]}
+    res = {"card": card(), "what": "device ms per step over CUDA events, best of the alternated rounds"}
+    if a.sequence:
+        res["workloads"] = [sequence_workload(500, 64, 100, a.rounds, a.steps, a.warmup),
+                            sequence_workload(2000, 8, 300, a.rounds, a.steps, a.warmup)]
+    else:
+        res["workloads"] = [workload(500, 64, 100, a.rounds, a.steps, a.warmup, **flags),
+                            workload(2000, 8, 300, a.rounds, a.steps, a.warmup, **flags)]
     os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
     with open(a.out, "w") as f:
         json.dump(res, f, indent=1)
